@@ -38,6 +38,23 @@ def log(*a):
     print(*a, file=sys.stderr, flush=True)
 
 
+DUMP_BYTES = 8 << 20          # decoded bytes sampled by --dump-outputs: 32 MiB as float32, the rest of 64 MB left to the per-frame results
+
+
+def dump_outputs(out_dir, torch, dst, res, n, fb):
+    """--dump-outputs: what the last timed step handed its caller, as .npy files under `out_dir` -- every frame's result
+    (float64: the decoded size, or -code for a ZSTD error, which is returned as 2**64 - code and would round to one value as a
+    float) and the decoded bytes (float32) of a fixed, seeded sample of frames, rows in ascending frame order; the sample covers
+    at most DUMP_BYTES bytes, so two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    k = max(1, min(n, DUMP_BYTES // fb))
+    rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    sample = dst[:n * fb].view(n, fb)[torch.from_numpy(rows).to(dst.device), :min(fb, DUMP_BYTES)]
+    np.save(os.path.join(out_dir, "decoded_sample.npy"), sample.float().cpu().numpy())
+    results = np.array([r if r < 2**63 else -(2**64 - r) for r in res], dtype=np.float64)
+    np.save(os.path.join(out_dir, "frame_results.npy"), results if results.nbytes <= (16 << 20) else results[rows])
+
+
 def make_corpus(nframes, frame_bytes, level=3, pool=64, seed_shift=0):
     """-> (raw [nframes, frame_bytes] uint8, list of compressed frames).  Every frame is distinct (rotated copies of `pool`
     frames per family) and the families are interleaved by a fixed permutation; the frames are compressed by the reference's
@@ -146,7 +163,7 @@ def run_reference(args, rank, world):
         return
     threads = os.cpu_count() or 1
     data, frames = make_corpus(args.frames, args.frame_bytes)
-    from oracle import cpubench
+    from oracle import cpubench, ref
     blob = np.frombuffer(b"".join(frames), dtype=np.uint8)
     fs = cpubench.FrameSet(blob, [len(f) for f in frames])
     caps = [args.frame_bytes] * len(frames)
@@ -155,7 +172,7 @@ def run_reference(args, rank, world):
     times = [cpubench.run("decompress", fs, caps, threads)[0] for _ in range(args.steps)]
     total = sum(times)
     val = len(frames) * args.frame_bytes * args.steps / total / 1e9
-    desc = f"all {args.frames} frames of one GPU's shard, {threads} threads, one DCtx per thread (oracle/_ref libzstd 1.5.6, oracle/cpu_bench.c)"
+    desc = f"all {args.frames} frames of one GPU's shard, {threads} threads, one DCtx per thread (system libzstd {ref.version()}, oracle/cpu_bench.c)"
     out = {"metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
            "ms_per_step": 1e3 * total / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
            "dtype": "u8", "data": "synthetic", "impl": "reference",
@@ -334,7 +351,7 @@ def compress_leg(torch, dist, z, args, dev, rank, world):
         dom = max((k for k in stages if stages[k] > 0), key=lambda k: stages[k], default=None)
         out[f"level{lvl}"] = {"GBps": world * n * fb / ms / 1e6, "ms": ms, "ratio": n * fb / csize, "size_vs_libzstd": ours / theirs,
                               "size_vs_libzstd_how": f"{len(range(0, n, max(1, n // 128)))} sampled frames, libzstd at the same level on the same slabs",
-                              "kernel_ms": kernel_ms, "stages_ms": stages,
+                              "kernel_ms": kernel_ms, "stages_ms": stages, "steps": iters,
                               "stages_how": "CUDA events between the kernels, summed over the waves of the last device-resident call (a call of more than 8,192 blocks runs in waves)",
                               "frames_per_gpu": n, "frame_bytes": fb, "n_gpus": world,
                               "roofline": {"bound": "hbm", "achieved": alg / ms / 1e6, "peak": peak, "unit": "GB/s", "frac": alg / ms / 1e6 / peak,
@@ -491,7 +508,7 @@ def dict_leg(torch, z, args, dev):
         c = host[int(coffs[i]):int(coffs[i]) + csz[i]].tobytes()
         assert rd.decompress(c, cap=sizes[i]) == objs[i], "GPU dictionary frame does not decode with libzstd"
         ours += csz[i]; theirs += len(rc.compress(objs[i])); refpipe += len(rc_ref.compress(objs[i]))
-    return {"objects": n, "bytes": total, "dict_bytes": len(d), "level": 3, "compress_GBps": total / ms_c / 1e6, "compress_ms": ms_c,
+    return {"objects": n, "bytes": total, "dict_bytes": len(d), "level": 3, "steps": 3, "compress_GBps": total / ms_c / 1e6, "compress_ms": ms_c,
             "decompress_GBps": total / ms_d / 1e6, "decompress_ms": ms_d, "ratio": total / sum(csz),
             "size_vs_libzstd_same_dict": ours / theirs, "size_vs_reference_pipeline": ours / refpipe,
             "size_vs_reference_pipeline_how": "GPU-trained dictionary + GPU compressor against ZDICT-trained dictionary + libzstd, level 3",
@@ -545,7 +562,7 @@ def large_frame_leg(torch, z, args, dev):
     e1.record(stream); torch.cuda.synchronize()
     ms_c = e0.elapsed_time(e1) / 5
     return {"rows": args.df_rows, "bytes": n, "frame_bytes_libzstd": len(frame), "frame_bytes_ours": csz, "size_vs_libzstd": csz / len(frame),
-            "decompress_GBps": n / ms_d / 1e6, "decompress_ms": ms_d, "compress_GBps": n / ms_c / 1e6, "compress_ms": ms_c,
+            "decompress_GBps": n / ms_d / 1e6, "decompress_ms": ms_d, "compress_GBps": n / ms_c / 1e6, "compress_ms": ms_c, "steps": 5,
             "libzstd_1thread_decompress_GBps": n / t_cd / 1e9, "libzstd_1thread_compress_GBps": n / t_cc / 1e9,
             "libzstd_nbWorkers_compress_GBps": n / t_w / 1e9, "libzstd_nbWorkers": threads, "libzstd_nbWorkers_frame_bytes": size_w,
             "cpu_baseline_how": "the reference's path for this config: one frame, level 3; num_threads = 1 (ZSTD_compress2 / ZSTD_decompressDCtx) and "
@@ -574,7 +591,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--config5-frames", type=int, default=262144, help="frames of configs[4] in total (32 GiB), split over the ranks")
     ap.add_argument("--no-config5", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output under DIR as .npy files (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -635,12 +655,14 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
     for _ in range(args.steps):
-        plan.decompress(dctx)
+        res = plan.decompress(dctx)
     e1.record(stream)
     sync_all()
     clocks = sampler.stop()
     ms_total = e0.elapsed_time(e1)
     launches = dctx.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, dst, res, n, fb)
     # per-kernel durations: the same batch as ONE slice on ONE stream with CUDA events between the kernels (the timed
     # region above runs the slice pipeline, where kernels of different slices overlap and have no duration of their own)
     dctx.set_profile(True)
@@ -663,7 +685,7 @@ def main():
     sync_all()
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e2.record(stream)
-    e2e_steps = max(3, args.steps)          # the same K steps as the device-resident arm (five used to scatter by +-3 % between runs)
+    e2e_steps = args.steps                  # the same K steps as the device-resident arm (five used to scatter by +-3 % between runs)
     for _ in range(e2e_steps):
         hplan.decompress(dctx, device=False)
     e3.record(stream)
@@ -732,7 +754,7 @@ def main():
                        "pcie_ceiling_GBps": total_bytes / ms_pcie / 1e6, "frac_of_pcie_ceiling": (total_bytes * e2e_steps / ms_e2e) / (total_bytes / ms_pcie),
                        "pcie_ceiling_how": "this step's H2D and D2H byte counts as two plain concurrent cudaMemcpyAsync (pinned <-> HBM) on every rank at once, "
                                            "slower direction, max over ranks, best of 3",
-                       "pageable": {"value": total_bytes / ms_page / 1e6, "unit": UNIT, "ms_per_step": ms_page,
+                       "pageable": {"value": total_bytes / ms_page / 1e6, "unit": UNIT, "ms_per_step": ms_page, "steps": 3,
                                     "how": "the same call with malloc'ed (pageable) host buffers, as the reference's C layer passes them"},
                        "cpu_affinity": affinity},
                "gpu_launches": int(launches), "clocks": clocks,
@@ -744,6 +766,8 @@ def main():
                             "serial_pipeline_ms": serial_ms,
                             "whole_pipeline_frac": (alg_bytes / (ms_total / args.steps) / 1e6) / peak},
                "stages_ms": {nm: float(v) for nm, v in zip(stage_names, stage_ms)},
+               "steps_note": "--steps sets the device-resident and pinned end-to-end arms; the pageable arm and the compress, config5, "
+                             "dict and large_frame legs time fixed repetitions, given in each as steps or in its how",
                "compression_ratio_of_input": n * fb / csize}
         traffic_path = os.path.join(ROOT, "profiles", "dominant_kernel_traffic.json")
         if os.path.exists(traffic_path):
@@ -755,6 +779,7 @@ def main():
             except (ValueError, OSError):
                 pass
         if world == 1 and not args.no_cpu:
+            from oracle import ref
             threads = os.cpu_count() or 1
             nsample = min(n, args.cpu_frames)
             step = max(1, n // nsample)
@@ -763,7 +788,7 @@ def main():
             v1, _, _ = cpu_leg(sample[:max(1, len(sample) // threads)], fb, 2.0, 1)
             out["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": threads, "kind": "reference",
                                    "sample": f"{len(sample)} of the {n} frames" + (f" (every {step}th, same family mix)" if step > 1 else "") +
-                                             f", frame-parallel, best of {passes} passes, oracle/_ref libzstd 1.5.6, one DCtx per thread",
+                                             f", frame-parallel, best of {passes} passes, system libzstd {ref.version()}, one DCtx per thread",
                                    "one_thread_GBps": v1,
                                    "note": "libzstd has no multi-threaded decompression: num_threads = cores changes nothing on this side (BASELINE.md section 3)"}
         if comp is not None:

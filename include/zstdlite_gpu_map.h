@@ -4,7 +4,7 @@
  * raw-file.c:52,74,150,155,189; raw-file-in.c:66,102; raw-file-out.c:89-118; dictionaries.c:52,54,155,198-207; zstd-info.c:61)
  * resolves to the zlg_-prefixed export of libzstdlite_gpu.so -- declarations in zstd.h / zdict.h are renamed with the calls, so the
  * sources stay unmodified and the vendored libzstd can stay linked beside it without a symbol clash.
- * oracle/Makefile builds the reference's C layer this way (oracle/_ref/librlayer_gpu.so; tests/test_rlayer.py). */
+ * The package's sources are not part of this repository, so no build here compiles them through this header. */
 #ifndef ZSTDLITE_GPU_MAP_H
 #define ZSTDLITE_GPU_MAP_H
 #define ZSTD_isError                          zlg_ZSTD_isError

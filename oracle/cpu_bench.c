@@ -1,8 +1,8 @@
 /*
  * cpu_bench.c -- TEST / BENCH INFRASTRUCTURE ONLY.  Never linked into the product.
  *
- * Frame-parallel CPU baseline over the reference's own libzstd 1.5.6 (oracle/_ref/libzstd_ref.so,
- * compiled from /root/reference/src/zstd/zstd.c by oracle/Makefile).  No interpreter in the timed
+ * Frame-parallel CPU baseline over the system's libzstd (libzstd.so.1, linked by oracle/Makefile;
+ * the reference vendors the same library at 1.5.6).  No interpreter in the timed
  * region: bench.py hands over packed buffers through ctypes and gets seconds back.
  *
  * Mirrors the reference's call sequences per frame:

@@ -1,6 +1,6 @@
-"""ctypes driver of oracle/_ref/libzl_cpubench.so (oracle/cpu_bench.c).  TEST / BENCH INFRA ONLY.
+"""ctypes driver of oracle/libzl_cpubench.so (oracle/cpu_bench.c).  TEST / BENCH INFRA ONLY.
 
-Times the reference's own libzstd (oracle/_ref/libzstd_ref.so) frame-parallel on the host cores:
+Times the system's libzstd (libzstd.so.1) frame-parallel on the host cores:
 one context per thread, frames pulled from a shared counter, no Python in the timed region.
 Used by bench.py (`cpu_baseline` leg and `--impl reference`) and by nothing in the product.
 """
@@ -11,15 +11,17 @@ import subprocess
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_PATH = os.path.join(_HERE, "_ref", "libzl_cpubench.so")
+_PATH = os.path.join(_HERE, "libzl_cpubench.so")
 _lib = None
 
 
 def lib():
     global _lib
     if _lib is None:
+        from oracle import ref
+        ref.lib()                                      # the harness links the same libzstd.so.1: refuse an unchecked release
         if not os.path.exists(_PATH):
-            subprocess.check_call(["make", "-s", "-C", _HERE, "_ref/libzl_cpubench.so"])
+            subprocess.check_call(["make", "-s", "-C", _HERE, "libzl_cpubench.so"])
         L = C.CDLL(_PATH, mode=os.RTLD_LOCAL)
         vp, sz = C.c_void_p, C.c_size_t
         L.zlb_run.argtypes = [C.c_int, vp, vp, vp, vp, vp, vp, vp, sz, C.c_int, C.c_int, vp, sz, C.c_int]

@@ -1,4 +1,4 @@
-"""-m gpu parity tests for the CUDA decoder: byte-exact against the reference's libzstd (oracle/_ref)
+"""-m gpu parity tests for the CUDA decoder: byte-exact against libzstd (oracle/ref.py)
 and the C restatement, through the C ABI (zl_decompress_batch / ZSTD_decompressDCtx)."""
 import os
 

@@ -1,7 +1,7 @@
 """-m gpu tests of dictionary training on the GPU (SURVEY.md 8f rank 4; csrc/zl_dict_train.cuh), through the C ABI
 (ZDICT_trainFromBuffer / ZDICT_optimizeTrainFromBuffer_cover) and the host mirrors zstd_train_dict_compress / _serialize.
 
-Oracle: the reference's own ZDICT (oracle/_ref).  Bars: (1) the dictionary is a standard Zstandard dictionary that the
+Oracle: libzstd's own ZDICT (oracle/ref.py).  Bars: (1) the dictionary is a standard Zstandard dictionary that the
 reference's libzstd loads, compresses with and decodes with; (2) at the k the reference's fastCOVER search picks, the selected
 CONTENT is identical to the reference's (same dictionary ID = same XXH64 of the content, same trailing bytes); (3) held-out
 objects compress within 5% of the reference pipeline (ZDICT dictionary + libzstd) when the GPU dictionary is used by the GPU

@@ -1,6 +1,6 @@
 """Stage-level differential tests against the reference (SURVEY.md 8c (iii)): the match finder and the entropy stage are compared with
 libzstd's SEPARATELY, through the reference's own experimental sequence API -- ZSTD_generateSequences (src/zstd/zstd.h:1584) and
-ZSTD_compressSequences (src/zstd/zstd.h:1632) of oracle/_ref/libzstd_ref.so -- on one block at a time:
+ZSTD_compressSequences (src/zstd/zstd.h:1632) of libzstd (oracle/ref.py) -- on one block at a time:
 
   * OUR sequences -> THEIR entropy stage: the frame decodes to the input, and our match finder + greedy walk leaves at most a few percent
     more to code than libzstd's fast / double-fast search at the same level (same entropy coder on both sides, so only the parse differs);

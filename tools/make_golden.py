@@ -1,6 +1,6 @@
-"""Regenerates tests/golden/frames.npz from the reference's libzstd (oracle/_ref/libzstd_ref.so).
+"""Regenerates tests/golden/frames.npz from libzstd (oracle/ref.py).  The committed file was made by the reference's
+vendored libzstd 1.5.6; tests/test_oracle.py checks that the libzstd in use still writes the same bytes.
 
-Run in the build container (needs oracle/_ref, i.e. /root/reference at build time):
     python tools/make_golden.py
 Each entry: name -> compressed frame; `<name>.raw` -> expected bytes.  Small on purpose (a few KB each).
 sample_dict.raw is the reference's inst/sample_dict.raw (binary fixture used by R/dictionaries.R:20-24).

@@ -3,13 +3,11 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <new>
-#include <algorithm>
 #include <chrono>
 #include <vector>
 #include <thread>
 #include "../../include/zstdlite_gpu.h"
-#include "zl_host.h"
-#include "zl_plan.h"
+#include "zl_batch_plan.h"            // (and zl_host.h)
 #include "zl_dec_entropy.cuh"     // ZL_HD table builders reused to digest dictionaries on the host (zstd.c:42053)
 
 #define ZL_EXPORT extern "C" __attribute__((visibility("default")))
@@ -355,24 +353,6 @@ ZL_ALIAS(size_t, ZSTD_DCtx_getParameter, (ZSTD_DCtx*, ZSTD_dParameter, int*))
 ZL_ALIAS(size_t, ZSTD_DCtx_loadDictionary, (ZSTD_DCtx*, const void*, size_t))
 
 // ---------------------------------------------------------------------------------------------- batched decode
-// contiguous host ranges of frames [a, b) -> copy runs placed in the device arena from `off` on; returns the end offset
-static size_t zl_build_runs(std::vector<ZlRun>& runs, const void* const* ptr, const size_t* size, size_t a, size_t b, size_t off)
-{
-    const size_t first = runs.size();
-    for (size_t i = a; i < b; i++) {
-        const u8* p = (const u8*)ptr[i];
-        if (runs.size() > first) {
-            ZlRun& r = runs.back();
-            if (p == r.hbase + r.bytes) { r.bytes += size[i]; r.count++; continue; }
-            off = (r.devOff + r.bytes + 255) & ~(size_t)255;
-        }
-        ZlRun r; r.first = i; r.count = 1; r.hbase = p; r.bytes = size[i]; r.devOff = off;
-        runs.push_back(r);
-    }
-    if (runs.size() > first) off = (runs.back().devOff + runs.back().bytes + 255) & ~(size_t)255;
-    return off;
-}
-
 static bool zl_dctx_lanes(ZSTD_DCtx* c)
 {
     if (c->forkEv) return true;
@@ -452,103 +432,21 @@ static size_t zl_decompress_batch_one(ZSTD_DCtx* c, const void* const* src, cons
 static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, const size_t* srcSize, void* const* dst,
                                        const size_t* dstCap, size_t* result, size_t n, int dev, bool worst)
 {
-    if (!c) return ZL_ERROR(GENERIC);
     if (n == 0) return 0;
-    if (n > 0x7FFFFFFFull / 8) return ZL_ERROR(memory_allocation);
+    static const ZlDecTuning tune = {getenv("ZL_DEC_SLICES") ? atoi(getenv("ZL_DEC_SLICES")) : 0, getenv("ZL_DEC_GRADE") ? atoi(getenv("ZL_DEC_GRADE")) : 6,
+                                     getenv("ZL_DEC_NOGRADE") != nullptr, getenv("ZL_DEC_NODEVBUILD") != nullptr, getenv("ZL_DEC_NOSORT") != nullptr,
+                                     getenv("ZL_DEC_NOMID") != nullptr, getenv("ZL_DEC_NOLAZY") != nullptr};      // (development switches)
     const auto hostT0 = std::chrono::steady_clock::now();
     auto hostMs = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - hostT0).count(); };
+    ZlDecPlan p;
+    if (const size_t r = zl_dec_plan(p, src, srcSize, dst, dstCap, n, dev != 0, worst, c->profileStages != 0, tune)) return r;
     if (!zl_ctx_stream(&c->stream, &c->ownStream, &c->ev0, &c->ev1)) return ZL_ERROR(memory_allocation);
     cudaStream_t st = c->stream;
     if (!c->hDescs.reserve(n * sizeof(ZlFrameDesc)) || !c->hResults.reserve(n * 8)) return ZL_ERROR(memory_allocation);
     ZlFrameDesc* hd = c->hDescs.as<ZlFrameDesc>();
-    // ---- slices: contiguous frame ranges of about equal content; one slice when profiling or when the batch is small
-    u64 contentTotal = 0, srcBytes = 0;
-    size_t maxSrc = 1, maxDst = 0;
-    for (size_t i = 0; i < n; i++) {
-        const size_t s = srcSize[i], d = dstCap[i];
-        maxSrc = s > maxSrc ? s : maxSrc; maxDst = d > maxDst ? d : maxDst;
-        contentTotal += d; srcBytes += s;
-    }
-    if (maxSrc > 0xFFFFFFF0ull || maxDst > 0x7FFFFFF0ull) return ZL_ERROR(memory_allocation);
-    size_t nslices = 1;
-    if (!c->profileStages) {
-        // Host buffers: slices overlap the PCIe copies with the kernels.  Device buffers: one slice per internal stream, so that
-        // the three kernels of different slices run side by side (measured on config 2: 1 slice 10.3 ms, 4 or 8 slices 8.8 ms;
-        // more slices than streams only queue behind each other and pay the ~1.5 ms chain latency of a frame again).
-        nslices = dev ? n / ZL_DEC_SLICE_DEV_FRAMES : (size_t)(contentTotal / ZL_DEC_SLICE_BYTES);
-        if (nslices > n / ZL_DEC_SLICE_MIN_FRAMES) nslices = n / ZL_DEC_SLICE_MIN_FRAMES;
-        if (nslices > ZL_DEC_MAX_SLICES) nslices = ZL_DEC_MAX_SLICES;
-        if (nslices < 1) nslices = 1;
-        static const int forceSlices = getenv("ZL_DEC_SLICES") ? atoi(getenv("ZL_DEC_SLICES")) : 0;      // (development switch)
-        if (forceSlices > 0) nslices = (size_t)forceSlices < n ? (size_t)forceSlices : n;
-    }
-    // Host buffers, large batches: the device-to-host copy engine bounds the call, so it must start early and never run dry:
-    // the first slices are small (their kernels end after little more than the chain latency of one frame, ~3 ms) and every
-    // slice is as large as all before it together (1/32, 1/32, 1/16, 1/8, 1/4, 1/2), so the copy back of a slice covers the
-    // kernels of the next.
-    static const bool gradeOff = getenv("ZL_DEC_NOGRADE") != nullptr;      // (development switch)
-    const bool graded = !dev && nslices >= 6 && !gradeOff;
-    static const int gradeN = getenv("ZL_DEC_GRADE") ? atoi(getenv("ZL_DEC_GRADE")) : 6;      // (development switch: 6, 7 or 8 graded slices -- measured the same: 23.4 - 23.7 ms per GiB step;
-    // the floor is the chain latency of ONE frame through the three kernels, 2.4 ms, before the first copy back can start, plus 1.07 GB at the D2H rate)
-    if (graded) nslices = gradeN < 6 ? 6 : (gradeN > ZL_DEC_MAX_SLICES ? ZL_DEC_MAX_SLICES : (size_t)gradeN);
-    if (nslices > 1 && !zl_dctx_lanes(c)) nslices = 1;
-    // Many SMALL frames in device memory (configs[3]: 1e5 objects of a few hundred bytes): the descriptors are built on the device from the
-    // caller's four arrays (zl_k_build_descs) -- the host copies 32 bytes per frame into pinned memory instead of planning and writing an
-    // 80-byte descriptor per frame (~10 ns each: 1.0 ms of a 2.0 ms call whose kernels take 0.8 ms).  Slices are cut by frame count and
-    // their arena shares sized from per-slice sums (upper bounds of the per-frame roundings); the kernel places the frames inside.
-    static const bool devBuildOff = getenv("ZL_DEC_NODEVBUILD") != nullptr;          // (development switch)
-    static_assert(sizeof(size_t) == 8 && sizeof(void*) == 8, "the raw descriptor arrays are copied as u64");
-    const bool devBuild = dev && !devBuildOff && nslices > 1 && n >= 4096 && maxSrc <= 4096 && maxDst <= 2 * ZL_BLOCKSIZE_MAX;
-    // Scheduling order (device buffers): the frames are handed to the kernels by decreasing compressed size -- longest work
-    // first, and frames of one kind next to each other, so that the quads of a warp and the warps of a CTA finish together.
-    // Measured on config 2 with the families interleaved: 112 -> 143 GB/s.  order[pos] = caller's index of the frame at
-    // position `pos`; slices are ranges of positions.  Host buffers keep the caller's order: their slices are contiguous runs
-    // of host memory for the copies, and the end-to-end time is bound by PCIe and the chain latency of one frame, not by
-    // balance (measured: sorting inside the slices 40.3 -> 39.8 GB/s).
-    std::vector<u32> order(n), tmpOrder;
-    for (size_t i = 0; i < n; i++) order[i] = (u32)i;
-    int keyShift = 0;
-    while ((maxSrc >> keyShift) >= 4096) keyShift++;
-    // stable counting sort of order[a, b) by decreasing size class (4,096 classes): O(n), ~50 us for 16,384 frames
-    auto sortRange = [&](size_t a, size_t b) {
-        if (b - a < 2) return;
-        u32 cnt[4097] = {0};
-        for (size_t i = a; i < b; i++) cnt[4095 - (srcSize[order[i]] >> keyShift)]++;
-        u32 run = 0;
-        for (u32 k = 0; k < 4096; k++) { const u32 t = cnt[k]; cnt[k] = run; run += t; }
-        tmpOrder.resize(b - a);
-        for (size_t i = a; i < b; i++) tmpOrder[cnt[4095 - (srcSize[order[i]] >> keyShift)]++] = order[i];
-        std::copy(tmpOrder.begin(), tmpOrder.end(), order.begin() + (ptrdiff_t)a);
-    };
-    static const bool sortOff = getenv("ZL_DEC_NOSORT") != nullptr;               // (development switch)
-    // (batches of small frames -- config 3's objects of a few hundred bytes -- are not sorted: the sort and the scattered access it causes in the
-    //  loops below cost the host 0.5 ms per 1e5 frames, the balance it buys the kernels 0.08 ms)
-    if (dev && !sortOff && maxSrc > 4096) sortRange(0, n);
-    const double tSort = hostMs();
-    std::vector<size_t> cut(nslices + 1, n);
-    if (devBuild) for (size_t k = 0; k <= nslices; k++) cut[k] = n * k / nslices;
-    else {
-        cut[0] = 0;
-        u64 acc = 0; size_t k = 1;
-        for (size_t i = 0; i < n && k < nslices; i++) {
-            acc += dstCap[order[i]];
-            // graded: slice 0 and 1 take 1/2^(S-1) of the batch each, every later slice as much as all before it together
-            const bool reached = graded ? (acc << (nslices - 1)) >= contentTotal * ((u64)1 << (k - 1))
-                                                        : acc * nslices >= contentTotal * k;
-            if (reached) cut[k++] = i + 1;
-        }
-    }
-    std::vector<ZlRun> sruns, druns;
-    std::vector<size_t> srunCut(nslices + 1, 0), drunCut(nslices + 1, 0);
-    size_t srcTotal = 0, dstTotal = 0;
-    if (!dev) {
-        for (size_t k = 0; k < nslices; k++) {
-            srcTotal = zl_build_runs(sruns, src, srcSize, cut[k], cut[k + 1], srcTotal);
-            dstTotal = zl_build_runs(druns, (const void* const*)dst, dstCap, cut[k], cut[k + 1], dstTotal);
-            srunCut[k + 1] = sruns.size(); drunCut[k + 1] = druns.size();
-        }
-        if (!c->dSrc.reserve(srcTotal + 64) || !c->dDst.reserve(dstTotal + 64)) return ZL_ERROR(memory_allocation);
-    }
+    if (p.nslices > 1 && !zl_dctx_lanes(c)) zl_dec_plan(p, src, srcSize, dst, dstCap, n, dev != 0, worst, true, tune);     // no internal streams
+    const size_t nslices = p.nslices;
+    if (!dev && (!c->dSrc.reserve(p.srcTotal + 64) || !c->dDst.reserve(p.dstTotal + 64))) return ZL_ERROR(memory_allocation);
     // Scattered host buffers (a list of separately allocated objects: thousands of copy runs): one cudaMemcpyAsync per run would
     // cost more than the decode (~2.5 us each).  The runs of a slice are then packed into / unpacked from pinned staging
     // buffers by the host, and each slice moves with ONE copy per direction.
@@ -556,108 +454,44 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
     // memory runs through the driver's staging on one thread (config 2: 8.4 GB/s end to end).  Staging is pipelined with the slices:
     // the host packs slice k+1 (zl_host.h, ZlCopyPool) while the device works on slice k, and unpacks slice k while k+1 is in flight.
     // (small pageable calls stay with the driver's path: its staging is fine below a few MiB)
-    const bool stageIn = !dev && (sruns.size() > 64 + 2 * nslices || (srcTotal >= (4u << 20) && zl_is_pageable(sruns[0].hbase)));
-    const bool stageOut = !dev && (druns.size() > 64 + 2 * nslices || (dstTotal >= (4u << 20) && zl_is_pageable(druns[0].hbase)));
+    const bool stageIn = !dev && (p.sruns.size() > 64 + 2 * nslices || (p.srcTotal >= (4u << 20) && zl_is_pageable(p.sruns[0].hbase)));
+    const bool stageOut = !dev && (p.druns.size() > 64 + 2 * nslices || (p.dstTotal >= (4u << 20) && zl_is_pageable(p.druns[0].hbase)));
     ZlStagePool& sp = ZlStagePool::get();
     std::unique_lock<std::mutex> stageLock(sp.m, std::defer_lock);
     if (stageIn || stageOut) stageLock.lock();
-    if (stageIn && !sp.in.reserve(srcTotal + 64)) return ZL_ERROR(memory_allocation);
-    if (stageOut && !sp.out.reserve(dstTotal + 64)) return ZL_ERROR(memory_allocation);
+    if (stageIn && !sp.in.reserve(p.srcTotal + 64)) return ZL_ERROR(memory_allocation);
+    if (stageOut && !sp.out.reserve(p.dstTotal + 64)) return ZL_ERROR(memory_allocation);
     if (stageOut && c->sliceDone.size() < nslices) {
         const size_t have = c->sliceDone.size();
         c->sliceDone.resize(nslices);
         for (size_t k = have; k < nslices; k++) if (cudaEventCreateWithFlags(&c->sliceDone[k], cudaEventDisableTiming) != cudaSuccess) { c->sliceDone.resize(k); return ZL_ERROR(memory_allocation); }
     }
     std::vector<ZlCopySeg> copySegs;
-    std::vector<u32> srunOf, drunOf;                 // copy run of every frame (host buffers), by caller's index
-    if (!dev) {
-        srunOf.resize(n); drunOf.resize(n);
-        size_t sr = 0, dr = 0;
-        for (size_t i = 0; i < n; i++) {
-            while (sr + 1 < sruns.size() && i >= sruns[sr + 1].first) sr++;
-            while (dr + 1 < druns.size() && i >= druns[dr + 1].first) dr++;
-            srunOf[i] = (u32)sr; drunOf[i] = (u32)dr;
-        }
-    }
-    // Descriptors.  Pass 1 only adds up the arenas (and the sums at every slice start); the 80-byte descriptors of a slice are written
-    // and uploaded right before the slice is launched, so that the device starts after 1/8 of the host work and the rest of it
-    // hides behind the kernels (config 3's 1e5 small frames: 8 MB of descriptors, 1.0 of 2.4 ms spent before the first launch).
-    // Batches with large frames (their index is uploaded up front) write everything first, as before.
-    static const bool midOff = getenv("ZL_DEC_NOMID") != nullptr;                 // (development switch)
-    auto isLarge = [&](u32 cap) { return cap >= ZL_LARGE_FRAME_BYTES || (!midOff && n <= 16 && cap > 2 * ZL_BLOCKSIZE_MAX); };
-    struct Sums { u64 lit, rec, hdr, par; };
-    std::vector<Sums> sliceBase(nslices + 1);
-    u64 lit = 0, rec = 0, hdr = 0, par = 0;
-    size_t nLargeTotal = 0;
-    if (devBuild) {
-        for (size_t k = 0; k < nslices; k++) {
-            sliceBase[k] = {lit, rec, hdr, par};
-            u64 S = 0, D = 0;
-            for (size_t i = cut[k]; i < cut[k + 1]; i++) { S += srcSize[i]; D += dstCap[i]; }
-            unsigned long long bl, br, bh;                                     // >= the sums of the frames' litCap (16-aligned), recCap (even) and hdrCap
-            zl_plan_slice_bound(S, D, cut[k + 1] - cut[k], worst, &bl, &br, &bh);
-            hdr += bh; rec += br; lit += bl;
-        }
-        sliceBase[nslices] = {lit, rec, hdr, par};
-    } else {
-        size_t k = 0;
-        for (size_t pos = 0; pos < n; pos++) {
-            while (k < nslices && pos == cut[k]) sliceBase[k++] = {lit, rec, hdr, par};
-            const size_t i = order[pos];
-            u32 litCap, recCap, hdrCap;
-            zl_plan_frame((u32)srcSize[i], (u32)dstCap[i], worst, &litCap, &recCap, &hdrCap);
-            if (isLarge((u32)dstCap[i])) { par += ((u64)dstCap[i] + 3) & ~3ull; nLargeTotal++; }
-            lit += ((u64)litCap + 15) & ~15ull; rec += recCap; hdr += hdrCap;
-        }
-        while (k <= nslices) sliceBase[k++] = {lit, rec, hdr, par};
-    }
-    auto fillDescs = [&](size_t a, size_t b, Sums s) {
-        for (size_t pos = a; pos < b; pos++) {
-            const size_t i = order[pos];
-            ZlFrameDesc& d = hd[pos];
-            if (dev) { d.src = (const u8*)src[i]; d.dst = (u8*)dst[i]; }
-            else {
-                const ZlRun& rs = sruns[srunOf[i]]; const ZlRun& rd = druns[drunOf[i]];
-                d.src = c->dSrc.as<u8>() + rs.devOff + ((const u8*)src[i] - rs.hbase);
-                d.dst = c->dDst.as<u8>() + rd.devOff + ((const u8*)dst[i] - rd.hbase);
-            }
-            d.srcSize = (u32)srcSize[i]; d.dstCap = (u32)dstCap[i];
-            zl_plan_frame(d.srcSize, d.dstCap, worst, &d.litCap, &d.recCap, &d.hdrCap);
-            d.litBase = s.lit; d.recBase = s.rec; d.hdrBase = s.hdr; d.parBase = s.par;
-            // block-parallel execute path (zl_dec_large.cuh): frames of >= 1 MiB, and in batches of a few frames -- where a warp walking
-            // a frame block after block is the whole critical path -- every frame of more than two blocks
-            d.large = isLarge(d.dstCap) ? 1u : 0u;
-            if (d.large) s.par += ((u64)d.dstCap + 3) & ~3ull;
-            s.lit += ((u64)d.litCap + 15) & ~15ull; s.rec += d.recCap; s.hdr += d.hdrCap;
-        }
-    };
-    const double tPass1 = hostMs();
-    static const bool lazyOff = getenv("ZL_DEC_NOLAZY") != nullptr;                // (development switch)
+    const double tPlan = hostMs();
     // (filling the descriptors of >= 32,768 frames with the copy pool's threads was measured and lost: 1e5 small frames 2.94 ms against
     //  2.03 ms slice by slice on this thread -- waking the workers costs more than the 0.5 ms of stores they share)
-    const bool lazyDescs = nLargeTotal == 0 && nslices > 1 && !lazyOff && !devBuild;
-    if (!lazyDescs && !devBuild) fillDescs(0, n, Sums{0, 0, 0, 0});
-    if (devBuild && !c->dRaw.reserve(n * 32)) return ZL_ERROR(memory_allocation);
+    if (!p.lazyDescs && !p.devBuild) zl_plan_fill_descs(p, 0, n, p.base[0], c->dSrc.as<u8>(), c->dDst.as<u8>(), hd);
+    if (p.devBuild && !c->dRaw.reserve(n * 32)) return ZL_ERROR(memory_allocation);
+    const ZlArenaSums& tot = p.base[nslices];
     if (!c->dDescs.reserve(n * sizeof(ZlFrameDesc)) || !c->dInfos.reserve(n * sizeof(ZlFrameInfo)) || !c->dResults.reserve(n * 8) ||
-        !c->dLit.reserve(lit + 64) || !c->dRec.reserve(rec * 8) ||
+        !c->dLit.reserve(tot.lit + 64) || !c->dRec.reserve(tot.rec * 8) ||
         !c->dNorm.reserve(nslices * (size_t)ZL_NORM_SLOTS * 3 * ZL_NORM_STRIDE * sizeof(i16)) ||
-        !c->dHdr.reserve(hdr * sizeof(ZlBlockHdr)) || !c->dUnits.reserve(hdr * sizeof(ZlUnit)) || !c->dCounters.reserve(nslices * 16))
+        !c->dHdr.reserve(tot.hdr * sizeof(ZlBlockHdr)) || !c->dUnits.reserve(tot.hdr * sizeof(ZlUnit)) || !c->dCounters.reserve(nslices * 16))
         return ZL_ERROR(memory_allocation);
-    u32* hLarge = nullptr;
-    if (nLargeTotal) {                          // scratch of the block-parallel path for large frames (zl_dec_large.cuh)
-        if (!c->hLargeIdx.reserve(nLargeTotal * 4) || !c->dLargeIdx.reserve(nLargeTotal * 4) || !c->dLb.reserve(hdr * sizeof(ZlLBlock)) || !c->dLc.reserve(((rec >> ZL_LCHUNK_LOG) + hdr + 2) * sizeof(ZlLChunk)) ||
-            !c->dParent.reserve(par * 4 + 64) || !c->dRemain.reserve(nslices * 64 * sizeof(u32)) || !c->hRemain.reserve(nslices * 64))
+    if (p.nLarge) {                             // scratch of the block-parallel path for large frames (zl_dec_large.cuh)
+        if (!c->hLargeIdx.reserve(p.nLarge * 4) || !c->dLargeIdx.reserve(p.nLarge * 4) || !c->dLb.reserve(tot.hdr * sizeof(ZlLBlock)) ||
+            !c->dLc.reserve(((tot.rec >> ZL_LCHUNK_LOG) + tot.hdr + 2) * sizeof(ZlLChunk)) ||
+            !c->dParent.reserve(tot.par * 4 + 64) || !c->dRemain.reserve(nslices * 64 * sizeof(u32)) || !c->hRemain.reserve(nslices * 64))
             return ZL_ERROR(memory_allocation);
-        hLarge = c->hLargeIdx.as<u32>();
+        u32* hLarge = c->hLargeIdx.as<u32>();
         size_t w = 0;
-        for (size_t k = 0; k < nslices; k++) for (size_t i = cut[k]; i < cut[k + 1]; i++) if (hd[i].large) hLarge[w++] = (u32)(i - cut[k]);
-        cudaMemcpyAsync(c->dLargeIdx.p, hLarge, nLargeTotal * 4, cudaMemcpyHostToDevice, st);
+        for (size_t k = 0; k < nslices; k++) for (size_t i = p.cut[k]; i < p.cut[k + 1]; i++) if (hd[i].large) hLarge[w++] = (u32)(i - p.cut[k]);
+        cudaMemcpyAsync(c->dLargeIdx.p, hLarge, p.nLarge * 4, cudaMemcpyHostToDevice, st);
     }
     size_t largeSeen = 0;
     const double tPrep = hostMs();
-    if (!lazyDescs && !devBuild) cudaMemcpyAsync(c->dDescs.p, hd, n * sizeof(ZlFrameDesc), cudaMemcpyHostToDevice, st);
+    if (!p.lazyDescs && !p.devBuild) cudaMemcpyAsync(c->dDescs.p, hd, n * sizeof(ZlFrameDesc), cudaMemcpyHostToDevice, st);
     if (!c->stageEv[0]) for (cudaEvent_t& e : c->stageEv) cudaEventCreate(&e);
-    const int verify = !c->forceIgnoreChecksum;
     cudaEventRecord(c->ev0, st);
     if (nslices > 1) cudaEventRecord(c->forkEv, st);
     cudaError_t e = cudaSuccess;
@@ -667,7 +501,7 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
     std::vector<cudaEvent_t> tev;
     if (trace) { tev.resize(3 * nslices + 1); for (cudaEvent_t& x : tev) cudaEventCreate(&x); cudaEventRecord(tev[3 * nslices], st); }
     for (size_t k = 0; k < nslices && e == cudaSuccess; k++) {
-        const size_t a = cut[k], cnt = cut[k + 1] - a;
+        const size_t a = p.cut[k], cnt = p.cut[k + 1] - a;
         if (!cnt) continue;
         cudaStream_t ls = nslices > 1 ? c->lane[k % ZL_DEC_LANES] : st;
         if (nslices > 1 && k < ZL_DEC_LANES) cudaStreamWaitEvent(ls, c->forkEv, 0);
@@ -675,45 +509,43 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
             // host-to-device copies in slice order: each waits for the previous slice's (left alone, the copy engine served the
             // streams 0, 4, 1, 5, ...; a dedicated copy stream aliased a hardware queue with a lane and stalled behind its copy back)
             if (nslices > 1 && k > 0) cudaStreamWaitEvent(ls, c->inDone[(k - 1) % ZL_DEC_LANES], 0);
-            if (stageIn) {
-                if (srunCut[k + 1] > srunCut[k]) {
-                    u8* hs = sp.in.as<u8>();
-                    copySegs.clear();
-                    for (size_t r = srunCut[k]; r < srunCut[k + 1]; r++) if (sruns[r].bytes) copySegs.push_back({hs + sruns[r].devOff, sruns[r].hbase, sruns[r].bytes});
-                    ZlCopyPool::get().run(copySegs);                   // (the device is busy with the slices before this one)
-                    const size_t o0 = sruns[srunCut[k]].devOff, o1 = sruns[srunCut[k + 1] - 1].devOff + sruns[srunCut[k + 1] - 1].bytes;
-                    if (o1 > o0) cudaMemcpyAsync(c->dSrc.as<u8>() + o0, hs + o0, o1 - o0, cudaMemcpyHostToDevice, ls);
-                }
-            } else
-            for (size_t r = srunCut[k]; r < srunCut[k + 1]; r++)
-                if (sruns[r].bytes) cudaMemcpyAsync(c->dSrc.as<u8>() + sruns[r].devOff, sruns[r].hbase, sruns[r].bytes, cudaMemcpyHostToDevice, ls);
+            const size_t r0 = p.srunCut[k], r1 = p.srunCut[k + 1];
+            if (stageIn && r1 > r0) {
+                u8* hs = sp.in.as<u8>();
+                copySegs.clear();
+                for (size_t r = r0; r < r1; r++) if (p.sruns[r].bytes) copySegs.push_back({hs + p.sruns[r].devOff, p.sruns[r].hbase, p.sruns[r].bytes});
+                ZlCopyPool::get().run(copySegs);                       // (the device is busy with the slices before this one)
+                const size_t o0 = p.sruns[r0].devOff, o1 = p.sruns[r1 - 1].devOff + p.sruns[r1 - 1].bytes;
+                if (o1 > o0) cudaMemcpyAsync(c->dSrc.as<u8>() + o0, hs + o0, o1 - o0, cudaMemcpyHostToDevice, ls);
+            } else if (!stageIn)
+            for (size_t r = r0; r < r1; r++)
+                if (p.sruns[r].bytes) cudaMemcpyAsync(c->dSrc.as<u8>() + p.sruns[r].devOff, p.sruns[r].hbase, p.sruns[r].bytes, cudaMemcpyHostToDevice, ls);
             if (nslices > 1) cudaEventRecord(c->inDone[k % ZL_DEC_LANES], ls);
         }
-        if (devBuild) {
+        if (p.devBuild) {
+            static_assert(sizeof(size_t) == 8 && sizeof(void*) == 8, "the raw descriptor arrays are copied as u64");
             u64* hraw = reinterpret_cast<u64*>(hd) + 4 * a;                    // (the pinned descriptor buffer holds 80 bytes per frame)
             memcpy(hraw, src + a, cnt * 8); memcpy(hraw + cnt, dst + a, cnt * 8);
             memcpy(hraw + 2 * cnt, srcSize + a, cnt * 8); memcpy(hraw + 3 * cnt, dstCap + a, cnt * 8);
             cudaMemcpyAsync(c->dRaw.as<u64>() + 4 * a, hraw, cnt * 32, cudaMemcpyHostToDevice, ls);
-            e = zl_launch_build_descs(c->dRaw.as<u64>() + 4 * a, (u32)cnt, c->dDescs.as<ZlFrameDesc>() + a, sliceBase[k].lit, sliceBase[k].rec, sliceBase[k].hdr, worst, ls);
+            e = zl_launch_build_descs(c->dRaw.as<u64>() + 4 * a, (u32)cnt, c->dDescs.as<ZlFrameDesc>() + a, p.base[k].lit, p.base[k].rec, p.base[k].hdr, worst, ls);
             c->launches += 1;
             if (e != cudaSuccess) break;
         }
-        if (lazyDescs) {
-            fillDescs(a, a + cnt, sliceBase[k]);
+        if (p.lazyDescs) {
+            zl_plan_fill_descs(p, a, a + cnt, p.base[k], c->dSrc.as<u8>(), c->dDst.as<u8>(), hd);
             cudaMemcpyAsync(c->dDescs.as<ZlFrameDesc>() + a, hd + a, cnt * sizeof(ZlFrameDesc), cudaMemcpyHostToDevice, ls);
         }
         if (trace) cudaEventRecord(tev[3 * k], ls);
-        ZlDecodeLaunch L;
+        ZlDecodeLaunch L{};
         L.descs = c->dDescs.as<ZlFrameDesc>() + a; L.infos = c->dInfos.as<ZlFrameInfo>() + a; L.hdrArena = c->dHdr.as<ZlBlockHdr>();
         L.descsAll = c->dDescs.as<ZlFrameDesc>(); L.infosAll = c->dInfos.as<ZlFrameInfo>(); L.frameBase = (u32)a;
         L.recArena = c->dRec.as<u64>(); L.litArena = c->dLit.as<u8>();
         L.normArena = c->dNorm.as<i16>() + k * (size_t)ZL_NORM_SLOTS * 3 * ZL_NORM_STRIDE; L.normSlots = ZL_NORM_SLOTS;
-        {   const u64 u0 = sliceBase[k].hdr, u1 = sliceBase[k + 1].hdr;                             // the slice's share of the unit arena
+        {   const u64 u0 = p.base[k].hdr, u1 = p.base[k + 1].hdr;                                   // the slice's share of the unit arena
             L.units = c->dUnits.as<ZlUnit>() + u0; L.unitCap = (u32)((u1 - u0) > 0xFFFFFFF0ull ? 0xFFFFFFF0ull : (u1 - u0)); }
         L.counters = c->dCounters.as<u32>() + 4 * k;
-        L.nLarge = 0; L.largeIdx = nullptr; L.largeMaxBlocks = 0; L.largeMaxBytes = 0; L.lbArena = nullptr; L.lcArena = nullptr; L.parentArena = nullptr;
-        L.remain = nullptr; L.remainHost = nullptr;
-        if (nLargeTotal) {
+        if (p.nLarge) {
             L.largeIdx = c->dLargeIdx.as<u32>() + largeSeen;
             for (size_t i = a; i < a + cnt; i++) if (hd[i].large) {
                 L.nLarge++;
@@ -725,7 +557,7 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
             L.remain = c->dRemain.as<u32>() + 64 * k; L.remainHost = c->hRemain.as<u32>() + 16 * k;
         }
         L.results = c->dResults.as<u64>() + a;
-        L.nframes = (u32)cnt; L.verifyChecksum = verify; L.dict = c->hasDict ? c->dDict.as<ZlDictDev>() : nullptr;
+        L.nframes = (u32)cnt; L.verifyChecksum = !c->forceIgnoreChecksum; L.dict = c->hasDict ? c->dDict.as<ZlDictDev>() : nullptr;
         L.stageEv = stageTimed ? c->stageEv : nullptr;
         // host buffers only: literals next to sequences shortens the chain of a slice, i.e. the wait before its copy back can
         // start (measured 39.9 -> 41.4 GB/s end to end); device-resident batches are throughput-bound and lose (143 -> 125 GB/s)
@@ -735,16 +567,17 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
         L.launched = &c->launches;
         e = zl_launch_decode(L, ls);
         if (trace) cudaEventRecord(tev[3 * k + 1], ls);
+        const size_t r0 = p.drunCut[k], r1 = p.drunCut[k + 1];            // (none for device buffers)
         if (!dev && stageOut) {
-            if (drunCut[k + 1] > drunCut[k]) {
-                const size_t o0 = druns[drunCut[k]].devOff, o1 = druns[drunCut[k + 1] - 1].devOff + druns[drunCut[k + 1] - 1].bytes;
+            if (r1 > r0) {
+                const size_t o0 = p.druns[r0].devOff, o1 = p.druns[r1 - 1].devOff + p.druns[r1 - 1].bytes;
                 if (o1 > o0) cudaMemcpyAsync(sp.out.as<u8>() + o0, c->dDst.as<u8>() + o0, o1 - o0, cudaMemcpyDeviceToHost, ls);
             }
             cudaMemcpyAsync(c->hResults.as<u64>() + a, c->dResults.as<u64>() + a, cnt * 8, cudaMemcpyDeviceToHost, ls);
             cudaEventRecord(c->sliceDone[k], ls);
         } else
-        if (!dev) for (size_t r = drunCut[k]; r < drunCut[k + 1]; r++)
-            if (druns[r].bytes) cudaMemcpyAsync((void*)druns[r].hbase, c->dDst.as<u8>() + druns[r].devOff, druns[r].bytes, cudaMemcpyDeviceToHost, ls);
+        for (size_t r = r0; r < r1; r++)
+            if (p.druns[r].bytes) cudaMemcpyAsync((void*)p.druns[r].hbase, c->dDst.as<u8>() + p.druns[r].devOff, p.druns[r].bytes, cudaMemcpyDeviceToHost, ls);
         if (trace) cudaEventRecord(tev[3 * k + 2], ls);
     }
     if (nslices > 1)
@@ -753,25 +586,11 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
     if (e != cudaSuccess) { cudaStreamSynchronize(st); fprintf(stderr, "zstdlite_gpu: kernel launch failed: %s\n", cudaGetErrorString(e)); return ZL_ERROR(GENERIC); }
     const double tLaunch = hostMs();
     if (stageOut && e == cudaSuccess) {
-        // unpack slice after slice as its copy back lands (only what each frame produced), while the later slices are still in flight
-        const u8* ho = sp.out.as<u8>();
-        const u64* hrs = c->hResults.as<u64>();
+        // unpack slice after slice as its copy back lands, while the later slices are still in flight
         for (size_t k = 0; k < nslices; k++) {
-            if (cut[k + 1] == cut[k]) continue;
+            if (p.cut[k + 1] == p.cut[k]) continue;
             if (cudaEventSynchronize(c->sliceDone[k]) != cudaSuccess) break;
-            copySegs.clear();
-            for (size_t r = drunCut[k]; r < drunCut[k + 1]; r++) {
-                const ZlRun& run = druns[r];
-                size_t off = 0, segBeg = 0, segLen = 0;                // frames that filled their slot merge into one copy
-                for (size_t i = run.first; i < run.first + run.count; i++) {
-                    const size_t got = (size_t)hrs[i];
-                    const size_t take = zl_is_error(got) ? 0 : (got < dstCap[i] ? got : dstCap[i]);
-                    if (segLen && segBeg + segLen == off) segLen += take; else { if (segLen) copySegs.push_back({(u8*)run.hbase + segBeg, ho + run.devOff + segBeg, segLen}); segBeg = off; segLen = take; }
-                    if (take != dstCap[i]) { if (segLen) copySegs.push_back({(u8*)run.hbase + segBeg, ho + run.devOff + segBeg, segLen}); segLen = 0; }
-                    off += dstCap[i];
-                }
-                if (segLen) copySegs.push_back({(u8*)run.hbase + segBeg, ho + run.devOff + segBeg, segLen});
-            }
+            zl_plan_unstage(p, k, c->hResults.as<u64>(), sp.out.as<u8>(), copySegs);
             ZlCopyPool::get().run(copySegs);
         }
     }
@@ -784,9 +603,9 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
         for (size_t k = 0; k < nslices; k++) {
             float t0 = 0, t1 = 0, t2 = 0;
             cudaEventElapsedTime(&t0, tev[3 * nslices], tev[3 * k]); cudaEventElapsedTime(&t1, tev[3 * nslices], tev[3 * k + 1]); cudaEventElapsedTime(&t2, tev[3 * nslices], tev[3 * k + 2]);
-            fprintf(stderr, "slice %zu (%zu frames): h2d done %.2f, kernels done %.2f, d2h done %.2f ms\n", k, cut[k + 1] - cut[k], t0, t1, t2);
+            fprintf(stderr, "slice %zu (%zu frames): h2d done %.2f, kernels done %.2f, d2h done %.2f ms\n", k, p.cut[k + 1] - p.cut[k], t0, t1, t2);
         }
-        fprintf(stderr, "total %.2f ms; host: sorted %.3f, arenas summed %.3f, descriptors ready %.3f, launches issued %.3f, synchronised %.3f ms\n", ms, tSort, tPass1, tPrep, tLaunch, tSync);
+        fprintf(stderr, "total %.2f ms; host: planned %.3f, descriptors ready %.3f, launches issued %.3f, synchronised %.3f ms\n", ms, tPlan, tPrep, tLaunch, tSync);
         for (cudaEvent_t x : tev) cudaEventDestroy(x);
     }
     for (int k = 0; k < ZL_DEC_STAGES; k++) {
@@ -795,8 +614,8 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
         c->lastStageMs[k] = t;
     }
     const u64* hr = c->hResults.as<u64>();
-    if (devBuild) memcpy(result, hr, n * 8);                                  // (the caller's order was kept)
-    else for (size_t pos = 0; pos < n; pos++) result[order[pos]] = (size_t)hr[pos];
+    if (p.devBuild) memcpy(result, hr, n * 8);                                // (the caller's order was kept)
+    else for (size_t pos = 0; pos < n; pos++) result[p.order[pos]] = (size_t)hr[pos];
     return 0;
 }
 

@@ -7,7 +7,7 @@
 #include <chrono>
 #include "../../include/zstdlite_gpu.h"
 #include <thread>
-#include "zl_host.h"
+#include "zl_batch_plan.h"      // zl_build_runs
 #include "zl_enc_dict.h"          // host-side dictionary digest (shared with the CPU emulation in tests/emul)
 
 #define ZL_EXPORT extern "C" __attribute__((visibility("default")))
@@ -464,26 +464,18 @@ static size_t zl_compress_batch_one(ZSTD_CCtx* c, const void* const* src, const 
         return 0;
     }
     // host pointers: stage contiguous runs to the device, compress, copy the produced bytes back
-    std::vector<ZlRun> sruns;
-    size_t srcTotal = 0, dstTotal = 0;
-    {   size_t off = 0;
-        for (size_t i = 0; i < n; i++) {
-            const u8* p = (const u8*)src[i];
-            if (!sruns.empty()) { ZlRun& r = sruns.back(); if (p == r.hbase + r.bytes) { r.bytes += srcSize[i]; r.count++; continue; } off = (r.devOff + r.bytes + 255) & ~(size_t)255; }
-            ZlRun r; r.first = i; r.count = 1; r.hbase = p; r.bytes = srcSize[i]; r.devOff = off; sruns.push_back(r);
-        }
-        srcTotal = sruns.back().devOff + sruns.back().bytes;
-    }
+    std::vector<ZlRun> sruns; std::vector<u32> srunOf(n);
+    size_t cut[2] = {0, n}, runCut[2], dstTotal = 0;
+    zl_build_runs(sruns, srunOf.data(), runCut, src, srcSize, cut, 1);
+    const size_t srcTotal = sruns.back().devOff + sruns.back().bytes;
     std::vector<const u8*> dsrc(n); std::vector<u8*> ddst(n);
     for (size_t i = 0; i < n; i++) dstTotal += (dstCap[i] + 15) & ~(size_t)15;
     if (!c->dSrc.reserve(srcTotal + 64) || !c->dDst.reserve(dstTotal + 64)) return ZL_ERROR(memory_allocation);
-    {   size_t sr = 0, doff = 0;
-        for (size_t i = 0; i < n; i++) {
-            while (sr + 1 < sruns.size() && i >= sruns[sr + 1].first) sr++;
-            dsrc[i] = c->dSrc.as<u8>() + sruns[sr].devOff + ((const u8*)src[i] - sruns[sr].hbase);
-            ddst[i] = c->dDst.as<u8>() + doff;
-            doff += (dstCap[i] + 15) & ~(size_t)15;
-        }
+    for (size_t i = 0, doff = 0; i < n; i++) {
+        const ZlRun& r = sruns[srunOf[i]];
+        dsrc[i] = c->dSrc.as<u8>() + r.devOff + ((const u8*)src[i] - r.hbase);
+        ddst[i] = c->dDst.as<u8>() + doff;
+        doff += (dstCap[i] + 15) & ~(size_t)15;
     }
     // scattered inputs (a list of separately allocated objects): packed by the host into pinned staging, ONE copy in; the frames
     // are then gathered on the device, copied back with ONE copy and unpacked by the host (a cudaMemcpyAsync per object costs ~2.5 us)

@@ -66,9 +66,6 @@ struct ZlHostFrameHeader {
 size_t zl_host_frame_header(ZlHostFrameHeader* h, const void* src, size_t srcSize);
 size_t zl_host_find_frame_size(const void* src, size_t srcSize, unsigned* nblocksOut);
 
-// contiguous-run staging between host buffers and a device arena
-struct ZlRun { size_t first, count; const uint8_t* hbase; size_t bytes; size_t devOff; };
-
 // ---- host copy pool ---------------------------------------------------------------------------------------------------
 // The reference's C layer hands over PAGEABLE memory (R vectors: src/raw-file.c:166,189).  cudaMemcpyAsync on such memory goes
 // through the driver's own staging, synchronously and on one thread (measured: 8.4 GB/s for config 2 end to end against 41 GB/s

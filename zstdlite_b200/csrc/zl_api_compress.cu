@@ -1,20 +1,21 @@
 // zl_api_compress.cu -- compression half of the C ABI (include/zstdlite_gpu.h): ZSTD_CCtx lifecycle and parameters
 // (call sites: /root/reference/src/cctx.c:205-312,352-354), ZSTD_compressBound / ZSTD_compress2 (src/raw-file.c:52,74;
-// src/serialize.c:73,91), and the batch / split extensions.  All compute runs in the kernels of zl_enc_kernels.cu.
+// src/serialize.c:73,91), and the batch / split extensions.  All compute runs in the kernels of zl_enc_kernels.cu.  The host arithmetic
+// of a batch (waves, parts, descriptors, placement of host buffers, gather tables, split chunks) is planned in zl_enc_plan.h; this file
+// reserves the buffers and issues the copies and launches the plan describes.
 #include <stdio.h>
 #include <stdlib.h>
 #include <new>
 #include <chrono>
 #include "../../include/zstdlite_gpu.h"
 #include <thread>
-#include "zl_batch_plan.h"      // zl_build_runs
+#include "zl_enc_plan.h"
 #include "zl_enc_dict.h"          // host-side dictionary digest (shared with the CPU emulation in tests/emul)
 
 #define ZL_EXPORT extern "C" __attribute__((visibility("default")))
 #define ZL_ALIAS(ret, name, params) extern "C" __attribute__((visibility("default"), alias(#name))) ret zlg_##name params;
 
 #define ZL_MAX_SERVED_LEVEL 5           // levels 4 and 5: the level-3 engine, within 3 % of libzstd at those levels (ZSTD_c_compressionLevel below)
-#define ZL_WAVE_BLOCKS 8192u          // blocks per launch wave (bounds the scratch arenas: ~0.9 MB per 128 KiB block)
 
 struct ZSTD_CCtx_s {
     int level = 3, nbWorkers = 0, checksumFlag = 0, stableIn = 0, stableOut = 0, windowLog = 0;
@@ -240,109 +241,68 @@ static int zl_engine_level(int level) { return level < 1 ? 1 : (level > 3 ? 3 : 
 // ---- one wave: frames [f0, f1) with DEVICE src/dst pointers; asynchronous on the context's stream.
 // results land in c->dResults[f0..f1).
 static size_t zl_enc_wave(ZSTD_CCtx* c, const u8* const* dsrc, const size_t* srcSize, u8* const* ddst, const size_t* dstCap, size_t f0, size_t f1,
-                          size_t nbTotalFrames, bool timeIt)
+                          size_t nbTotalFrames)
 {
+    static const ZlEncTuning tune = [] {                                  // (development switches)
+        ZlEncTuning t;
+        if (const char* v = getenv("ZL_ENC_HLOG")) t.hlog = sscanf(v, "%u,%u", &t.hlogS, &t.hlogL) == 2;
+        if (const char* v = getenv("ZL_ENC_SIDE")) t.side = atoi(v);
+        if (const char* v = getenv("ZL_ENC_PARTS")) t.parts = atoi(v);
+        t.noFar = getenv("ZL_ENC_NOFAR") != nullptr;
+        return t;
+    }();
     cudaStream_t st = c->stream;
-    const size_t nf = f1 - f0;
     ZlEncParams P = zl_enc_params(zl_engine_level(c->level));
     const ZlEncDictDev* dict = zl_cctx_dict(c, P);
-    if (const char* hl = getenv("ZL_ENC_HLOG")) { unsigned a = 0, b2 = 0; if (sscanf(hl, "%u,%u", &a, &b2) == 2 && !dict) { P.hlogS = a; if (P.hlogL) P.hlogL = b2; } }   // (development: table sizes)
-    if (c->windowLog) P.farMaxOff = c->windowLog <= 17 ? 0u : (c->windowLog >= 24 ? ZL_FAR_MAX_OFF : (1u << c->windowLog));
+    zl_enc_tune_params(P, dict != nullptr, c->windowLog, tune);
     if (c->dictErr && !c->dictRaw.empty()) return c->dictErr;
-    size_t nb = 0; u32 maxBlock = 0;
-    for (size_t i = f0; i < f1; i++) {
-        const size_t s = srcSize[i];
-        nb += s ? (s + ZL_BLOCKSIZE_MAX - 1) / ZL_BLOCKSIZE_MAX : 1;
-        const u32 mb = (u32)(s < ZL_BLOCKSIZE_MAX ? s : ZL_BLOCKSIZE_MAX);
-        if (mb > maxBlock) maxBlock = mb;
-    }
-    if (nb > 0x3FFFFFFFull) return ZL_ERROR(memory_allocation);
-    const u32 S = ((maxBlock < 512 ? 512 : maxBlock) + 255) & ~255u;      // slot layout below needs S >= 264
-    const u32 slotM = S, slotRec = S / 5 + 32, slotLit = S + 16;      // records: ZL_PARSE_WARPS segments of <= ZL_PARSE_SEG_RECS (zl_enc_match.cuh)
-    const u32 streamCapWords = (((S / 4 + 1) * 11) / 8 + 16 + 3) / 4, streamWordsPerBlock = 4 * streamCapWords, seqCapWords = S / 4;
+    ZlEncWave w;
+    if (const size_t e = zl_enc_wave_layout(w, dsrc, srcSize, ddst, dstCap, f0, f1, c->statsDev != nullptr, P, tune)) return e;
+    const size_t nb = w.nb, nf = w.nf;
     if (!c->hBlocks.reserve(nb * sizeof(ZlEncBlock)) || !c->hFrames.reserve(nf * sizeof(ZlEncFrame))) return ZL_ERROR(memory_allocation);
-    if (!c->dBlocks.reserve(nb * sizeof(ZlEncBlock)) || !c->dFrames.reserve(nf * sizeof(ZlEncFrame)) || !c->dM.reserve(nb * (size_t)slotM * 4) ||
-        !c->dRecs.reserve(nb * (size_t)slotRec * 8) || !c->dLit.reserve(nb * (size_t)slotLit) || !c->dHist.reserve(nb * 1024) ||
+    if (!c->dBlocks.reserve(nb * sizeof(ZlEncBlock)) || !c->dFrames.reserve(nf * sizeof(ZlEncFrame)) || !c->dM.reserve(nb * (size_t)w.slotM * 4) ||
+        !c->dRecs.reserve(nb * (size_t)w.slotRec * 8) || !c->dLit.reserve(nb * (size_t)w.slotLit) || !c->dHist.reserve(nb * 1024) ||
         !c->dMetas.reserve(nb * sizeof(ZlEncBlockMeta)) || !c->dOuts.reserve(nb * sizeof(ZlEncBlockOut)) || !c->dPlans.reserve(nb * sizeof(ZlEncBlockPlan)) ||
         !c->dResults.reserve(nbTotalFrames * 8))
         return ZL_ERROR(memory_allocation);
     ZlEncBlock* hb = c->hBlocks.as<ZlEncBlock>();
     ZlEncFrame* hf = c->hFrames.as<ZlEncFrame>();
     if (c->checksumFlag && (!c->hAux.reserve(nf * 16) || !c->dXxhPtrs.reserve(nf * 8) || !c->dXxhSizes.reserve(nf * 4) || !c->dXxh.reserve(nf * 8))) return ZL_ERROR(memory_allocation);
-    static const bool farOff_disabled = getenv("ZL_ENC_NOFAR") != nullptr;      // (development switch)
-    static const int sideMode = getenv("ZL_ENC_SIDE") ? atoi(getenv("ZL_ENC_SIDE")) : 2;       // (development: 0 off, 1 few blocks, 2 always; measured +3..4% on 4,096 blocks, +13% on 128)
-    // A wave of very many one-block frames (configs[3]: 1e5 small objects) is described, uploaded and launched in ZL_ENC_PARTS parts: writing
-    // 1e5 frame and block descriptors takes the host about a millisecond, a quarter of what the device then needs for them -- this way the
-    // device starts after the first part.  The parts use disjoint ranges of every host and device array; stream order keeps them apart.
-    static const int partsEnv = getenv("ZL_ENC_PARTS") ? atoi(getenv("ZL_ENC_PARTS")) : ZL_ENC_PARTS;      // (development switch)
-    const size_t parts = (nb == nf && nf >= 16384 && !c->statsDev && partsEnv > 1) ? (size_t)(partsEnv > ZL_ENC_PARTS ? ZL_ENC_PARTS : partsEnv) : 1;
-    c->waveParts = (int)parts;
-    size_t bi = 0, farEntries = 0;
-    for (size_t part = 0; part < parts; part++) {
-        const size_t fa = nf * part / parts, fb = nf * (part + 1) / parts;      // frames of the part, relative to f0
-        const size_t b0 = bi;                                                  // its first block
-        u32 nSmall = 0;
-        for (size_t r = fa; r < fb; r++) {
-            const size_t i = f0 + r;
-            ZlEncFrame& f = hf[r];
-            memset(&f, 0, sizeof(f));
-            const size_t s = srcSize[i];
-            f.dst = ddst[i]; f.dstCap = dstCap[i]; f.firstBlock = (u32)(bi - b0); f.checksumFlag = (u32)c->checksumFlag;
-            const size_t nblk = s ? (s + ZL_BLOCKSIZE_MAX - 1) / ZL_BLOCKSIZE_MAX : 1;
-            f.nblocks = (u32)nblk;
-            // far candidates (zl_enc_match.cuh): a frame of several blocks gets a frame-wide table, while the wave's tables fit 4 GiB
-            bool far = false;
-            if (nblk > 1 && s < 0xFFFFFF00ull && !farOff_disabled && P.farMaxOff) {
-                const u32 flog = zl_far_log(s);
-                const size_t fe = (size_t)zl_far_entries(s);                  // one table per 8 MiB region
-                if (farEntries + fe <= ((size_t)1 << 30)) { f.pad = (u64)farEntries | ((u64)flog << 56); farEntries += fe; far = true; }
-            }
-            f.hdrSize = zl_write_frame_header(f.hdr, s, dict ? c->dictID : 0u, (u32)c->checksumFlag, far ? P.farMaxOff : 0u);
-            for (size_t k = 0; k < nblk; k++) {
-                ZlEncBlock& b = hb[bi++];
-                b.src = dsrc[i] + k * ZL_BLOCKSIZE_MAX;
-                const size_t rem = s - k * ZL_BLOCKSIZE_MAX;
-                b.srcSize = (u32)(rem < ZL_BLOCKSIZE_MAX ? rem : ZL_BLOCKSIZE_MAX);
-                b.frame = (u32)(r - fa);
-                b.flags = (k == 0 ? ZL_BLK_FIRST : 0u) | (k + 1 == nblk ? ZL_BLK_LAST : 0u);
-                b.pad = (u32)(k * ZL_BLOCKSIZE_MAX);
-                if (b.srcSize && b.srcSize <= ZL_SMALL_BLOCK) nSmall++;
-            }
-        }
-        const size_t pnb = bi - b0, pnf = fb - fa;
-        if (farEntries) {                                             // (only with parts == 1: frames of several blocks)
-            if (!c->dFar.reserve(farEntries * 4)) return ZL_ERROR(memory_allocation);
-            cudaMemsetAsync(c->dFar.p, 0xFF, farEntries * 4, st);
+    const u8** hp = c->checksumFlag ? c->hAux.as<const u8*>() : nullptr;    // XXH64 of every frame's content (zstd.c:27022-27023)
+    u32* hs = c->checksumFlag ? reinterpret_cast<u32*>(hp + nf) : nullptr;
+    c->waveParts = (int)w.parts;
+    for (size_t part = 0; part < w.parts; part++) {
+        const ZlEncPart q = zl_enc_fill_part(w, part, dict ? c->dictID : 0u, (u32)c->checksumFlag, hf, hb, hp, hs);
+        const size_t b0 = q.b0, fa = q.fa, pnb = q.nb, pnf = q.fb - q.fa;
+        if (w.farEntries) {                                           // (only with parts == 1: frames of several blocks)
+            if (!c->dFar.reserve(w.farEntries * 4)) return ZL_ERROR(memory_allocation);
+            cudaMemsetAsync(c->dFar.p, 0xFF, w.farEntries * 4, st);
         }
         cudaMemcpyAsync(c->dBlocks.as<ZlEncBlock>() + b0, hb + b0, pnb * sizeof(ZlEncBlock), cudaMemcpyHostToDevice, st);
         cudaMemcpyAsync(c->dFrames.as<ZlEncFrame>() + fa, hf + fa, pnf * sizeof(ZlEncFrame), cudaMemcpyHostToDevice, st);
         if (c->evDescUp) cudaEventRecord(c->evDescUp, st);
         const u64* xxh = nullptr;
-        if (c->checksumFlag) {                                        // XXH64 of every frame's content (zstd.c:27022-27023)
-            const u8** hp = c->hAux.as<const u8*>();
-            u32* hs = reinterpret_cast<u32*>(hp + nf);
-            bool anyLarge = false;
-            for (size_t r = fa; r < fb; r++) { hp[r] = dsrc[f0 + r]; hs[r] = (u32)srcSize[f0 + r]; if (srcSize[f0 + r] >= ZL_LARGE_FRAME_BYTES) anyLarge = true; }
+        if (c->checksumFlag) {
             cudaMemcpyAsync(c->dXxhPtrs.as<const u8*>() + fa, hp + fa, pnf * 8, cudaMemcpyHostToDevice, st);
             cudaMemcpyAsync(c->dXxhSizes.as<u32>() + fa, hs + fa, pnf * 4, cudaMemcpyHostToDevice, st);
-            if (zl_launch_xxh64(c->dXxhPtrs.as<const u8*>() + fa, c->dXxhSizes.as<u32>() + fa, c->dXxh.as<u64>() + fa, (u32)pnf, st, anyLarge) != cudaSuccess) return ZL_ERROR(GENERIC);
+            if (zl_launch_xxh64(c->dXxhPtrs.as<const u8*>() + fa, c->dXxhSizes.as<u32>() + fa, c->dXxh.as<u64>() + fa, (u32)pnf, st, q.anyLarge) != cudaSuccess) return ZL_ERROR(GENERIC);
             c->launches += 1;
             xxh = c->dXxh.as<u64>() + fa;
         }
         ZlEncodeLaunch L;
         L.blocks = c->dBlocks.as<ZlEncBlock>() + b0; L.nblocks = (u32)pnb; L.frames = c->dFrames.as<ZlEncFrame>() + fa; L.nframes = (u32)pnf;
         L.params = P; L.dict = dict;
-        L.M = c->dM.as<u32>() + b0 * (size_t)slotM; L.slotM = slotM; L.recs = c->dRecs.as<u64>() + b0 * (size_t)slotRec; L.slotRec = slotRec;
-        L.lit = c->dLit.as<u8>() + b0 * (size_t)slotLit; L.slotLit = slotLit;
+        L.M = c->dM.as<u32>() + b0 * (size_t)w.slotM; L.slotM = w.slotM; L.recs = c->dRecs.as<u64>() + b0 * (size_t)w.slotRec; L.slotRec = w.slotRec;
+        L.lit = c->dLit.as<u8>() + b0 * (size_t)w.slotLit; L.slotLit = w.slotLit;
         L.hist = c->dHist.as<u32>() + b0 * 256; L.metas = c->dMetas.as<ZlEncBlockMeta>() + b0; L.outs = c->dOuts.as<ZlEncBlockOut>() + b0;
         L.plans = c->dPlans.as<ZlEncBlockPlan>() + b0;
-        L.streamCapWords = streamCapWords; L.streamWordsPerBlock = streamWordsPerBlock; L.seqCapWords = seqCapWords;
-        L.far = farEntries ? c->dFar.as<u32>() : nullptr;
-        L.nSmall = nSmall;
-        L.results = c->dResults.as<u64>() + f0 + fa; L.xxh = xxh; L.stageEv = timeIt ? c->stageEv[part] : nullptr; L.stats = c->statsDev; L.maxBlock = maxBlock;
-        if (sideMode == 2 || (sideMode == 1 && pnb <= 1024)) { L.side = c->side; L.sideFork = c->sideFork; L.sideJoin = c->sideJoin; }
+        L.streamCapWords = w.streamCapWords; L.streamWordsPerBlock = w.streamWordsPerBlock; L.seqCapWords = w.seqCapWords;
+        L.far = w.farEntries ? c->dFar.as<u32>() : nullptr;
+        L.nSmall = q.nSmall;
+        L.results = c->dResults.as<u64>() + f0 + fa; L.xxh = xxh; L.stageEv = c->stageEv[part]; L.stats = c->statsDev; L.maxBlock = w.maxBlock;
+        if (zl_enc_side(tune, pnb)) { L.side = c->side; L.sideFork = c->sideFork; L.sideJoin = c->sideJoin; }
         cudaError_t e = zl_launch_encode(L, st);
-        c->launches += 6 + (farEntries ? 2 : 0) + ((nSmall && nSmall < pnb) ? 1 : 0);
+        c->launches += 6 + (w.farEntries ? 2 : 0) + ((q.nSmall && q.nSmall < pnb) ? 1 : 0);
         if (e != cudaSuccess) { fprintf(stderr, "zstdlite_gpu: kernel launch failed: %s\n", cudaGetErrorString(e)); return ZL_ERROR(GENERIC); }
     }
     return 0;
@@ -354,31 +314,21 @@ static size_t zl_enc_run(ZSTD_CCtx* c, const u8* const* dsrc, const size_t* srcS
 {
     if (!c->hResults.reserve(n * 8)) return ZL_ERROR(memory_allocation);
     cudaStream_t st = c->stream;
-    for (size_t i = 0; i < n; i++) if (srcSize[i] >= 0xFFFFFFF0ull) return ZL_ERROR(srcSize_wrong);
-    // blocks per wave: the scratch of a block scales with the largest block of the batch (zl_enc_wave), so batches of small
-    // inputs run in far fewer waves (config 4's 1e5 objects: one wave instead of 13, each of which ended in a host sync)
-    size_t maxSrc = 512;
-    for (size_t i = 0; i < n; i++) if (srcSize[i] > maxSrc) maxSrc = srcSize[i];
-    if (maxSrc > ZL_BLOCKSIZE_MAX) maxSrc = ZL_BLOCKSIZE_MAX;
-    size_t waveBlocks = (size_t)ZL_WAVE_BLOCKS * (ZL_BLOCKSIZE_MAX / ((maxSrc + 255) & ~(size_t)255));
-    if (waveBlocks > ((size_t)1 << 20)) waveBlocks = (size_t)1 << 20;
-    size_t f0 = 0;
-    bool firstWave = true;
+    size_t waveBlocks = 0;
+    if (const size_t e = zl_enc_wave_blocks(srcSize, n, &waveBlocks)) return e;
     double total = 0.0; double stage[ZL_ENC_STAGES] = {};
-    while (f0 < n) {
-        size_t f1 = f0, nb = 0;
-        while (f1 < n) {
-            const size_t k = srcSize[f1] ? (srcSize[f1] + ZL_BLOCKSIZE_MAX - 1) / ZL_BLOCKSIZE_MAX : 1;
-            if (f1 > f0 && nb + k > waveBlocks) break;
-            nb += k; f1++;
-        }
-        if (!firstWave) {                                         // the wave's host-side descriptor buffers are reused: drain first
+    auto addTimes = [&]() {                                       // kernel and per-stage times of the wave just finished
+        float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1); total += ms;
+        for (int q = 0; q < c->waveParts; q++) for (int k = 0; k < ZL_ENC_STAGES; k++) { float t = 0; cudaEventElapsedTime(&t, c->stageEv[q][k], c->stageEv[q][k + 1]); stage[k] += t; }
+    };
+    for (size_t f0 = 0; f0 < n;) {
+        const size_t f1 = zl_enc_wave_end(srcSize, n, f0, waveBlocks);
+        if (f0 > 0) {                                             // the wave's host-side descriptor buffers are reused: drain first
             if (cudaStreamSynchronize(st) != cudaSuccess) return ZL_ERROR(GENERIC);
-            float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1); total += ms;
-            for (int q = 0; q < c->waveParts; q++) for (int k = 0; k < ZL_ENC_STAGES; k++) { float t = 0; cudaEventElapsedTime(&t, c->stageEv[q][k], c->stageEv[q][k + 1]); stage[k] += t; }
+            addTimes();
         }
         cudaEventRecord(c->ev0, st);
-        const size_t r = zl_enc_wave(c, dsrc, srcSize, ddst, dstCap, f0, f1, n, true);
+        const size_t r = zl_enc_wave(c, dsrc, srcSize, ddst, dstCap, f0, f1, n);
         cudaEventRecord(c->ev1, st);
         if (c->pendIn.valid) {
             // staging copy of the NEXT chunk (zl_compress_split_pipelined): behind this wave's descriptor uploads -- a copy engine serves its
@@ -390,15 +340,13 @@ static size_t zl_enc_run(ZSTD_CCtx* c, const u8* const* dsrc, const size_t* srcS
             c->pendIn.valid = false;
         }
         if (zl_is_error(r)) { cudaStreamSynchronize(st); return r; }
-        firstWave = false;
         f0 = f1;
     }
     if (zl_launch_results_out(c->dResults.as<u64>(), c->hResults.as<u64>(), (u32)n, st) != cudaSuccess) return ZL_ERROR(GENERIC);
     c->launches += 1;
     const cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) { fprintf(stderr, "zstdlite_gpu: device error: %s\n", cudaGetErrorString(e)); return ZL_ERROR(GENERIC); }
-    float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1); total += ms;
-    for (int q = 0; q < c->waveParts; q++) for (int k = 0; k < ZL_ENC_STAGES; k++) { float t = 0; cudaEventElapsedTime(&t, c->stageEv[q][k], c->stageEv[q][k + 1]); stage[k] += t; }
+    addTimes();
     c->lastKernelMs = total;
     for (int k = 0; k < ZL_ENC_STAGES; k++) c->lastStageMs[k] = stage[k];
     return 0;
@@ -464,57 +412,32 @@ static size_t zl_compress_batch_one(ZSTD_CCtx* c, const void* const* src, const 
         return 0;
     }
     // host pointers: stage contiguous runs to the device, compress, copy the produced bytes back
-    std::vector<ZlRun> sruns; std::vector<u32> srunOf(n);
-    size_t cut[2] = {0, n}, runCut[2], dstTotal = 0;
-    zl_build_runs(sruns, srunOf.data(), runCut, src, srcSize, cut, 1);
-    const size_t srcTotal = sruns.back().devOff + sruns.back().bytes;
+    ZlEncPlace pl;
+    zl_enc_place(pl, src, srcSize, dstCap, n);
+    if (!c->dSrc.reserve(pl.srcTotal + 64) || !c->dDst.reserve(pl.dstTotal + 64)) return ZL_ERROR(memory_allocation);
     std::vector<const u8*> dsrc(n); std::vector<u8*> ddst(n);
-    for (size_t i = 0; i < n; i++) dstTotal += (dstCap[i] + 15) & ~(size_t)15;
-    if (!c->dSrc.reserve(srcTotal + 64) || !c->dDst.reserve(dstTotal + 64)) return ZL_ERROR(memory_allocation);
-    for (size_t i = 0, doff = 0; i < n; i++) {
-        const ZlRun& r = sruns[srunOf[i]];
-        dsrc[i] = c->dSrc.as<u8>() + r.devOff + ((const u8*)src[i] - r.hbase);
-        ddst[i] = c->dDst.as<u8>() + doff;
-        doff += (dstCap[i] + 15) & ~(size_t)15;
-    }
-    // scattered inputs (a list of separately allocated objects): packed by the host into pinned staging, ONE copy in; the frames
-    // are then gathered on the device, copied back with ONE copy and unpacked by the host (a cudaMemcpyAsync per object costs ~2.5 us)
-    // ... and so are PAGEABLE inputs of a few MiB and more (what the reference's C layer passes to ZSTD_compress2: an R vector,
-    // src/raw-file.c:74): the host copy pool (zl_host.h) packs 64 MiB pieces into the process-wide pinned staging while the copy
-    // engine moves the piece before (the driver's own pageable path is one thread, ~8 GB/s)
-    const bool staged = sruns.size() > 64 || n > 256 || (srcTotal >= (4u << 20) && zl_is_pageable(sruns[0].hbase));
+    zl_enc_place_ptrs(pl, src, dstCap, n, c->dSrc.as<u8>(), c->dDst.as<u8>(), dsrc.data(), ddst.data());
+    const bool staged = zl_enc_staged(pl, n, [&] { return zl_is_pageable(pl.runs[0].hbase); });
     ZlStagePool& sp = ZlStagePool::get();
     std::unique_lock<std::mutex> stageLock(sp.m, std::defer_lock);
     if (staged) {
         stageLock.lock();
-        if (!sp.in.reserve(srcTotal + 64)) return ZL_ERROR(memory_allocation);
+        if (!sp.in.reserve(pl.srcTotal + 64)) return ZL_ERROR(memory_allocation);
         u8* hs = sp.in.as<u8>();
-        std::vector<ZlCopySeg> segs;
-        const size_t piece = (size_t)64 << 20;
-        size_t sent = 0;                                               // staging bytes already handed to the copy engine
-        auto flush = [&](size_t upTo) { if (upTo > sent) { ZlCopyPool::get().run(segs); segs.clear(); cudaMemcpyAsync(c->dSrc.as<u8>() + sent, hs + sent, upTo - sent, cudaMemcpyHostToDevice, st); sent = upTo; } };
-        for (const ZlRun& r : sruns) {
-            for (size_t o = 0; o < r.bytes; o += piece) {
-                const size_t len = r.bytes - o < piece ? r.bytes - o : piece;
-                segs.push_back({hs + r.devOff + o, r.hbase + o, len});
-                if (r.devOff + o + len - sent >= piece) flush(r.devOff + o + len);
-            }
+        for (const ZlUpload& u : zl_enc_stage_uploads(pl, hs)) {
+            ZlCopyPool::get().run(u.segs);
+            cudaMemcpyAsync(c->dSrc.as<u8>() + u.from, hs + u.from, u.to - u.from, cudaMemcpyHostToDevice, st);
         }
-        flush(srcTotal);
     } else
-    for (const ZlRun& r : sruns) if (r.bytes) cudaMemcpyAsync(c->dSrc.as<u8>() + r.devOff, r.hbase, r.bytes, cudaMemcpyHostToDevice, st);
+    for (const ZlRun& r : pl.runs) if (r.bytes) cudaMemcpyAsync(c->dSrc.as<u8>() + r.devOff, r.hbase, r.bytes, cudaMemcpyHostToDevice, st);
     const size_t r = zl_enc_run(c, dsrc.data(), srcSize, ddst.data(), dstCap, n);
     if (zl_is_error(r)) return r;
     const u64* hr = c->hResults.as<u64>();
     if (staged) {
         if (!c->hAux.reserve(n * 24) || !c->dAux.reserve(n * 24)) return ZL_ERROR(memory_allocation);
-        u64* hsz = c->hAux.as<u64>(); u64* hoff = hsz + n; const u8** hptr = reinterpret_cast<const u8**>(hoff + n);
-        size_t total = 0;
-        for (size_t i = 0; i < n; i++) {
-            result[i] = (size_t)hr[i];
-            const size_t got = zl_is_error(result[i]) ? 0 : result[i];
-            hsz[i] = got; hoff[i] = total; hptr[i] = ddst[i]; total += got;
-        }
+        u64* hsz = c->hAux.as<u64>();
+        for (size_t i = 0; i < n; i++) result[i] = (size_t)hr[i];
+        const size_t total = zl_enc_gather_table(hsz, hr, ddst.data(), n);
         if (!c->dOutStage.reserve(total + 64) || !sp.out.reserve(total + 64)) return ZL_ERROR(memory_allocation);
         cudaMemcpyAsync(c->dAux.p, hsz, n * 24, cudaMemcpyHostToDevice, st);
         const u64* dsz = c->dAux.as<u64>();
@@ -524,7 +447,7 @@ static size_t zl_compress_batch_one(ZSTD_CCtx* c, const void* const* src, const 
         if (cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
         const u8* ho = sp.out.as<u8>();
         std::vector<ZlCopySeg> osegs;
-        for (size_t i = 0; i < n; i++) if (hsz[i]) osegs.push_back({dst[i], ho + hoff[i], (size_t)hsz[i]});
+        for (size_t i = 0; i < n; i++) if (hsz[i]) osegs.push_back({dst[i], ho + hsz[n + i], (size_t)hsz[i]});
         ZlCopyPool::get().run(osegs);
         return 0;
     }
@@ -595,7 +518,7 @@ static void zl_copy_pieces(void* dst, const void* src, size_t bytes, cudaMemcpyK
         cudaMemcpyAsync((u8*)dst + o, (const u8*)src + o, bytes - o < piece ? bytes - o : piece, kind, s);
 }
 static size_t zl_compress_split_pipelined(ZSTD_CCtx* c, void* dst, size_t dstCap, const u8* src, size_t srcSize, size_t frameSize,
-                                          size_t* frameSizes, size_t nf, size_t slot, size_t chunkFrames)
+                                          size_t* frameSizes, const ZlSplitPlan& sp, size_t slot)
 {
     cudaStream_t st = c->stream;
     if (!c->copyIn) {
@@ -605,58 +528,40 @@ static size_t zl_compress_split_pipelined(ZSTD_CCtx* c, void* dst, size_t dstCap
             if (cudaEventCreateWithFlags(&c->evIn[i], cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&c->evOut[i], cudaEventDisableTiming) != cudaSuccess ||
                 cudaEventCreateWithFlags(&c->evGather[i], cudaEventDisableTiming) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(memory_allocation); }
     }
-    const size_t chunkBytes = chunkFrames * frameSize, inHalf = (chunkBytes + 255) & ~(size_t)255, outHalf = (chunkFrames * slot + 255) & ~(size_t)255;
+    const size_t chunkFrames = sp.chunkFrames, chunkBytes = chunkFrames * frameSize;
+    const size_t inHalf = (chunkBytes + 255) & ~(size_t)255, outHalf = (chunkFrames * slot + 255) & ~(size_t)255;
     if (!c->dSrc.reserve(2 * inHalf + 64) || !c->dDst.reserve(chunkFrames * slot + 64) || !c->dOutStage.reserve(2 * outHalf + 64) ||
         !c->hAux.reserve(chunkFrames * 24) || !c->dAux.reserve(chunkFrames * 24)) return ZL_ERROR(memory_allocation);
-    // chunk sizes grow 1/8, 1/4, 1/2, 1, 1, ... of a full chunk: the first staging copy, which nothing can overlap, is short
-    // (shrinking them again towards the end, for a short last copy back, was measured: the same 143 ms per 4 GiB -- small chunks compress less
-    //  efficiently, which eats what the shorter tail saves)
-    std::vector<size_t> cstart;
-    for (size_t f = 0, sz = chunkFrames / 8 ? chunkFrames / 8 : 1; f < nf; f += sz, sz = sz * 2 < chunkFrames ? sz * 2 : chunkFrames) cstart.push_back(f);
-    cstart.push_back(nf);
-    const size_t nchunks = cstart.size() - 1;
+    const size_t nchunks = sp.cstart.size() - 1;
     std::vector<const u8*> dsrc(chunkFrames); std::vector<u8*> ddst(chunkFrames); std::vector<size_t> ssz(chunkFrames), caps(chunkFrames, slot);
-    auto chunkRange = [&](size_t k, size_t* f0, size_t* bytes) {
-        *f0 = cstart[k];
-        const size_t b0 = cstart[k] * frameSize, b1 = cstart[k + 1] * frameSize < srcSize ? cstart[k + 1] * frameSize : srcSize;
-        *bytes = b1 - b0;
-    };
+    auto chunkBytesOf = [&](size_t k) { return std::min(sp.cstart[k + 1] * frameSize, srcSize) - sp.cstart[k] * frameSize; };
     size_t total = 0, err = 0;
     static const bool trace = getenv("ZL_ENC_TRACE") != nullptr;      // (development: host timeline of the chunks on stderr)
     const auto t00 = std::chrono::steady_clock::now();
     auto nowMs = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t00).count(); };
-    {   size_t f0, bytes; chunkRange(0, &f0, &bytes);
-        zl_copy_pieces(c->dSrc.p, src, bytes, cudaMemcpyHostToDevice, c->copyIn); cudaEventRecord(c->evIn[0], c->copyIn); }
+    zl_copy_pieces(c->dSrc.p, src, chunkBytesOf(0), cudaMemcpyHostToDevice, c->copyIn);
+    cudaEventRecord(c->evIn[0], c->copyIn);
     for (size_t k = 0; k < nchunks && !err; k++) {
-        size_t f0, bytes; chunkRange(k, &f0, &bytes);
-        const size_t cnt = cstart[k + 1] - f0;
-        u8* inBase = c->dSrc.as<u8>() + (k & 1) * inHalf;
+        const size_t f0 = sp.cstart[k], cnt = sp.cstart[k + 1] - f0;
         if (k + 1 < nchunks) {                                   // next chunk's input (its half was last read by chunk k-1, finished)
-            size_t g0, gbytes; chunkRange(k + 1, &g0, &gbytes);
-            c->pendIn.valid = true; c->pendIn.dst = c->dSrc.as<u8>() + ((k + 1) & 1) * inHalf; c->pendIn.src = src + g0 * frameSize;
-            c->pendIn.bytes = gbytes; c->pendIn.slot = (int)((k + 1) & 1);
+            c->pendIn.valid = true; c->pendIn.dst = c->dSrc.as<u8>() + ((k + 1) & 1) * inHalf; c->pendIn.src = src + sp.cstart[k + 1] * frameSize;
+            c->pendIn.bytes = chunkBytesOf(k + 1); c->pendIn.slot = (int)((k + 1) & 1);
         }
         cudaStreamWaitEvent(st, c->evIn[k & 1], 0);
-        for (size_t i = 0; i < cnt; i++) {
-            dsrc[i] = inBase + i * frameSize;
-            const size_t rem = bytes - i * frameSize;
-            ssz[i] = rem < frameSize ? rem : frameSize;
-            ddst[i] = c->dDst.as<u8>() + i * slot;
-        }
+        zl_enc_split_frames(c->dSrc.as<u8>() + (k & 1) * inHalf, chunkBytesOf(k), frameSize, c->dDst.as<u8>(), slot, cnt, dsrc.data(), ssz.data(), ddst.data());
         const double tA = nowMs();
         const size_t r = zl_enc_run(c, dsrc.data(), ssz.data(), ddst.data(), caps.data(), cnt);
         if (zl_is_error(r)) { err = r; break; }
         if (trace) fprintf(stderr, "chunk %zu: compress call %.1f -> %.1f ms (kernels %.1f ms: match %.1f parse %.1f literals %.1f sequences %.1f assemble %.1f)\n", k, tA, nowMs(),
                            c->lastKernelMs, c->lastStageMs[0], c->lastStageMs[1], c->lastStageMs[2], c->lastStageMs[3], c->lastStageMs[4]);
         const u64* hr = c->hResults.as<u64>();
-        u64* hsz = c->hAux.as<u64>(); u64* hoff = hsz + cnt; const u8** hptr = reinterpret_cast<const u8**>(hoff + cnt);
-        size_t ctotal = 0;
-        for (size_t i = 0; i < cnt; i++) {
-            if (zl_is_error((size_t)hr[i])) { err = (size_t)hr[i]; break; }
-            hsz[i] = hr[i]; hoff[i] = ctotal; hptr[i] = ddst[i]; ctotal += (size_t)hr[i];
-            if (frameSizes) frameSizes[f0 + i] = (size_t)hr[i];
+        for (size_t i = 0; i < cnt && !err; i++) {
+            if (zl_is_error((size_t)hr[i])) err = (size_t)hr[i];
+            else if (frameSizes) frameSizes[f0 + i] = (size_t)hr[i];
         }
         if (err) break;
+        u64* hsz = c->hAux.as<u64>();
+        const size_t ctotal = zl_enc_gather_table(hsz, hr, ddst.data(), cnt);
         if (total + ctotal > dstCap) { err = ZL_ERROR(dstSize_tooSmall); break; }
         // the gather reads its sizes / offsets / pointers straight from the pinned (device-mapped) host array: as a cudaMemcpyAsync these
         // 24 bytes per frame queued up behind the NEXT chunk's input on the host-to-device copy engine (measured: 1.3 and 4.2 ms of idle
@@ -691,15 +596,10 @@ ZL_EXPORT size_t zl_compress_split(ZSTD_CCtx* c, void* dst, size_t dstCap, const
     if (!guard.ok) return ZL_ERROR(GENERIC);
     if (!zl_cctx_ready(c)) return ZL_ERROR(memory_allocation);
     cudaStream_t st = c->stream;
-    const size_t nf = srcSize ? (srcSize + frameSize - 1) / frameSize : 1;
+    const ZlSplitPlan sp = zl_enc_split_plan(srcSize, frameSize, dev != 0);
+    const size_t nf = sp.nf;
     const size_t slot = (ZSTD_compressBound(frameSize) + 4 + 15) & ~(size_t)15;
-    {   // host buffers of >= 2 chunks of ~1 GiB (at most ZL_WAVE_BLOCKS blocks each): the pipelined path
-        const size_t blocksPerFrame = (frameSize + ZL_BLOCKSIZE_MAX - 1) / ZL_BLOCKSIZE_MAX;
-        size_t chunkFrames = ZL_WAVE_BLOCKS / blocksPerFrame;
-        if (chunkFrames * frameSize > ((size_t)1 << 30)) chunkFrames = ((size_t)1 << 30) / frameSize;
-        if (!dev && chunkFrames >= 1 && nf >= 2 * chunkFrames && chunkFrames * frameSize >= ((size_t)64 << 20))
-            return zl_compress_split_pipelined(c, dst, dstCap, (const u8*)src, srcSize, frameSize, frameSizes, nf, slot, chunkFrames);
-    }
+    if (sp.pipelined) return zl_compress_split_pipelined(c, dst, dstCap, (const u8*)src, srcSize, frameSize, frameSizes, sp, slot);
     const u8* dsrcBase = (const u8*)src;
     if (!dev) {
         if (!c->dSrc.reserve(srcSize + 64)) return ZL_ERROR(memory_allocation);
@@ -708,24 +608,18 @@ ZL_EXPORT size_t zl_compress_split(ZSTD_CCtx* c, void* dst, size_t dstCap, const
     }
     if (!c->dDst.reserve(nf * slot + 64)) return ZL_ERROR(memory_allocation);
     std::vector<const u8*> dsrc(nf); std::vector<u8*> ddst(nf); std::vector<size_t> ssz(nf), caps(nf, slot);
-    for (size_t i = 0; i < nf; i++) {
-        dsrc[i] = dsrcBase + i * frameSize;
-        const size_t rem = srcSize - i * frameSize;
-        ssz[i] = rem < frameSize ? rem : frameSize;
-        ddst[i] = c->dDst.as<u8>() + i * slot;
-    }
+    zl_enc_split_frames(dsrcBase, srcSize, frameSize, c->dDst.as<u8>(), slot, nf, dsrc.data(), ssz.data(), ddst.data());
     const size_t r = zl_enc_run(c, dsrc.data(), ssz.data(), ddst.data(), caps.data(), nf);
     if (zl_is_error(r)) return r;
     const u64* hr = c->hResults.as<u64>();
     // exclusive scan of the frame sizes (host: nf integers), then one gather launch
     if (!c->hAux.reserve(nf * 24) || !c->dAux.reserve(nf * 24)) return ZL_ERROR(memory_allocation);
-    u64* hsz = c->hAux.as<u64>(); u64* hoff = hsz + nf; const u8** hptr = reinterpret_cast<const u8**>(hoff + nf);
-    size_t total = 0;
     for (size_t i = 0; i < nf; i++) {
         if (zl_is_error((size_t)hr[i])) return (size_t)hr[i];
-        hsz[i] = hr[i]; hoff[i] = total; hptr[i] = ddst[i]; total += (size_t)hr[i];
         if (frameSizes) frameSizes[i] = (size_t)hr[i];
     }
+    u64* hsz = c->hAux.as<u64>();
+    const size_t total = zl_enc_gather_table(hsz, hr, ddst.data(), nf);
     if (total > dstCap) return ZL_ERROR(dstSize_tooSmall);
     cudaMemcpyAsync(c->dAux.p, hsz, nf * 24, cudaMemcpyHostToDevice, st);
     u8* out = (u8*)dst;

@@ -483,6 +483,7 @@ ZL_HD void zl_huf_fill(ZlLitSm& f, u32 q)
     }
 }
 
+#define ZL_NO_RING 0xFFFFFFFFu       // `ring` argument of the decoders: no stream ring (the CPU emulation)
 #if defined(__CUDACC__)
 // ---- device-only fast paths: branch-free refills (predicated PTX loads write straight into the look-ahead register,
 // so the load stays in flight until the next refill), shared-space table loads, rotated loops. ------------------------
@@ -510,62 +511,59 @@ __device__ __forceinline__ u32 zl_lds16(u32 a) { u32 v; asm("ld.shared.u16 %0, [
         n += (i32)(need_ << 5);                                                                                \
         wi -= (i32)need_;                                                                                      \
     }
-// ---- stream ring: the lane's next words come from shared memory, filled by cp.async in 16-byte chunks --------------------
-// `ring` = shared-space address of the lane's 16-byte column; slot k of the ring lies at ring + (k << SH); NS slots (4 or 8).
-// Word indices are relative to the 16-byte aligned `wb16`; `clow` = chunk holding the first byte of the stream (nothing below
-// it is read).  zl_ring_start fetches chunks c0 .. c0-(NS-1) (slot = chunk & (NS-1)); later, entering chunk c fetches chunk
-// c-(NS-1) into the slot chunk c+1 has just left.
+// ---- stream ring: the 64-bit reader of the fast loops ------------------------------------------------------------------------
+// A lane's ring is NS 16-byte slots, contiguous in shared memory at `ring` (aligned to 16 NS): chunk c of the stream (the 16 bytes at
+// wb16 + 16 c, `wb16` = the frame's src rounded down to 16 bytes) lives in slot c & (NS-1), so stream word w is at
+// ring | (4 w & (16 NS - 4)).  The reader keeps one number, `pos`: the stream bits below the next unread one, counted from wb16.
+// A reload takes the three words that hold the 64 bits below pos and funnel-shifts them into (hi:lo), the next bit to consume being
+// the MSB of hi: after every reload all 64 bits are valid, whatever pos is (the byte-granular container of BIT_reloadDStream keeps
+// >= 57).  Chunks are copied by cp.async: when pos enters chunk X, chunk X-(NS-1) is fetched into the slot chunk X+1 has left, never
+// below `clow`, the chunk that holds the stream's first byte (bits read below the start reach only a stream that runs past its
+// start, which the exact count in pos rejects).  A reload moves pos by less than 128 bits, so it issues at most one copy.
+#define ZL_LIT_RING_NS 8          // literal lanes: 128 bytes each, 4 KB per warp
+#define ZL_SEQ_RING_NS 4          // sequence units: 64 bytes each, 1 KB per warp
+__device__ __forceinline__ u32 zl_ring_lds(u32 a) { u32 v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
+// chunks c0 .. c0-(NS-1) below the unread bit, c0 = (pos - 1) >> 7; slots under the start get chunk clow (never read for a valid stream)
 template <int NS>
-__device__ __forceinline__ void zl_ring_start(u32 ring, u32 sh, const u32* wb16, i32 wi, i32 clow)
+__device__ __forceinline__ void zl_ring_start(u32 ring, const u32* wb16, i32 pos, i32 clow)
 {
-    const i32 c0 = wi >> 2;
+    const i32 c0 = (pos - 1) >> 7;
 #pragma unroll
     for (i32 k = 0; k < NS; k++) {
         const i32 c = (c0 - k) < clow ? clow : (c0 - k);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(ring + (((u32)(c0 - k) & (u32)(NS - 1)) << sh)), "l"(wb16 + 4 * c) : "memory");
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(ring | (((u32)(c0 - k) & (u32)(NS - 1)) << 4)), "l"(wb16 + 4 * c) : "memory");
     }
     asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
 }
-// One refill.  SYNC = the commit / wait_group text: with a group per refill a chunk is first read 4 (NS-1) refills after its
-// copy was issued, so "wait_group N" with N < 4 (NS-1) always covers it while the warp only waits for copies N+1 refills old.
-// PF = 1 adds an L2 prefetch 256 bytes further down the stream (needed with 4 slots: 9 refills do not cover DRAM latency).
-#define ZL_REFILL_RING_(SH, NS, PF, SYNC)                                                                      \
-    {                                                                                                          \
-        const u32 need_ = (n <= 32) ? 1u : 0u;                                                                 \
-        hi |= zl_shr(nextw, (u32)n);                                                                           \
-        lo |= zl_shl(nextw, 32u - (u32)n);                                                                     \
-        const i32 c_ = (wi >> 2) - ((NS) - 1);                                                                 \
-        const i32 cl_ = c_ < clow ? clow : c_;                                                                 \
-        const i32 pf_ = (PF) ? ((c_ - 16) < clow ? clow : (c_ - 16)) : cl_;                                    \
-        const u32 cross_ = need_ & (((u32)wi & 3u) == 3u ? 1u : 0u);                                           \
-        const u32 pfneed_ = (PF) ? (cross_ & (((u32)c_ & 1u) ? 0u : 1u)) : 0u;                                 \
-        asm volatile("{\n\t.reg .pred p, q, r;\n\tsetp.ne.u32 p, %5, 0;\n\tsetp.ne.u32 q, %6, 0;\n\tsetp.ne.u32 r, %7, 0;\n\t" \
-                     "@q cp.async.cg.shared.global [%1], [%2], 16;\n\t@r prefetch.global.L2 [%3];\n\t"        \
-                     SYNC "@p ld.shared.u32 %0, [%4];\n\t}"                                                   \
-                     : "+r"(nextw)                                                                             \
-                     : "r"(ring + (((u32)c_ & (u32)((NS) - 1)) << (SH))), "l"(wb16 + 4 * cl_), "l"(wb16 + 4 * pf_), \
-                       "r"(ring + ((((u32)wi >> 2) & (u32)((NS) - 1)) << (SH)) + (((u32)wi & 3u) << 2)), "r"(need_), "r"(cross_), "r"(pfneed_) \
-                     : "memory");                                                                              \
-        n += (i32)(need_ << 5);                                                                                \
-        wi -= (i32)need_;                                                                                      \
+// Reload (hi:lo) at `pos`; `prev` = pos at the previous reload, `gb` = wb16 - 16 (NS-1), `cmin` = clow + NS-1.  SYNC = the
+// commit / wait text placed between the copy and the word loads.
+#define ZL_RING_RELOAD(NS, SYNC, ring, gb, cmin, pos, prev, hi, lo)                                                    \
+    {                                                                                                                  \
+        const i32 x_ = (pos) >> 7;                                                                                     \
+        const u32 t_ = (u32)(pos) >> 3;                                                                                \
+        const u32 need_ = ((u32)((pos) ^ (prev)) > 127u && x_ >= (cmin)) ? 1u : 0u;                                  \
+        asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %2, 0;\n\t@p cp.async.cg.shared.global [%0], [%1], 16;\n\t" SYNC "}" \
+                     ::"r"(((t_ + 16u) & (16u * ((NS) - 1))) | (ring)), "l"((gb) + (i64)x_ * 16), "r"(need_) : "memory"); \
+        const u32 w0_ = zl_ring_lds((t_ & (16u * (NS) - 4u)) | (ring));                                               \
+        const u32 w1_ = zl_ring_lds(((t_ - 4u) & (16u * (NS) - 4u)) | (ring));                                        \
+        const u32 w2_ = zl_ring_lds(((t_ - 8u) & (16u * (NS) - 4u)) | (ring));                                        \
+        hi = __funnelshift_r(w1_, w0_, (u32)(pos));                                                                    \
+        lo = __funnelshift_r(w2_, w1_, (u32)(pos));                                                                    \
     }
-#ifndef ZL_LIT_RING_SLOTS
-#define ZL_LIT_RING_SLOTS 8
-#endif
-#ifndef ZL_LIT_RING_SYNC
-#define ZL_LIT_RING_SYNC 2          // one group per four symbols (two refills); 1: one per refill (literals 1.13 -> 1.11 ms with 2)
-#endif
-#if ZL_LIT_RING_SLOTS == 8 && ZL_LIT_RING_SYNC == 2
-#define ZL_REFILL_RING_LIT() ZL_REFILL_RING_(9, 8, 0, "cp.async.commit_group;\n\tcp.async.wait_group 10;\n\t")
-#define ZL_REFILL_RING_LIT2() ZL_REFILL_RING_(9, 8, 0, "")
-#elif ZL_LIT_RING_SLOTS == 8
-#define ZL_REFILL_RING_LIT() ZL_REFILL_RING_(9, 8, 0, "cp.async.commit_group;\n\tcp.async.wait_group 20;\n\t")
-#else
-#define ZL_REFILL_RING_LIT() ZL_REFILL_RING_(9, 4, 1, "cp.async.commit_group;\n\tcp.async.wait_group 8;\n\t")
-#endif
-#ifndef ZL_REFILL_RING_LIT2
-#define ZL_REFILL_RING_LIT2() ZL_REFILL_RING_LIT()
-#endif
+// hand-off to the generic reader: n = 32 + (pos & 31) bits in (hi:lo), the word below them in `nextw`
+template <int NS>
+__device__ __forceinline__ void zl_ring_to_br(ZlBitR& b, u32 ring, i32 pos, i32 s16)
+{
+    asm volatile("cp.async.wait_all;" ::: "memory");
+    const u32 t = (u32)pos >> 3, r = (u32)pos & 31u;
+    const u32 w0 = zl_ring_lds((t & (16u * NS - 4u)) | ring), w1 = zl_ring_lds(((t - 4u) & (16u * NS - 4u)) | ring),
+              w2 = zl_ring_lds(((t - 8u) & (16u * NS - 4u)) | ring);
+    b.hi = __funnelshift_r(w1, w0, r);
+    b.lo = zl_shl(w1, 32u - r);
+    b.n = 32 + (i32)r;
+    b.nextw = w2;
+    b.wi = (pos >> 5) - 3 - s16;
+}
 __device__ __forceinline__ u32 zl_selp(u32 a, u32 b, bool c)          // c ? a : b, guaranteed to stay a select
 {
     u32 r;
@@ -577,11 +575,11 @@ __device__ __forceinline__ u32 zl_opaque(u32 x) { asm volatile("" : "+r"(x)); re
 
 // one Huffman stream per lane: zstd.c:38626-38650.  Returns 0 when the stream ends exactly, 2 when bits are left over,
 // 1 when the reader ran past the start (or the end mark is missing).
-// `ring` (device only; 0 = none): shared-space address of this lane's 16-byte column of the warp's stream ring (4 slots of
-// 32 x 16 bytes).  With a ring the stream words reach the lane through cp.async (16-byte chunk three chunks ahead of the
-// one being consumed) and an LDS, instead of a global load per word: the per-warp scoreboard made every refill wait for
-// the global load some other lane had issued one refill earlier (ncu: long scoreboard 6.5 of 10 cycles per issue).
-ZL_HD u32 zl_huf_stream(const u16* huf, u32 tlog, const u32* wbase, u32 bias, u32 beg, u32 end, u8* out, u32 n, u32 ring = 0)
+// `ring` (device only; ZL_NO_RING = none): shared-space address of this lane's ring (ZL_LIT_RING_NS slots).  With a ring the
+// stream reaches the lane through cp.async and LDS instead of a global load per word: the per-warp scoreboard made every refill
+// wait for the global load some other lane had issued one refill earlier (ncu: long scoreboard 6.5 of 10 cycles per issue).
+// The ring loop decodes 20 symbols per iteration, five per reload (5 x 11 bits <= 64), and stores them as five aligned words.
+ZL_HD u32 zl_huf_stream(const u16* huf, u32 tlog, const u32* wbase, u32 bias, u32 beg, u32 end, u8* out, u32 n, u32 ring = ZL_NO_RING)
 {
     ZlBitR b;
     if (!zl_br_init(b, wbase, bias, beg, end)) return 1;
@@ -590,31 +588,46 @@ ZL_HD u32 zl_huf_stream(const u16* huf, u32 tlog, const u32* wbase, u32 bias, u3
 #define ZL_HUF_SYM(dst) { const u32 e = huf[b.hi >> sh]; zl_br_skip(b, e >> 8); dst = e & 0xFF; }
     while (i < n && (((size_t)(out + i)) & 3)) { u32 s; zl_br_refill(b, wbase); ZL_HUF_SYM(s); out[i++] = (u8)s; }
 #if defined(__CUDA_ARCH__)
-    if (ring) {
-        const u32 count = n;                       // `n` below is the window's valid-bit count (macro convention)
-        u32 hi = b.hi, lo = b.lo, nextw = b.nextw;
-        const u32 s16 = (u32)(((size_t)wbase >> 2) & 3);
-        const u32* wb16 = wbase - s16;             // 16-byte aligned; word indices below are relative to it
-        i32 wi = b.wi + (i32)s16;
-        const i32 clow = (b.wlow + (i32)s16) >> 2; // chunk holding the first byte of the stream (never read below it)
-        const u32 th = zl_smem_addr(huf);
-        zl_ring_start<ZL_LIT_RING_SLOTS>(ring, 9, wb16, wi, clow);
-        {
-            i32 n = b.n;
-#define ZL_HUF_SYM_DEV(dst) { const u32 e = zl_lds16(th + ((hi >> sh) << 1)); const u32 nb = e >> 8; \
-                              hi = zl_fsl(lo, hi, nb); lo <<= nb; n -= (i32)nb; dst = e & 0xFF; }
-            while (i + 4 <= count) {
-                u32 s0, s1, s2, s3;
-                ZL_REFILL_RING_LIT(); ZL_HUF_SYM_DEV(s0); ZL_HUF_SYM_DEV(s1);
-                ZL_REFILL_RING_LIT2(); ZL_HUF_SYM_DEV(s2); ZL_HUF_SYM_DEV(s3);
-                __stcs((u32*)(out + i), s0 | (s1 << 8) | (s2 << 16) | (s3 << 24));
-                i += 4;
+    if (ring != ZL_NO_RING) {
+        if (i + 20 <= n) {
+            const i32 s16 = (i32)(((size_t)wbase >> 2) & 3);
+            const u32* wb16 = wbase - s16;                             // 16-byte aligned; positions below are relative to it
+            const i32 clow = (b.wlow + s16) >> 2;                      // chunk holding the first byte of the stream
+            const u8* gb = reinterpret_cast<const u8*>(wb16) - 16 * (ZL_LIT_RING_NS - 1);
+            const i32 cmin = clow + (ZL_LIT_RING_NS - 1);
+            const u32 th = zl_smem_addr(huf);
+            i32 pos = 32 * (b.wi + 2 + s16) + b.n, prev = pos;
+            zl_ring_start<ZL_LIT_RING_NS>(ring, wb16, pos, clow);
+            // a chunk is first read >= 13 reloads after its copy (7 chunks of lead, <= 55 bits per reload), so one group per
+            // iteration and "wait_group 2" always cover it
+#define ZL_HUF_SYM5(e0, e1, e2, e3, e4)                                                                                     \
+            {                                                                                                               \
+                u32 hi, lo;                                                                                                 \
+                ZL_RING_RELOAD(ZL_LIT_RING_NS, "", ring, gb, cmin, pos, prev, hi, lo);                                      \
+                prev = pos;                                                                                                 \
+                e0 = zl_lds16(th + ((hi >> sh) << 1)); hi = __funnelshift_l(lo, hi, e0 >> 8); lo <<= e0 >> 8;              \
+                e1 = zl_lds16(th + ((hi >> sh) << 1)); hi = __funnelshift_l(lo, hi, e1 >> 8); lo <<= e1 >> 8;              \
+                e2 = zl_lds16(th + ((hi >> sh) << 1)); hi = __funnelshift_l(lo, hi, e2 >> 8); lo <<= e2 >> 8;              \
+                e3 = zl_lds16(th + ((hi >> sh) << 1)); hi = __funnelshift_l(lo, hi, e3 >> 8);                              \
+                e4 = zl_lds16(th + ((hi >> sh) << 1));                                                                      \
+                pos -= (i32)((e0 >> 8) + (e1 >> 8) + (e2 >> 8) + (e3 >> 8) + (e4 >> 8));                                   \
             }
-#undef ZL_HUF_SYM_DEV
-            asm volatile("cp.async.wait_all;" ::: "memory");
-            b.n = n;
+            do {
+                u32 e[20];
+                asm volatile("cp.async.wait_group 2;" ::: "memory");
+                ZL_HUF_SYM5(e[0], e[1], e[2], e[3], e[4]);
+                ZL_HUF_SYM5(e[5], e[6], e[7], e[8], e[9]);
+                ZL_HUF_SYM5(e[10], e[11], e[12], e[13], e[14]);
+                ZL_HUF_SYM5(e[15], e[16], e[17], e[18], e[19]);
+                asm volatile("cp.async.commit_group;" ::: "memory");
+#pragma unroll
+                for (u32 k = 0; k < 5; k++)            // streaming stores: keep L1 for the table
+                    __stcs((u32*)(out + i) + k, __byte_perm(__byte_perm(e[4 * k], e[4 * k + 1], 0x40u), __byte_perm(e[4 * k + 2], e[4 * k + 3], 0x40u), 0x5410u));
+                i += 20;
+            } while (i + 20 <= n);
+#undef ZL_HUF_SYM5
+            zl_ring_to_br<ZL_LIT_RING_NS>(b, ring, pos, s16);
         }
-        b.hi = hi; b.lo = lo; b.nextw = nextw; b.wi = wi - (i32)s16;
     } else {
         const u32 count = n;                       // `n` below is the window's valid-bit count (macro convention)
         u32 hi = b.hi, lo = b.lo, nextw = b.nextw;
@@ -913,12 +926,6 @@ ZL_HD void zl_seq_step(const ZlSeqSm& f, ZlBitR& b, const u32* wbase, const ZlCo
 }
 
 #if defined(__CUDACC__)
-#ifndef ZL_SEQ_RING_PF
-#define ZL_SEQ_RING_PF 0          // L2 prefetch of the sequence ring: its address arithmetic costs more than it hides
-#endif
-#ifndef ZL_SEQ_RING_SYNC
-#define ZL_SEQ_RING_SYNC 2
-#endif
 // code -> (base value | additional bits << 24) for LL (36 entries) then ML (53 entries), in shared memory
 #define ZL_XTAB_WORDS (36 + 53)
 // Fast path over consecutive non-last sequences whose additional bits fit one 32-bit snapshot and whose lengths fit
@@ -926,6 +933,8 @@ ZL_HD void zl_seq_step(const ZlSeqSm& f, ZlBitR& b, const u32* wbase, const ZlCo
 // zl_seq_step takes that one).  The loop is rotated: the three table cells of the next sequence are requested as soon as
 // the new states are known.  States are kept "primed" (state + table size): a primed state is simply the cell's ns with
 // the nbBits fresh stream bits shifted in from the right -- one funnel shift -- and indexes the table at (base - size).
+// With a ring, one reload per sequence: a sequence takes at most 32 + 26 bits of the 64, and the reload for the next one
+// runs beside that sequence's cell loads, off the chain of dependent instructions.
 __device__ __forceinline__ u32 zl_seq_fast_loop(const ZlSeqSm& f, const u32* xtab, ZlBitR& b, const u32* wbase,
                                                 ZlSeqRegs& r, u64* rp, u32 maxIter, u32 safeCap, u32 ring)
 {
@@ -935,54 +944,66 @@ __device__ __forceinline__ u32 zl_seq_fast_loop(const ZlSeqSm& f, const u32* xta
               tML = zl_opaque(zl_smem_addr(f.fseML) - 2u * zML);
     const u32 kLL = 31u - gLL, kOF = 31u - gOF, kML = 31u - gML;          // nbBits = clz(ns) - k
     const u32 cLL = zl_opaque(zl_smem_addr(xtab)), cML = cLL + 36u * 4u;
-    u32 hi = b.hi, lo = b.lo, nextw = b.nextw;
-    i32 n = b.n, wi = b.wi;
-    const i32 wlow = b.wlow;
     u32 sLL = r.sLL + zLL, sOF = r.sOF + zOF, sML = r.sML + zML;
     u64* wp = rp + r.nrec;
     const u32 room = safeCap > r.nrec ? safeCap - r.nrec : 0u;
     if (maxIter > room) maxIter = room;
     u32 eLL = zl_lds16(tLL + (sLL << 1)), eOF = zl_lds16(tOF + (sOF << 1)), eML = zl_lds16(tML + (sML << 1));
     u32 it = 0;
-#define ZL_SEQ_LOOP(REFILL, REFILL2) \
-    while (it < maxIter) { \
-        const u32 llCode = ZL_CELL_SYM(eLL), mlCode = ZL_CELL_SYM(eML), aOF = ZL_CELL_SYM(eOF); \
-        const u32 xl = zl_lds32(cLL + (llCode << 2)), xm = zl_lds32(cML + (mlCode << 2)); \
-        const u32 nLL = ZL_CELL_NS(eLL), nML = ZL_CELL_NS(eML), nOF = ZL_CELL_NS(eOF); \
-        const u32 bLL = (u32)__clz((int)nLL) - kLL, bML = (u32)__clz((int)nML) - kML, bOF = (u32)__clz((int)nOF) - kOF; \
-        const u32 cA = aOF + (xl >> 24) + (xm >> 24); \
-        if (cA > 32 || llCode >= 35 || mlCode >= 50) break; \
-        REFILL; \
-        const u32 snap = hi; \
-        hi = zl_fsl(lo, hi, cA); lo = zl_shl(lo, cA); n -= (i32)cA; \
-        REFILL2; \
-        const u32 d2 = bLL + bML, cB = d2 + bOF; \
-        sLL = __funnelshift_l(hi, nLL, bLL); \
-        sML = __funnelshift_l(zl_fsl(lo, hi, bLL), nML, bML); \
-        sOF = __funnelshift_l(zl_fsl(lo, hi, d2), nOF, bOF); \
-        hi = zl_fsl(lo, hi, cB); lo <<= cB; n -= (i32)cB; \
-        eLL = zl_lds16(tLL + (sLL << 1)); eOF = zl_lds16(tOF + (sOF << 1)); eML = zl_lds16(tML + (sML << 1)); \
-        __stcs(wp++, zl_rec_a(snap, llCode, mlCode, aOF)); \
-        it++; \
-    }
-    if (ring) {
-        const u32 s16 = (u32)(((size_t)wbase >> 2) & 3);
+#define ZL_SEQ_HEAD                                                                                                         \
+        const u32 llCode = ZL_CELL_SYM(eLL), mlCode = ZL_CELL_SYM(eML), aOF = ZL_CELL_SYM(eOF);                             \
+        const u32 xl = zl_lds32(cLL + (llCode << 2)), xm = zl_lds32(cML + (mlCode << 2));                                   \
+        const u32 nLL = ZL_CELL_NS(eLL), nML = ZL_CELL_NS(eML), nOF = ZL_CELL_NS(eOF);                                      \
+        const u32 bLL = (u32)__clz((int)nLL) - kLL, bML = (u32)__clz((int)nML) - kML, bOF = (u32)__clz((int)nOF) - kOF;     \
+        const u32 cA = aOF + (xl >> 24) + (xm >> 24);                                                                       \
+        if (cA > 32 || llCode >= 35 || mlCode >= 50) break;                                                                 \
+        const u32 d2 = bLL + bML, cB = d2 + bOF;
+    if (ring != ZL_NO_RING) {
+        const i32 s16 = (i32)(((size_t)wbase >> 2) & 3);
         const u32* wb16 = wbase - s16;
-        const i32 clow = (wlow + (i32)s16) >> 2;
-        wi += (i32)s16;
-        zl_ring_start<4>(ring, ZL_SEQ_RING_SH, wb16, wi, clow);
-#if ZL_SEQ_RING_SYNC == 1
-        ZL_SEQ_LOOP(ZL_REFILL_RING_(ZL_SEQ_RING_SH, 4, ZL_SEQ_RING_PF, "cp.async.commit_group;\n\tcp.async.wait_group 8;\n\t"), ZL_REFILL_RING_(ZL_SEQ_RING_SH, 4, ZL_SEQ_RING_PF, "cp.async.commit_group;\n\tcp.async.wait_group 8;\n\t"))
-#else   // one group per sequence (two refills): a chunk is used 6 sequences or more after its copy was issued
-        ZL_SEQ_LOOP(ZL_REFILL_RING_(ZL_SEQ_RING_SH, 4, ZL_SEQ_RING_PF, "cp.async.commit_group;\n\tcp.async.wait_group 4;\n\t"), ZL_REFILL_RING_(ZL_SEQ_RING_SH, 4, ZL_SEQ_RING_PF, ""))
-#endif
-        asm volatile("cp.async.wait_all;" ::: "memory");
-        wi -= (i32)s16;
+        const i32 clow = (b.wlow + s16) >> 2;
+        const u8* gb = reinterpret_cast<const u8*>(wb16) - 16 * (ZL_SEQ_RING_NS - 1);
+        const i32 cmin = clow + (ZL_SEQ_RING_NS - 1);
+        i32 pos = 32 * (b.wi + 2 + s16) + b.n;
+        zl_ring_start<ZL_SEQ_RING_NS>(ring, wb16, pos, clow);
+        u32 hi, lo;
+        // one group per sequence: a chunk is first read >= 4 reloads after its copy (3 chunks of lead, <= 58 bits per reload)
+        ZL_RING_RELOAD(ZL_SEQ_RING_NS, "cp.async.commit_group;\n\tcp.async.wait_group 4;\n\t", ring, gb, cmin, pos, pos, hi, lo);
+        while (it < maxIter) {
+            ZL_SEQ_HEAD
+            const u32 h2 = zl_fsl(lo, hi, cA), l2 = zl_shl(lo, cA);
+            sLL = __funnelshift_l(h2, nLL, bLL);
+            sML = __funnelshift_l(zl_fsl(l2, h2, bLL), nML, bML);
+            sOF = __funnelshift_l(zl_fsl(l2, h2, d2), nOF, bOF);
+            eLL = zl_lds16(tLL + (sLL << 1)); eOF = zl_lds16(tOF + (sOF << 1)); eML = zl_lds16(tML + (sML << 1));
+            __stcs(wp++, zl_rec_a(hi, llCode, mlCode, aOF));
+            const i32 np = pos - (i32)(cA + cB);
+            ZL_RING_RELOAD(ZL_SEQ_RING_NS, "cp.async.commit_group;\n\tcp.async.wait_group 4;\n\t", ring, gb, cmin, np, pos, hi, lo);
+            pos = np;
+            it++;
+        }
+        zl_ring_to_br<ZL_SEQ_RING_NS>(b, ring, pos, s16);
     } else {
-        ZL_SEQ_LOOP(ZL_REFILL_DEV(), ZL_REFILL_DEV())
+        u32 hi = b.hi, lo = b.lo, nextw = b.nextw;
+        i32 n = b.n, wi = b.wi;
+        const i32 wlow = b.wlow;
+        while (it < maxIter) {
+            ZL_SEQ_HEAD
+            ZL_REFILL_DEV();
+            const u32 snap = hi;
+            hi = zl_fsl(lo, hi, cA); lo = zl_shl(lo, cA); n -= (i32)cA;
+            ZL_REFILL_DEV();
+            sLL = __funnelshift_l(hi, nLL, bLL);
+            sML = __funnelshift_l(zl_fsl(lo, hi, bLL), nML, bML);
+            sOF = __funnelshift_l(zl_fsl(lo, hi, d2), nOF, bOF);
+            hi = zl_fsl(lo, hi, cB); lo <<= cB; n -= (i32)cB;
+            eLL = zl_lds16(tLL + (sLL << 1)); eOF = zl_lds16(tOF + (sOF << 1)); eML = zl_lds16(tML + (sML << 1));
+            __stcs(wp++, zl_rec_a(snap, llCode, mlCode, aOF));
+            it++;
+        }
+        b.hi = hi; b.lo = lo; b.nextw = nextw; b.n = n; b.wi = wi;
     }
-#undef ZL_SEQ_LOOP
-    b.hi = hi; b.lo = lo; b.nextw = nextw; b.n = n; b.wi = wi;
+#undef ZL_SEQ_HEAD
     r.sLL = sLL - zLL; r.sOF = sOF - zOF; r.sML = sML - zML;
     r.nrec += it;
     return it;
@@ -991,11 +1012,11 @@ __device__ __forceinline__ u32 zl_seq_fast_loop(const ZlSeqSm& f, const u32* xta
 
 // serial sequence decode of one block (lane 0): zstd.c:44627-44700.  Completes the block's ZlBlockHdr (nrec, recOff);
 // the regenerated size is only known once K2 has added up the lengths.
-// `xtab` and `ring` (the lane's column of the stream ring, slots 128 bytes apart; 0 = none) are only used by the device
-// fast path (null in the CPU emulation).
+// `xtab` and `ring` (the unit's stream ring, ZL_SEQ_RING_NS slots; ZL_NO_RING = none) are only used by the device fast path
+// (null / none in the CPU emulation).
 // `recs` = this block's slice of the record arena (room for nbSeq + 4 records: a block regenerates <= 128 KiB, so at most
 // two lengths can be split); returns the number of records written.
-ZL_HD u32 zl_seq_decode(ZlSeqSm& f, u64* recs, const u32* wbase, u32 bias, const ZlConstTables& ct, const u32* xtab, u32 ring = 0)
+ZL_HD u32 zl_seq_decode(ZlSeqSm& f, u64* recs, const u32* wbase, u32 bias, const ZlConstTables& ct, const u32* xtab, u32 ring = ZL_NO_RING)
 {
     (void)xtab; (void)ring;
     ZlSeqCtl& c = f.ctl;

@@ -45,16 +45,17 @@ __global__ void __launch_bounds__(32)
 zl_k_literals(const ZlFrameDesc* __restrict__ descs, ZlFrameInfo* __restrict__ infos, const ZlBlockHdr* hdrArena,
               u8* litArena, const ZlUnit* __restrict__ units, const u32* __restrict__ unitCount, u32* cursor, const ZlDictDev* dict)
 {
-    extern __shared__ __align__(16) u8 smraw[];
-    ZlLitSm* fs = reinterpret_cast<ZlLitSm*>(smraw);
+    extern __shared__ __align__(128) u8 smraw[];
+    // stream ring first (its lanes' slots must be aligned to their 128 bytes, zl_huf_stream), then the eight units
+    const u32 ringBytes = ZL_LIT_RING ? 32u * 16u * ZL_LIT_RING_NS : 0u;
+    ZlLitSm* fs = reinterpret_cast<ZlLitSm*>(smraw + ringBytes);
     const u32 lane = threadIdx.x, quad = lane >> 2, q = lane & 3;
     const u32 qmask = 0xFu << (quad * 4);
     ZlLitSm& f = fs[quad];
-    // stream ring: ZL_LIT_RING_SLOTS slots of 32 x 16 bytes behind the eight units (zl_huf_stream)
-    const u32 ring = ZL_LIT_RING ? zl_smem_addr(smraw + ZL_QUADS_PER_WARP * sizeof(ZlLitSm)) + lane * 16u : 0u;
-    // the dictionary's Huffman table, once per CTA (behind the ring): units with treeless literals that fall back on it decode from this
+    const u32 ring = ZL_LIT_RING ? zl_smem_addr(smraw) + lane * 16u * ZL_LIT_RING_NS : ZL_NO_RING;
+    // the dictionary's Huffman table, once per CTA (behind the units): units with treeless literals that fall back on it decode from this
     // copy instead of copying 4 KB each (config 3: every object of a few hundred bytes did -- 512 load/store pairs per lane and unit)
-    u16* dictHuf = reinterpret_cast<u16*>(smraw + ZL_QUADS_PER_WARP * sizeof(ZlLitSm) + (ZL_LIT_RING ? ZL_LIT_RING_SLOTS * 32 * 16 : 0));
+    u16* dictHuf = reinterpret_cast<u16*>(smraw + ringBytes + ZL_QUADS_PER_WARP * sizeof(ZlLitSm));
     if (dict && dict->hasEntropy) {
         const uint4* g = reinterpret_cast<const uint4*>(dict->huf);
         for (u32 i = lane; i < 2048 * 2 / 16; i += 32) reinterpret_cast<uint4*>(dictHuf)[i] = g[i];
@@ -98,16 +99,18 @@ zl_k_literals(const ZlFrameDesc* __restrict__ descs, ZlFrameInfo* __restrict__ i
 // ---- K1b: sequences -----------------------------------------------------------------------------------------
 #define ZL_XTAB_BYTES ((ZL_XTAB_WORDS * 4 + 15) & ~15)
 #ifndef ZL_SEQ_RING
-#define ZL_SEQ_RING 1        // 4 slots, a group per sequence, no L2 prefetch: the kernel alone 2.38 -> 2.43 ms, the sliced step 151.3 -> 155.6 GB/s
+#define ZL_SEQ_RING 1        // 0: stream words by global loads (kept for A/B measurements)
 #endif
 __global__ void __launch_bounds__(32)
 zl_k_sequences(const ZlFrameDesc* __restrict__ descs, ZlFrameInfo* __restrict__ infos, ZlBlockHdr* hdrArena,
                u64* recArena, i16* normArena, const ZlUnit* __restrict__ units, const u32* __restrict__ unitCount, u32* cursor,
                const ZlDictDev* dict)
 {
-    extern __shared__ __align__(16) u8 smraw[];
-    u32* xtab = reinterpret_cast<u32*>(smraw);
-    ZlSeqSm* fs = reinterpret_cast<ZlSeqSm*>(smraw + ZL_XTAB_BYTES);
+    extern __shared__ __align__(128) u8 smraw[];
+    // stream ring first (its units' slots must be aligned to their 64 bytes, zl_seq_fast_loop), then the code table and the units
+    const u32 ringBytes = ZL_SEQ_RING ? 16u * ZL_SEQ_RING_NS * ZL_SEQ_UNITS : 0u;
+    u32* xtab = reinterpret_cast<u32*>(smraw + ringBytes);
+    ZlSeqSm* fs = reinterpret_cast<ZlSeqSm*>(smraw + ringBytes + ZL_XTAB_BYTES);
     const ZlConstTables& ct = c_tables;          // constant memory: only the header parser and the rare generic step index it
     // ZL_SEQ_G lanes share a unit (ZL_SEQ_UNITS units per warp): lane 0 of the group runs the serial chains, all of them build the tables
     const u32 lane = threadIdx.x, quad = lane / ZL_SEQ_G, q = lane % ZL_SEQ_G;
@@ -116,8 +119,7 @@ zl_k_sequences(const ZlFrameDesc* __restrict__ descs, ZlFrameInfo* __restrict__ 
         xtab[i] = i < 36 ? (c_tables.llBase[i] | ((u32)c_tables.llBits[i] << 24)) : (c_tables.mlBase[i - 36] | ((u32)c_tables.mlBits[i - 36] << 24));
     __syncwarp();
     ZlSeqSm& f = fs[quad];
-    // stream ring of the decoding lanes: 4 slots of ZL_SEQ_UNITS x 16 bytes behind the units (zl_seq_fast_loop)
-    const u32 ring = ZL_SEQ_RING ? zl_smem_addr(smraw + ZL_XTAB_BYTES + ZL_SEQ_UNITS * sizeof(ZlSeqSm)) + quad * 16u : 0u;
+    const u32 ring = ZL_SEQ_RING ? zl_smem_addr(smraw) + quad * 16u * ZL_SEQ_RING_NS : ZL_NO_RING;
     i16* norm = normArena + ((size_t)blockIdx.x * ZL_SEQ_UNITS + quad) * (3 * ZL_NORM_STRIDE);     // scratch per resident unit
     const u32 nunits = *unitCount;
     // few units in all (one large frame, the first small slices of a host-buffer call): a warp takes 8 of them instead of 16, so that
@@ -399,9 +401,9 @@ zl_k_xxh64_large(const u8* const* __restrict__ ptrs, const u32* __restrict__ siz
 }
 
 // ---- launchers ---------------------------------------------------------------------------------------
-size_t zl_literals_smem_bytes() { return ZL_QUADS_PER_WARP * sizeof(ZlLitSm) + (ZL_LIT_RING ? ZL_LIT_RING_SLOTS * 32 * 16 : 0); }
+size_t zl_literals_smem_bytes() { return ZL_QUADS_PER_WARP * sizeof(ZlLitSm) + (ZL_LIT_RING ? 32 * 16 * ZL_LIT_RING_NS : 0); }
 static size_t zl_literals_smem_dict_bytes() { return zl_literals_smem_bytes() + 2048 * sizeof(u16); }      // + the dictionary's Huffman table
-size_t zl_sequences_smem_bytes() { return ZL_XTAB_BYTES + ZL_SEQ_UNITS * sizeof(ZlSeqSm) + (ZL_SEQ_RING ? 4 * ZL_SEQ_UNITS * 16 : 0); }
+size_t zl_sequences_smem_bytes() { return ZL_XTAB_BYTES + ZL_SEQ_UNITS * sizeof(ZlSeqSm) + (ZL_SEQ_RING ? 16 * ZL_SEQ_RING_NS * ZL_SEQ_UNITS : 0); }
 
 // occupancy of the two persistent entropy kernels, per device (function attributes are per device too); guarded: contexts of
 // several host threads may decode for the first time at once

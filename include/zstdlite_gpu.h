@@ -131,6 +131,36 @@ size_t zl_compress_batch(ZSTD_CCtx* cctx, const void* const* src, const size_t* 
 size_t zl_compress_split(ZSTD_CCtx* cctx, void* dst, size_t dstCapacity, const void* src, size_t srcSize,
                          size_t frameSize, size_t* frameSizes, int ptrs_are_device);
 
+/* ---- seekable streams (Zstandard's seekable format, zstd's contrib/seekable_format) ----
+ * A seekable stream is N >= 1 independent frames followed by a skippable frame holding the seek table:
+ *   magic 0x184D2A5E, Frame_Size u32, N entries {Compressed_Size u32, Decompressed_Size u32[, Checksum u32]},
+ *   then a 9-byte footer: Number_Of_Frames u32, Seek_Table_Descriptor u8 (bit 7: entries carry a checksum; bits 6-2: 0),
+ *   Seekable_Magic_Number u32 = 0x8F92EAB1.  All little-endian; Checksum is the low 32 bits of the XXH64 (seed 0) of the frame's content.
+ * Every Zstandard reader, ZSTD_decompressDCtx included, still decodes the whole stream: the table is a skippable frame.  A table is valid
+ * when Frame_Size = 8N + 9 (12N + 9 with checksums), the reserved bits are 0, N <= 0x8000000 and the Compressed_Size values plus the
+ * table frame add up to the stream's length; anything else is corruption_detected.  A stream that does not end in the seekable magic
+ * gives prefix_unknown.
+ *
+ * zl_compress_seekable: zl_compress_split's frames, byte for byte, then their seek table (with checksums when the context has
+ * ZSTD_c_checksumFlag: the frames' own trailers).  frameSize must be 1 .. 0x40000000 (parameter_outOfBound otherwise).  With
+ * ptrs_are_device the table is written to device memory after the frames.  Returns the stream's size or an error code.
+ * zl_compress_seekable_bound: a dstCapacity that is always enough for zl_compress_seekable (or an error code for a bad frameSize). */
+size_t zl_compress_seekable(ZSTD_CCtx* cctx, void* dst, size_t dstCapacity, const void* src, size_t srcSize, size_t frameSize,
+                            int ptrs_are_device);
+size_t zl_compress_seekable_bound(size_t srcSize, size_t frameSize, int checksum);
+/* The seek table of a stream: returns N, or an error code.  When cap >= N, cSizes / dSizes / checksums (each optional, N entries)
+ * receive the table's fields; call with cap = 0 to learn N first.  *hasChecksums (optional) says whether the table has checksums.
+ * With ptrs_are_device the footer and then the entries are copied from device memory on the current device (no GPU is needed otherwise). */
+size_t zl_seekable_frames(const void* src, size_t srcSize, int ptrs_are_device, unsigned* cSizes, unsigned* dSizes,
+                          unsigned* checksums, size_t cap, int* hasChecksums);
+/* Bytes [offset, offset + length) of a seekable stream's content into dst; a range past the end is clamped, like pread.  Returns the
+ * bytes written, min(length, total - offset).  Only the frames the range touches are decoded, in one batch on the context's device, with
+ * its dictionary; every frame must produce exactly its table size (corruption_detected otherwise) and, unless ZSTD_d_forceIgnoreChecksum
+ * is set, match the table's checksum as well as its own trailer (checksum_wrong).  offset > total: parameter_outOfBound; dstCapacity
+ * below the result: dstSize_tooSmall.  ptrs_are_device: src and dst are device memory. */
+size_t zl_decompress_range(ZSTD_DCtx* dctx, void* dst, size_t dstCapacity, const void* src, size_t srcSize, size_t offset,
+                           size_t length, int ptrs_are_device);
+
 /* Several GPUs from ONE process (frames are independent: SURVEY.md 8e).  Batches of HOST buffers (zl_decompress_batch / zl_compress_batch, and
  * ZSTD_decompressDCtx on a multi-frame stream) are cut into contiguous frame ranges of about equal bytes, one per device, each handled by a helper
  * context on its own host thread; no collective, no peer traffic.  How many GPUs: zl_dctx_set_gpus(n) for a DCtx; num_threads (ZSTD_c_nbWorkers) >= 2 for

@@ -177,17 +177,29 @@ class zstd_cctx:
             self._p = None
 
 
-def zstd_compress(src, cctx=None, frame_size=None, **opts):
+def zstd_compress(src, cctx=None, frame_size=None, seekable=False, **opts):
     """zstd_compress(src, ..., cctx)  (src/raw-file.c:25-118): raw vector or string -> one zstd frame.
 
     frame_size=N (extension, SURVEY.md 8b): the input is cut into independent frames of N content bytes, returned as one
-    standard concatenated stream (zl_compress_split); zstd_decompress(all_frames=True) or any zstd reader decodes it."""
+    standard concatenated stream (zl_compress_split); zstd_decompress(all_frames=True) or any zstd reader decodes it.
+    seekable=True (with frame_size): the same frames followed by a seek table in Zstandard's seekable format
+    (zl_compress_seekable), so that zstd_decompress_range can decode any byte range without decoding the rest."""
     L = _lib.lib()
     if cctx is None:
         cctx = zstd_cctx(**opts)
     buf, n, _keep = _as_buffer(src)
     L.ZSTD_CCtx_setParameter(cctx._p, _lib.ZSTD_c_stableInBuffer, 1)      # src/cctx.c:70-96
     L.ZSTD_CCtx_setParameter(cctx._p, _lib.ZSTD_c_stableOutBuffer, 1)
+    if seekable:
+        if not frame_size:
+            raise ZstdError("zstd_compress(): seekable=True needs frame_size")
+        v = C.c_int(0)
+        L.ZSTD_CCtx_getParameter(cctx._p, _lib.ZSTD_c_checksumFlag, C.byref(v))
+        cap = _check(L.zl_compress_seekable_bound(n, int(frame_size), v.value), "zstd_compress(): frame_size")
+        dst, dptr = _scratch(cap)
+        r = L.zl_compress_seekable(cctx._p, dptr, cap, buf, n, int(frame_size), 0)
+        _check(r, "zstd_compress(): Compression error")
+        return dst[:r].tobytes()
     if frame_size:
         frame_size = int(frame_size)
         nfr = max(1, -(-n // frame_size))
@@ -230,6 +242,69 @@ def zstd_decompress(src, type="raw", dctx=None, all_frames=False, **opts):
     if r != usize:
         out = out[:r]
     return out.decode("utf-8") if type == "string" else out
+
+
+def _source(src):
+    """bytes-like, or a 1-D contiguous torch.uint8 CUDA tensor (duck-typed: torch is not imported for it) ->
+    (pointer, length, object that keeps the memory alive, is_device)"""
+    if getattr(src, "is_cuda", False):
+        if src.dim() != 1 or not src.is_contiguous() or str(src.dtype) != "torch.uint8":
+            raise ZstdError("a device source must be a 1-D contiguous torch.uint8 CUDA tensor")
+        return C.c_void_p(src.data_ptr() or None), src.numel(), src, True
+    buf, n, keep = _as_buffer(src)
+    return buf, n, keep, False
+
+
+def _seek_table(buf, n, dev):
+    L = _lib.lib()
+    k = _check(L.zl_seekable_frames(buf, n, 1 if dev else 0, None, None, None, 0, None), "zstd_seek_table()")
+    cs, ds, ck, has = (C.c_uint * max(1, k))(), (C.c_uint * max(1, k))(), (C.c_uint * max(1, k))(), C.c_int(0)
+    _check(L.zl_seekable_frames(buf, n, 1 if dev else 0, cs, ds, ck, k, C.byref(has)), "zstd_seek_table()")
+    return [(cs[i], ds[i], ck[i] if has.value else None) for i in range(k)]
+
+
+def zstd_seek_table(src):
+    """The seek table of a seekable stream (zstd_compress(..., seekable=True), or any writer of Zstandard's seekable format):
+    a list of (compressed_size, decompressed_size, checksum or None), one per frame.  `src` is bytes-like or a CUDA tensor."""
+    buf, n, _keep, dev = _source(src)
+    if dev:
+        import torch
+        torch.cuda.current_stream(src.device).synchronize()
+    return _seek_table(buf, n, dev)
+
+
+def zstd_decompress_range(src, offset, length, dctx=None, type="raw", out=None, **opts):
+    """Bytes [offset, offset + length) of a seekable stream's content, clamped to its end; only the frames the range touches are decoded
+    (zl_decompress_range).  A bytes-like `src` gives bytes (str with type="string"); a CUDA tensor gives a CUDA uint8 tensor, or the
+    first bytes of `out` (a CUDA uint8 tensor) written in place.  The table's checksums are verified unless validate_checksum=False."""
+    L = _lib.lib()
+    if dctx is None:
+        dctx = zstd_dctx(**opts)
+    buf, n, _keep, dev = _source(src)
+    offset, length = int(offset), int(length)
+    if offset < 0 or length < 0:
+        raise ZstdError("zstd_decompress_range(): offset and length must be >= 0")
+    if dev:
+        import torch
+        torch.cuda.current_stream(src.device).synchronize()               # the library reads on its own stream
+    total = sum(d for _, d, _ in _seek_table(buf, n, dev))
+    want = max(0, min(length, total - offset))
+    if dev:
+        if out is None:
+            out = torch.empty(max(1, want), dtype=torch.uint8, device=src.device)
+        elif not getattr(out, "is_cuda", False) or out.dim() != 1 or not out.is_contiguous() or out.dtype != torch.uint8:
+            raise ZstdError("zstd_decompress_range(): out must be a 1-D contiguous torch.uint8 CUDA tensor")
+        else:
+            torch.cuda.current_stream(out.device).synchronize()
+        r = L.zl_decompress_range(dctx._p, C.c_void_p(out.data_ptr()), out.numel(), buf, n, offset, length, 1)
+        _check(r, "zstd_decompress_range(): De-compression error")
+        return out[:r]
+    if out is not None:
+        raise ZstdError("zstd_decompress_range(): out is only taken for a CUDA source")
+    res, rptr = _new_bytes(want)
+    r = L.zl_decompress_range(dctx._p, rptr, want, buf, n, offset, length, 0)
+    _check(r, "zstd_decompress_range(): De-compression error")
+    return res.decode("utf-8") if type == "string" else res
 
 
 def zstd_serialize(obj, cctx=None, frame_size=None, **opts):

@@ -8,6 +8,7 @@
 #include <thread>
 #include "../../include/zstdlite_gpu.h"
 #include "zl_batch_plan.h"            // (and zl_host.h)
+#include "zl_seek.h"
 #include "zl_dec_entropy.cuh"     // ZL_HD table builders reused to digest dictionaries on the host (zstd.c:42053)
 
 #define ZL_EXPORT extern "C" __attribute__((visibility("default")))
@@ -211,6 +212,7 @@ struct ZSTD_DCtx_s {
     size_t sOutPos = 0;
     ZlDevBuf dRaw, dDescs, dInfos, dResults, dHdr, dRec, dCk, dLit, dNorm, dUnits, dCounters, dLargeIdx, dLb, dLc, dParent, dRemain, dSrc, dDst;
     ZlPinBuf hDescs, hResults, hLargeIdx, hRemain;
+    ZlDevBuf dSeek; std::vector<u8> hSeek;  // zl_decompress_range: the edge frames of a range, decoded whole (device / host buffers)
     std::vector<cudaEvent_t> sliceDone;    // staged host buffers: the copy back of a slice has landed
     // devices: the context's own (bound on first use) and, for batches of host buffers, the helpers on the other GPUs of the box
     int device = -1, gpus = 0;             // gpus: 0 = ZSTDLITE_GPUS (default 1)
@@ -235,7 +237,7 @@ ZL_EXPORT size_t ZSTD_freeDCtx(ZSTD_DCtx* c)
     for (ZSTD_DCtx_s* k : c->kids) ZSTD_freeDCtx(k);
     c->kids.clear();
     ZlDeviceGuard guard(c->device);
-    ZlDevBuf* bufs[] = {&c->dDictContent, &c->dDict, &c->dRaw, &c->dDescs, &c->dInfos, &c->dResults, &c->dHdr, &c->dRec, &c->dCk, &c->dLit, &c->dNorm, &c->dUnits, &c->dCounters, &c->dLargeIdx, &c->dLb, &c->dLc, &c->dParent, &c->dRemain, &c->dSrc, &c->dDst};
+    ZlDevBuf* bufs[] = {&c->dDictContent, &c->dDict, &c->dRaw, &c->dDescs, &c->dInfos, &c->dResults, &c->dHdr, &c->dRec, &c->dCk, &c->dLit, &c->dNorm, &c->dUnits, &c->dCounters, &c->dLargeIdx, &c->dLb, &c->dLc, &c->dParent, &c->dRemain, &c->dSrc, &c->dDst, &c->dSeek};
     for (ZlDevBuf* b : bufs) b->release();
     c->hDescs.release(); c->hResults.release(); c->hLargeIdx.release(); c->hRemain.release();
     for (cudaEvent_t e : c->sliceDone) if (e) cudaEventDestroy(e);
@@ -368,10 +370,11 @@ static bool zl_dctx_lanes(ZSTD_DCtx* c)
     return true;
 }
 
+// expect (optional, by caller's index): checksums from a seek table that the frames' content must match as well as their own trailers
 static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, const size_t* srcSize, void* const* dst,
-                                       const size_t* dstCap, size_t* result, size_t n, int dev, bool worst);
+                                       const size_t* dstCap, size_t* result, size_t n, int dev, bool worst, const u32* expect);
 static size_t zl_decompress_batch_one(ZSTD_DCtx* c, const void* const* src, const size_t* srcSize, void* const* dst,
-                                      const size_t* dstCap, size_t* result, size_t n, int dev);
+                                      const size_t* dstCap, size_t* result, size_t n, int dev, const u32* expect = nullptr);
 // extension: GPUs a context spreads batches of HOST buffers over (0: ZSTDLITE_GPUS, default 1); frames are independent, so the
 // frame list is cut into contiguous ranges of about equal content, one per device, each decoded by a helper context on its own
 // host thread (copies, kernels and staging of the devices overlap); no data moves between the devices
@@ -414,23 +417,23 @@ ZL_EXPORT size_t zl_decompress_batch(ZSTD_DCtx* c, const void* const* src, const
     return 0;
 }
 static size_t zl_decompress_batch_one(ZSTD_DCtx* c, const void* const* src, const size_t* srcSize, void* const* dst,
-                                      const size_t* dstCap, size_t* result, size_t n, int dev)
+                                      const size_t* dstCap, size_t* result, size_t n, int dev, const u32* expect)
 {
     ZlDeviceGuard guard(zl_bind_device(&c->device));
     if (!guard.ok) return ZL_ERROR(GENERIC);
-    size_t r = zl_decompress_batch_impl(c, src, srcSize, dst, dstCap, result, n, dev, false);
+    size_t r = zl_decompress_batch_impl(c, src, srcSize, dst, dstCap, result, n, dev, false, expect);
     if (zl_is_error(r)) return r;
     bool retry = false;
     for (size_t i = 0; i < n; i++) if (result[i] == (size_t)0 - (size_t)ZL_E_INTERNAL_hdrCap) { retry = true; break; }
     if (retry) {                          // a frame with very many small blocks: run again with worst-case block arenas
-        r = zl_decompress_batch_impl(c, src, srcSize, dst, dstCap, result, n, dev, true);
+        r = zl_decompress_batch_impl(c, src, srcSize, dst, dstCap, result, n, dev, true, expect);
         if (zl_is_error(r)) return r;
         for (size_t i = 0; i < n; i++) if (result[i] == (size_t)0 - (size_t)ZL_E_INTERNAL_hdrCap) result[i] = ZL_ERROR(GENERIC);
     }
     return 0;
 }
 static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, const size_t* srcSize, void* const* dst,
-                                       const size_t* dstCap, size_t* result, size_t n, int dev, bool worst)
+                                       const size_t* dstCap, size_t* result, size_t n, int dev, bool worst, const u32* expect)
 {
     if (n == 0) return 0;
     static const ZlDecTuning tune = {getenv("ZL_DEC_SLICES") ? atoi(getenv("ZL_DEC_SLICES")) : 0, getenv("ZL_DEC_GRADE") ? atoi(getenv("ZL_DEC_GRADE")) : 6,
@@ -491,6 +494,13 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
     size_t largeSeen = 0;
     const double tPrep = hostMs();
     if (!p.lazyDescs && !p.devBuild) cudaMemcpyAsync(c->dDescs.p, hd, n * sizeof(ZlFrameDesc), cudaMemcpyHostToDevice, st);
+    std::vector<u32> expectPos;                                             // (pageable: the copy has taken it when the call returns)
+    if (expect && !c->forceIgnoreChecksum) {                               // in launch order, like the descriptors
+        expectPos.resize(n);
+        for (size_t pos = 0; pos < n; pos++) expectPos[pos] = expect[p.devBuild ? pos : p.order[pos]];
+        if (!c->dCk.reserve(n * 4)) return ZL_ERROR(memory_allocation);
+        cudaMemcpyAsync(c->dCk.p, expectPos.data(), n * 4, cudaMemcpyHostToDevice, st);
+    }
     if (!c->stageEv[0]) for (cudaEvent_t& e : c->stageEv) cudaEventCreate(&e);
     cudaEventRecord(c->ev0, st);
     if (nslices > 1) cudaEventRecord(c->forkEv, st);
@@ -558,6 +568,7 @@ static size_t zl_decompress_batch_impl(ZSTD_DCtx* c, const void* const* src, con
         }
         L.results = c->dResults.as<u64>() + a;
         L.nframes = (u32)cnt; L.verifyChecksum = !c->forceIgnoreChecksum; L.dict = c->hasDict ? c->dDict.as<ZlDictDev>() : nullptr;
+        L.expect = expectPos.empty() ? nullptr : c->dCk.as<u32>() + a;
         L.stageEv = stageTimed ? c->stageEv : nullptr;
         // host buffers only: literals next to sequences shortens the chain of a slice, i.e. the wait before its copy back can
         // start (measured 39.9 -> 41.4 GB/s end to end); device-resident batches are throughput-bound and lose (143 -> 125 GB/s)
@@ -715,3 +726,90 @@ ZL_EXPORT size_t ZSTD_decompressStream(ZSTD_DCtx* c, ZSTD_outBuffer* out, ZSTD_i
     }
 }
 ZL_ALIAS(size_t, ZSTD_decompressStream, (ZSTD_DCtx*, ZSTD_outBuffer*, ZSTD_inBuffer*))
+
+// ---------------------------------------------------------------------------------------------- seekable streams (zl_seek.h)
+// The seek table of a stream in host or device memory: its footer, then the table frame, copied to the host on `st` when the stream is
+// in device memory (the library never walks the frames' block headers for it).
+static size_t zl_seek_read(ZlSeekTable& t, const void* srcv, size_t srcSize, bool dev, cudaStream_t st)
+{
+    const u8* src = (const u8*)srcv;
+    if (srcSize && !src) return ZL_ERROR(GENERIC);
+    std::vector<u8> copy;
+    auto fetch = [&](size_t off, size_t n) -> const u8* {
+        if (!dev) return src + off;
+        copy.resize(n);
+        if (cudaMemcpyAsync(copy.data(), src + off, n, cudaMemcpyDeviceToHost, st) != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) {
+            (void)cudaGetLastError(); return nullptr;
+        }
+        return copy.data();
+    };
+    const size_t tail = srcSize < ZL_SEEK_FOOTER ? srcSize : ZL_SEEK_FOOTER;
+    const u8* f = fetch(srcSize - tail, tail);
+    if (!f) return ZL_ERROR(GENERIC);
+    u32 n = 0; bool ck = false;
+    const size_t size = zl_seek_footer(f, srcSize, &n, &ck);
+    if (zl_is_error(size)) return size;
+    const u8* table = fetch(srcSize - size, size);
+    if (!table) return ZL_ERROR(GENERIC);
+    return zl_seek_parse(t, table, size, srcSize);
+}
+
+ZL_EXPORT size_t zl_seekable_frames(const void* src, size_t srcSize, int ptrs_are_device, unsigned* cSizes, unsigned* dSizes,
+                                    unsigned* checksums, size_t cap, int* hasChecksums)
+{
+    ZlSeekTable t;
+    const size_t r = zl_seek_read(t, src, srcSize, ptrs_are_device != 0, nullptr);
+    if (zl_is_error(r)) return r;
+    if (hasChecksums) *hasChecksums = t.checksums ? 1 : 0;
+    if (cap >= t.n) {
+        if (cSizes) memcpy(cSizes, t.cSize.data(), t.n * 4);
+        if (dSizes) memcpy(dSizes, t.dSize.data(), t.n * 4);
+        if (checksums && t.checksums) memcpy(checksums, t.checksum.data(), t.n * 4);
+    }
+    return t.n;
+}
+
+// Bytes [offset, offset + length) of a seekable stream's content: the frames the range touches are decoded as one batch on the context's
+// device, the interior ones straight into dst, the one or two edge frames whole into the context's scratch, from which the wanted bytes are
+// copied.  Every frame must produce exactly its table size; the table's checksums are verified in the checksum kernels.
+ZL_EXPORT size_t zl_decompress_range(ZSTD_DCtx* c, void* dst, size_t dstCap, const void* src, size_t srcSize, size_t offset, size_t length,
+                                     int ptrs_are_device)
+{
+    if (!c) return ZL_ERROR(GENERIC);
+    const bool dev = ptrs_are_device != 0;
+    ZlDeviceGuard guard(zl_bind_device(&c->device));
+    if (!guard.ok) return ZL_ERROR(GENERIC);
+    if (!zl_ctx_stream(&c->stream, &c->ownStream, &c->ev0, &c->ev1)) return ZL_ERROR(memory_allocation);
+    cudaStream_t st = c->stream;
+    ZlSeekTable t;
+    if (const size_t r = zl_seek_read(t, src, srcSize, dev, st)) return r;
+    ZlSeekPlan p;
+    if (const size_t r = zl_seek_plan_range(p, t, offset, length)) return r;
+    if (p.bytes > dstCap) return ZL_ERROR(dstSize_tooSmall);
+    if (!p.bytes) return 0;
+    if (!dst) return ZL_ERROR(dstBuffer_null);
+    u8* scratch = nullptr;
+    if (dev) { if (!c->dSeek.reserve(p.scratchBytes + 64)) return ZL_ERROR(memory_allocation); scratch = c->dSeek.as<u8>(); }
+    else { if (c->hSeek.size() < p.scratchBytes + 64) c->hSeek.resize(p.scratchBytes + 64); scratch = c->hSeek.data(); }
+    const size_t n = p.last - p.first;
+    std::vector<const void*> fsrc(n); std::vector<void*> fdst(n); std::vector<size_t> fsize(n), fcap(n), fres(n, 0);
+    for (size_t j = 0; j < n; j++) {
+        const size_t f = p.first + j;
+        fsrc[j] = (const u8*)src + t.cOff[f]; fsize[j] = t.cSize[f]; fcap[j] = t.dSize[f];
+        fdst[j] = (p.edge[j] ? scratch : (u8*)dst) + p.place[j];
+    }
+    const size_t r = zl_decompress_batch_one(c, fsrc.data(), fsize.data(), fdst.data(), fcap.data(), fres.data(), n, dev,
+                                             t.checksums ? t.checksum.data() + p.first : nullptr);
+    if (zl_is_error(r)) return r;
+    for (size_t j = 0; j < n; j++) {
+        if (zl_is_error(fres[j])) return fres[j];
+        if (fres[j] != fcap[j]) return ZL_ERROR(corruption_detected);       // the table's Decompressed_Size is wrong
+    }
+    for (size_t k = 0; k < p.nEdges; k++) {
+        const ZlSeekEdge& e = p.edges[k];
+        if (dev) cudaMemcpyAsync((u8*)dst + e.outOff, scratch + e.scratchOff + e.skip, e.take, cudaMemcpyDeviceToDevice, st);
+        else memcpy((u8*)dst + e.outOff, scratch + e.scratchOff + e.skip, e.take);
+    }
+    if (dev && cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
+    return p.bytes;
+}

@@ -11,6 +11,7 @@
 #include <thread>
 #include "zl_enc_plan.h"
 #include "zl_enc_dict.h"          // host-side dictionary digest (shared with the CPU emulation in tests/emul)
+#include "zl_seek.h"
 
 #define ZL_EXPORT extern "C" __attribute__((visibility("default")))
 #define ZL_ALIAS(ret, name, params) extern "C" __attribute__((visibility("default"), alias(#name))) ret zlg_##name params;
@@ -630,6 +631,59 @@ ZL_EXPORT size_t zl_compress_split(ZSTD_CCtx* c, void* dst, size_t dstCap, const
     if (!dev && total) cudaMemcpyAsync(dst, out, total, cudaMemcpyDeviceToHost, st);
     if (cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
     return total;
+}
+
+// Seekable format (zl_seek.h): the frames of zl_compress_split, unchanged, followed by their seek table.  With checksums every frame already
+// ends in the low 32 bits of its XXH64; the table takes those 4 bytes (gathered on the device for device buffers) instead of hashing again.
+static size_t zl_seek_frame_count(size_t srcSize, size_t frameSize)
+{
+    if (!frameSize || frameSize > ZL_SEEK_MAX_FRAME_SIZE) return ZL_ERROR(parameter_outOfBound);
+    const size_t nf = srcSize ? (srcSize - 1) / frameSize + 1 : 1;
+    return nf > ZL_SEEK_MAX_FRAMES ? ZL_ERROR(parameter_outOfBound) : nf;
+}
+ZL_EXPORT size_t zl_compress_seekable_bound(size_t srcSize, size_t frameSize, int checksum)
+{
+    const size_t nf = zl_seek_frame_count(srcSize, frameSize);
+    if (zl_is_error(nf)) return nf;
+    const size_t full = srcSize / frameSize, rest = srcSize - full * frameSize, trailer = checksum ? 4 : 0;
+    size_t b = full * (ZSTD_compressBound(frameSize) + trailer);
+    if (rest || !srcSize) b += ZSTD_compressBound(rest) + trailer;
+    return b + zl_seek_table_size(nf, checksum != 0);
+}
+ZL_EXPORT size_t zl_compress_seekable(ZSTD_CCtx* c, void* dst, size_t dstCap, const void* src, size_t srcSize, size_t frameSize, int dev)
+{
+    if (!c) return ZL_ERROR(GENERIC);
+    const size_t nf = zl_seek_frame_count(srcSize, frameSize);
+    if (zl_is_error(nf)) return nf;
+    std::vector<size_t> fs(nf, 0);
+    const size_t total = zl_compress_split(c, dst, dstCap, src, srcSize, frameSize, fs.data(), dev);
+    if (zl_is_error(total)) return total;
+    const bool ck = c->checksumFlag != 0;
+    const size_t tsz = zl_seek_table_size(nf, ck);
+    if (tsz > dstCap - total) return ZL_ERROR(dstSize_tooSmall);
+    ZlDeviceGuard guard(zl_bind_device(&c->device));
+    if (!guard.ok) return ZL_ERROR(GENERIC);
+    cudaStream_t st = c->stream;
+    std::vector<u32> cs(nf), ds(nf), sums(ck ? nf : 0);
+    size_t off = 0;
+    for (size_t i = 0; i < nf; i++) { cs[i] = (u32)fs[i]; ds[i] = (u32)std::min(frameSize, srcSize - std::min(srcSize, i * frameSize)); }
+    if (ck && !dev) for (size_t i = 0; i < nf; off += fs[i], i++) sums[i] = zl_rd32((const u8*)dst + off + fs[i] - 4);
+    if (ck && dev) {                            // one gather of the nf trailers (the table reads the pinned array in place) and one copy back
+        if (!c->hAux.reserve(nf * 28) || !c->dAux.reserve(nf * 4)) return ZL_ERROR(memory_allocation);
+        u64* t = c->hAux.as<u64>();
+        for (size_t i = 0; i < nf; off += fs[i], i++) { t[i] = 4; t[nf + i] = 4 * i; reinterpret_cast<const u8**>(t + 2 * nf)[i] = (const u8*)dst + off + fs[i] - 4; }
+        if (zl_launch_gather(reinterpret_cast<const u8* const*>(t + 2 * nf), t, t + nf, c->dAux.as<u8>(), (u32)nf, st) != cudaSuccess) return ZL_ERROR(GENERIC);
+        c->launches += 1;
+        cudaMemcpyAsync(t + 3 * nf, c->dAux.p, nf * 4, cudaMemcpyDeviceToHost, st);
+        if (cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
+        memcpy(sums.data(), t + 3 * nf, nf * 4);
+    }
+    std::vector<u8> table(tsz);
+    zl_seek_write(table.data(), nf, cs.data(), ds.data(), ck ? sums.data() : nullptr);
+    if (!dev) { memcpy((u8*)dst + total, table.data(), tsz); return total + tsz; }
+    cudaMemcpyAsync((u8*)dst + total, table.data(), tsz, cudaMemcpyHostToDevice, st);
+    if (cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
+    return total + tsz;
 }
 
 #include "zl_dict_train.cuh"

@@ -1,7 +1,7 @@
 // zl_dec_kernels.cu -- the decode kernels and their launchers (sm_100a).
 //   K1a zl_k_literals / K1b zl_k_sequences   quad-per-frame entropy decode -> literal / record / header arenas
 //   K2 zl_k_execute   warp-per-frame sequence execution -> frame output
-//   K3 zl_k_checksum  quad-per-frame XXH64 of the output, compared with the frame trailer
+//   K3 zl_k_checksum  quad-per-frame XXH64 of the output, compared with the frame trailer (and a seek table's checksum)
 #include "zl_dec_entropy.cuh"
 #include "zl_dec_exec.cuh"
 #include "zl_dec_large.cuh"
@@ -352,30 +352,38 @@ zl_k_lfinish(const u32* __restrict__ largeIdx, u32 nLarge, ZlFrameInfo* __restri
     results[frame] = err ? (u64)0 - (u64)err : (u64)infos[frame].totalOut;
 }
 
+// expect (optional, in launch order): a value every frame's hash must also match -- the checksums of a seek table (zl_seek.h).  A frame
+// with one is hashed even when it has no trailer of its own.
+static __device__ __forceinline__ bool zl_checksum_ok(const ZlFrameInfo& info, const u32* expect, u32 frame, u64 h)
+{
+    return (!info.checksumFlag || (u32)h == info.checksum) && (!expect || (u32)h == expect[frame]);
+}
 __global__ void __launch_bounds__(128)
-zl_k_checksum(const ZlFrameDesc* __restrict__ descs, const ZlFrameInfo* __restrict__ infos, u64* __restrict__ results, u32 nframes)
+zl_k_checksum(const ZlFrameDesc* __restrict__ descs, const ZlFrameInfo* __restrict__ infos, u64* __restrict__ results, u32 nframes,
+              const u32* __restrict__ expect)
 {
     const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
     const u32 frame = t >> 2, q = t & 3, lane = threadIdx.x & 31;
     const u32 qbase = lane & ~3u, qmask = 0xFu << qbase;
     if (frame >= nframes) return;
     const ZlFrameInfo info = infos[frame];
-    if (info.err || !info.checksumFlag) return;
+    if (info.err || (!info.checksumFlag && !expect)) return;
     if (descs[frame].large && !(((size_t)descs[frame].dst) & 15)) return;          // zl_k_checksum_large
     const u64 h = zl_quad_xxh64(descs[frame].dst, info.totalOut, q, qmask, qbase);
-    if (q == 0 && (u32)h != info.checksum) results[frame] = (u64)0 - (u64)ZL_E_checksum_wrong;   // zstd.c:41650-41657
+    if (q == 0 && !zl_checksum_ok(info, expect, frame, h)) results[frame] = (u64)0 - (u64)ZL_E_checksum_wrong;   // zstd.c:41650-41657
 }
 
 // large frames: a warp per frame (zl_warp_xxh64); frames whose output is not 16-byte aligned keep the quad path of zl_k_checksum
 __global__ void __launch_bounds__(32)
-zl_k_checksum_large(const u32* __restrict__ largeIdx, const ZlFrameDesc* __restrict__ descs, const ZlFrameInfo* __restrict__ infos, u64* __restrict__ results)
+zl_k_checksum_large(const u32* __restrict__ largeIdx, const ZlFrameDesc* __restrict__ descs, const ZlFrameInfo* __restrict__ infos, u64* __restrict__ results,
+                    const u32* __restrict__ expect)
 {
     __shared__ __align__(16) u8 buf[2][ZL_XXH_CHUNK];
     const u32 frame = largeIdx[blockIdx.x], lane = threadIdx.x;
     const ZlFrameInfo info = infos[frame];
-    if (info.err || !info.checksumFlag || (((size_t)descs[frame].dst) & 15)) return;
+    if (info.err || (!info.checksumFlag && !expect) || (((size_t)descs[frame].dst) & 15)) return;
     const u64 h = zl_warp_xxh64(descs[frame].dst, info.totalOut, buf, lane);
-    if (lane == 0 && (u32)h != info.checksum) results[frame] = (u64)0 - (u64)ZL_E_checksum_wrong;   // zstd.c:41650-41657
+    if (lane == 0 && !zl_checksum_ok(info, expect, frame, h)) results[frame] = (u64)0 - (u64)ZL_E_checksum_wrong;   // zstd.c:41650-41657
 }
 
 // generic XXH64 of independent buffers (used by the compressor for frame trailers)
@@ -517,8 +525,8 @@ cudaError_t zl_launch_decode(const ZlDecodeLaunch& L, cudaStream_t st)
     if (ev) cudaEventRecord(ev[3], st);
     if (L.verifyChecksum) {
         const u32 g3 = (L.nframes * 4 + 127) / 128;
-        zl_k_checksum<<<g3, 128, 0, st>>>(L.descs, L.infos, L.results, L.nframes);
-        if (L.nLarge) { zl_k_checksum_large<<<L.nLarge, 32, 0, st>>>(L.largeIdx, L.descs, L.infos, L.results); nk++; }
+        zl_k_checksum<<<g3, 128, 0, st>>>(L.descs, L.infos, L.results, L.nframes, L.expect);
+        if (L.nLarge) { zl_k_checksum_large<<<L.nLarge, 32, 0, st>>>(L.largeIdx, L.descs, L.infos, L.results, L.expect); nk++; }
         nk++;
     }
     if (ev) cudaEventRecord(ev[4], st);

@@ -82,6 +82,7 @@ struct ZlDecodeLaunch {          // one slice of a batch: frames [frameBase, fra
     u32* counters;               // this slice's {unit count, literal cursor, sequence cursor}
     u32 nframes;
     int verifyChecksum;
+    const u32* expect = nullptr; // optional, per frame of the slice: a checksum from a seek table the output must also match (zl_seek.h)
     // large frames of this slice (zl_dec_large.cuh); nLarge == 0: none
     const u32* largeIdx;         // device: indices (relative to the slice) of the large frames
     u32 nLarge, largeMaxBlocks;  // count; largest hdrCap among them (grid bound for the warp-per-block kernels)

@@ -160,6 +160,18 @@ size_t zl_seekable_frames(const void* src, size_t srcSize, int ptrs_are_device, 
  * below the result: dstSize_tooSmall.  ptrs_are_device: src and dst are device memory. */
 size_t zl_decompress_range(ZSTD_DCtx* dctx, void* dst, size_t dstCapacity, const void* src, size_t srcSize, size_t offset,
                            size_t length, int ptrs_are_device);
+/* Many ranges in one call: item i is bytes [offset[i], offset[i] + length[i]) of the seekable stream (src[i], srcSize[i]) into
+ * (dst[i], dstCapacity[i]).  result[i] receives what zl_decompress_range would return for that item alone -- the byte count, or the
+ * same error, checked in the same order: the table (prefix_unknown, corruption_detected), parameter_outOfBound, dstSize_tooSmall,
+ * dstBuffer_null, then the frames -- and dst[i] the same bytes; a failed item leaves its dst[i] unspecified.  Items with the same
+ * (src, srcSize) share one table read, and a frame touched by several items is decoded once; a frame that fails fails every item that
+ * touches it (an item touching several failing frames gets the error of the first in stream order), and the other items still get their
+ * bytes.  The arrays are host memory; with ptrs_are_device every src[i] and dst[i] is device memory on the context's device.  The
+ * destinations must not overlap each other or any source.  The whole call runs on the context's device, with its dictionary and
+ * ZSTD_d_forceIgnoreChecksum.  Returns 0 (also for n = 0), or an error for the whole call: null arguments, no device,
+ * memory_allocation (the scratch for the frames that are shared or only partly wanted), a failed launch. */
+size_t zl_decompress_ranges(ZSTD_DCtx* dctx, const void* const* src, const size_t* srcSize, const size_t* offset, const size_t* length,
+                            void* const* dst, const size_t* dstCapacity, size_t* result, size_t n, int ptrs_are_device);
 
 /* Several GPUs from ONE process (frames are independent: SURVEY.md 8e).  Batches of HOST buffers (zl_decompress_batch / zl_compress_batch, and
  * ZSTD_decompressDCtx on a multi-frame stream) are cut into contiguous frame ranges of about equal bytes, one per device, each handled by a helper

@@ -307,6 +307,65 @@ def zstd_decompress_range(src, offset, length, dctx=None, type="raw", out=None, 
     return res.decode("utf-8") if type == "string" else res
 
 
+def zstd_decompress_ranges(src, ranges, dctx=None, type="raw", out=None, **opts):
+    """Many byte ranges of one seekable stream in one call (zl_decompress_ranges): `ranges` is a sequence of (offset, length) pairs, each
+    clamped to the stream's end like zstd_decompress_range.  The table is read once and every touched frame is decoded once, however many
+    ranges share it.  A bytes-like `src` gives a list of bytes (str with type="string"); a CUDA tensor gives a list of CUDA uint8 tensors,
+    views into one tensor that holds the ranges back to back in request order -- `out` (a 1-D contiguous CUDA uint8 tensor) when given.
+    A failed range raises ZstdError naming the first failing range's index.  The table's checksums are verified unless
+    validate_checksum=False."""
+    import numpy as np
+    L = _lib.lib()
+    if dctx is None:
+        dctx = zstd_dctx(**opts)
+    buf, n, _keep, dev = _source(src)
+    rg = np.asarray(ranges, dtype=np.int64).reshape(-1, 2) if len(ranges) else np.zeros((0, 2), dtype=np.int64)
+    if (rg < 0).any():
+        raise ZstdError("zstd_decompress_ranges(): offsets and lengths must be >= 0")
+    k = len(rg)
+    if dev:
+        import torch
+        torch.cuda.current_stream(src.device).synchronize()               # the library reads on its own stream
+    try:
+        total = sum(d for _, d, _ in _seek_table(buf, n, dev))
+    except ZstdError:
+        total = 0                                                         # the call reports the table's error for every range
+    offs, lens = rg[:, 0].astype(np.uint64), rg[:, 1].astype(np.uint64)
+    want = np.clip(np.minimum(rg[:, 1], total - rg[:, 0]), 0, None).astype(np.uint64)
+    at = np.concatenate(([0], np.cumsum(want))).astype(np.uint64)          # each range's place in the packed output
+    if dev:
+        if out is None:
+            out = torch.empty(max(1, int(at[-1])), dtype=torch.uint8, device=src.device)
+        elif not getattr(out, "is_cuda", False) or out.dim() != 1 or not out.is_contiguous() or out.dtype != torch.uint8:
+            raise ZstdError("zstd_decompress_ranges(): out must be a 1-D contiguous torch.uint8 CUDA tensor")
+        else:
+            torch.cuda.current_stream(out.device).synchronize()
+        base = out.data_ptr()
+        caps = np.clip(np.minimum(want.astype(np.int64), out.numel() - at[:-1].astype(np.int64)), 0, None).astype(np.uint64)
+        dsts = base + at[:-1]
+        keep = None
+    else:
+        if out is not None:
+            raise ZstdError("zstd_decompress_ranges(): out is only taken for a CUDA source")
+        keep = [_new_bytes(int(w)) for w in want]
+        dsts = np.array([p for _, p in keep], dtype=np.uint64)
+        caps = want
+    srcs = np.full(k, C.cast(buf, C.c_void_p).value or 0, dtype=np.uint64)
+    sizes = np.full(k, n, dtype=np.uint64)
+    res = np.zeros(k, dtype=np.uint64)
+    pp, psz = C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)
+    _check(L.zl_decompress_ranges(dctx._p, srcs.ctypes.data_as(pp), sizes.ctypes.data_as(psz), offs.ctypes.data_as(psz),
+                                  lens.ctypes.data_as(psz), dsts.ctypes.data_as(pp), caps.ctypes.data_as(psz), res.ctypes.data_as(psz),
+                                  k, 1 if dev else 0), "zstd_decompress_ranges()")
+    failed = np.flatnonzero(res > np.uint64(2**64 - 121))                 # error codes are the last 120 values of size_t
+    if len(failed):
+        i = int(failed[0])
+        raise ZstdError(f"zstd_decompress_ranges(): range {i}: {L.ZSTD_getErrorName(int(res[i])).decode()}")
+    if dev:
+        return list(torch.split(out[:int(at[-1])], want.tolist()))
+    return [b.decode("utf-8") if type == "string" else b for b, _ in keep]
+
+
 def zstd_serialize(obj, cctx=None, frame_size=None, **opts):
     """zstd_serialize(robj, ..., cctx)  (R/serialize.R:56, src/serialize.c:41-118): serialize the object to bytes, compress them
     as one frame.  The reference serializes with R_Serialize (version 3, binary); R is not in this image, so this host mirror

@@ -212,7 +212,8 @@ struct ZSTD_DCtx_s {
     size_t sOutPos = 0;
     ZlDevBuf dRaw, dDescs, dInfos, dResults, dHdr, dRec, dCk, dLit, dNorm, dUnits, dCounters, dLargeIdx, dLb, dLc, dParent, dRemain, dSrc, dDst;
     ZlPinBuf hDescs, hResults, hLargeIdx, hRemain;
-    ZlDevBuf dSeek; std::vector<u8> hSeek;  // zl_decompress_range: the edge frames of a range, decoded whole (device / host buffers)
+    ZlDevBuf dSeek; std::vector<u8> hSeek;  // zl_decompress_ranges: the scratch frames, decoded whole (device / host buffers)
+    ZlDevBuf dScatter; ZlPinBuf hScatter;  // zl_decompress_ranges: the copy-out items of device buffers
     std::vector<cudaEvent_t> sliceDone;    // staged host buffers: the copy back of a slice has landed
     // devices: the context's own (bound on first use) and, for batches of host buffers, the helpers on the other GPUs of the box
     int device = -1, gpus = 0;             // gpus: 0 = ZSTDLITE_GPUS (default 1)
@@ -237,9 +238,9 @@ ZL_EXPORT size_t ZSTD_freeDCtx(ZSTD_DCtx* c)
     for (ZSTD_DCtx_s* k : c->kids) ZSTD_freeDCtx(k);
     c->kids.clear();
     ZlDeviceGuard guard(c->device);
-    ZlDevBuf* bufs[] = {&c->dDictContent, &c->dDict, &c->dRaw, &c->dDescs, &c->dInfos, &c->dResults, &c->dHdr, &c->dRec, &c->dCk, &c->dLit, &c->dNorm, &c->dUnits, &c->dCounters, &c->dLargeIdx, &c->dLb, &c->dLc, &c->dParent, &c->dRemain, &c->dSrc, &c->dDst, &c->dSeek};
+    ZlDevBuf* bufs[] = {&c->dDictContent, &c->dDict, &c->dRaw, &c->dDescs, &c->dInfos, &c->dResults, &c->dHdr, &c->dRec, &c->dCk, &c->dLit, &c->dNorm, &c->dUnits, &c->dCounters, &c->dLargeIdx, &c->dLb, &c->dLc, &c->dParent, &c->dRemain, &c->dSrc, &c->dDst, &c->dSeek, &c->dScatter};
     for (ZlDevBuf* b : bufs) b->release();
-    c->hDescs.release(); c->hResults.release(); c->hLargeIdx.release(); c->hRemain.release();
+    c->hDescs.release(); c->hResults.release(); c->hLargeIdx.release(); c->hRemain.release(); c->hScatter.release();
     for (cudaEvent_t e : c->sliceDone) if (e) cudaEventDestroy(e);
     if (c->ev0) { cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1); }
     for (cudaEvent_t e : c->stageEv) if (e) cudaEventDestroy(e);
@@ -769,47 +770,87 @@ ZL_EXPORT size_t zl_seekable_frames(const void* src, size_t srcSize, int ptrs_ar
     return t.n;
 }
 
-// Bytes [offset, offset + length) of a seekable stream's content: the frames the range touches are decoded as one batch on the context's
-// device, the interior ones straight into dst, the one or two edge frames whole into the context's scratch, from which the wanted bytes are
-// copied.  Every frame must produce exactly its table size; the table's checksums are verified in the checksum kernels.
-ZL_EXPORT size_t zl_decompress_range(ZSTD_DCtx* c, void* dst, size_t dstCap, const void* src, size_t srcSize, size_t offset, size_t length,
-                                     int ptrs_are_device)
+// Many byte ranges of seekable streams in one batch on the context's device (zl_seek.h, zl_ranges_plan): each distinct stream's table is
+// read once, every touched frame is decoded once -- straight into its item's dst when that item alone touches it and covers it whole,
+// else whole into the context's scratch -- and the pieces in scratch are copied out by one kernel launch (device buffers) or on the host.
+// Frames of streams whose tables have checksums are checked against them in a batch of their own: the engine's expect array covers a
+// whole batch.
+ZL_EXPORT size_t zl_decompress_ranges(ZSTD_DCtx* c, const void* const* src, const size_t* srcSize, const size_t* offset, const size_t* length,
+                                      void* const* dst, const size_t* dstCap, size_t* result, size_t n, int ptrs_are_device)
 {
     if (!c) return ZL_ERROR(GENERIC);
+    if (!n) return 0;
+    if (!src || !srcSize || !offset || !length || !dst || !dstCap || !result) return ZL_ERROR(GENERIC);
     const bool dev = ptrs_are_device != 0;
     ZlDeviceGuard guard(zl_bind_device(&c->device));
     if (!guard.ok) return ZL_ERROR(GENERIC);
     if (!zl_ctx_stream(&c->stream, &c->ownStream, &c->ev0, &c->ev1)) return ZL_ERROR(memory_allocation);
     cudaStream_t st = c->stream;
-    ZlSeekTable t;
-    if (const size_t r = zl_seek_read(t, src, srcSize, dev, st)) return r;
-    ZlSeekPlan p;
-    if (const size_t r = zl_seek_plan_range(p, t, offset, length)) return r;
-    if (p.bytes > dstCap) return ZL_ERROR(dstSize_tooSmall);
-    if (!p.bytes) return 0;
-    if (!dst) return ZL_ERROR(dstBuffer_null);
+    std::vector<size_t> streamOf(n), firstItem;
+    const size_t ns = zl_ranges_streams(src, srcSize, n, streamOf.data(), firstItem);
+    std::vector<ZlSeekTable> tables(ns);
+    std::vector<size_t> tableErr(ns);
+    for (size_t s = 0; s < ns; s++) tableErr[s] = zl_seek_read(tables[s], src[firstItem[s]], srcSize[firstItem[s]], dev, st);
+    ZlRangesPlan p;
+    zl_ranges_plan(p, tables, tableErr, streamOf.data(), offset, length, dst, dstCap, n);
+    const size_t nd = p.decodes.size();
+    std::vector<size_t> dres(nd, 0);
+    if (!nd) { zl_ranges_results(p, dres.data(), result, n); return 0; }
     u8* scratch = nullptr;
     if (dev) { if (!c->dSeek.reserve(p.scratchBytes + 64)) return ZL_ERROR(memory_allocation); scratch = c->dSeek.as<u8>(); }
     else { if (c->hSeek.size() < p.scratchBytes + 64) c->hSeek.resize(p.scratchBytes + 64); scratch = c->hSeek.data(); }
-    const size_t n = p.last - p.first;
-    std::vector<const void*> fsrc(n); std::vector<void*> fdst(n); std::vector<size_t> fsize(n), fcap(n), fres(n, 0);
-    for (size_t j = 0; j < n; j++) {
-        const size_t f = p.first + j;
-        fsrc[j] = (const u8*)src + t.cOff[f]; fsize[j] = t.cSize[f]; fcap[j] = t.dSize[f];
-        fdst[j] = (p.edge[j] ? scratch : (u8*)dst) + p.place[j];
+    std::vector<const void*> fsrc(nd); std::vector<void*> fdst(nd); std::vector<size_t> fsize(nd), fcap(nd), fres(nd, 0), id(nd);
+    std::vector<u32> expect;
+    for (int withSums = 0; withSums < 2; withSums++) {              // streams without table checksums, then those with
+        size_t m = 0;
+        expect.clear();
+        for (size_t k = 0; k < nd; k++) {
+            const ZlRangeDecode& d = p.decodes[k];
+            const ZlSeekTable& t = tables[d.stream];
+            if (t.checksums != (withSums != 0)) continue;
+            fsrc[m] = (const u8*)src[firstItem[d.stream]] + t.cOff[d.frame]; fsize[m] = t.cSize[d.frame]; fcap[m] = d.size;
+            fdst[m] = (d.item == ZL_RANGE_SCRATCH ? scratch : (u8*)dst[d.item]) + d.place;
+            if (withSums) expect.push_back(t.checksum[d.frame]);
+            id[m++] = k;
+        }
+        if (!m) continue;
+        const size_t r = zl_decompress_batch_one(c, fsrc.data(), fsize.data(), fdst.data(), fcap.data(), fres.data(), m, dev,
+                                                 withSums ? expect.data() : nullptr);
+        if (zl_is_error(r)) return r;
+        for (size_t j = 0; j < m; j++) dres[id[j]] = fres[j];
     }
-    const size_t r = zl_decompress_batch_one(c, fsrc.data(), fsize.data(), fdst.data(), fcap.data(), fres.data(), n, dev,
-                                             t.checksums ? t.checksum.data() + p.first : nullptr);
-    if (zl_is_error(r)) return r;
-    for (size_t j = 0; j < n; j++) {
-        if (zl_is_error(fres[j])) return fres[j];
-        if (fres[j] != fcap[j]) return ZL_ERROR(corruption_detected);       // the table's Decompressed_Size is wrong
+    zl_ranges_results(p, dres.data(), result, n);
+    // the pieces of the items that succeeded
+    if (dev) {
+        size_t items = 0;
+        for (const ZlRangePiece& q : p.pieces) if (!zl_is_error(result[q.item])) items += (q.bytes + ZL_SCATTER_BYTES - 1) / ZL_SCATTER_BYTES;
+        if (items) {
+            if (!c->hScatter.reserve(items * sizeof(ZlScatterItem)) || !c->dScatter.reserve(items * sizeof(ZlScatterItem))) return ZL_ERROR(memory_allocation);
+            ZlScatterItem* h = c->hScatter.as<ZlScatterItem>();
+            size_t w = 0;
+            for (const ZlRangePiece& q : p.pieces) {
+                if (zl_is_error(result[q.item])) continue;
+                for (u64 o = 0; o < q.bytes; o += ZL_SCATTER_BYTES)
+                    h[w++] = {scratch + q.from + o, (u8*)dst[q.item] + q.outOff + o, (u32)std::min<u64>(q.bytes - o, ZL_SCATTER_BYTES)};
+            }
+            cudaMemcpyAsync(c->dScatter.p, h, items * sizeof(ZlScatterItem), cudaMemcpyHostToDevice, st);
+            if (zl_launch_range_scatter(c->dScatter.as<ZlScatterItem>(), (u32)items, st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
+            c->launches += 1;
+            if (cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
+        }
+    } else {
+        std::vector<ZlCopySeg> segs;
+        for (const ZlRangePiece& q : p.pieces) if (!zl_is_error(result[q.item])) segs.push_back({(u8*)dst[q.item] + q.outOff, scratch + q.from, q.bytes});
+        ZlCopyPool::get().run(segs);
     }
-    for (size_t k = 0; k < p.nEdges; k++) {
-        const ZlSeekEdge& e = p.edges[k];
-        if (dev) cudaMemcpyAsync((u8*)dst + e.outOff, scratch + e.scratchOff + e.skip, e.take, cudaMemcpyDeviceToDevice, st);
-        else memcpy((u8*)dst + e.outOff, scratch + e.scratchOff + e.skip, e.take);
-    }
-    if (dev && cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
-    return p.bytes;
+    return 0;
+}
+
+// One range: the one-item case of zl_decompress_ranges.
+ZL_EXPORT size_t zl_decompress_range(ZSTD_DCtx* c, void* dst, size_t dstCap, const void* src, size_t srcSize, size_t offset, size_t length,
+                                     int ptrs_are_device)
+{
+    size_t result = 0;
+    const size_t r = zl_decompress_ranges(c, &src, &srcSize, &offset, &length, &dst, &dstCap, &result, 1, ptrs_are_device);
+    return zl_is_error(r) ? r : result;
 }

@@ -2,6 +2,7 @@
 //   K1a zl_k_literals / K1b zl_k_sequences   quad-per-frame entropy decode -> literal / record / header arenas
 //   K2 zl_k_execute   warp-per-frame sequence execution -> frame output
 //   K3 zl_k_checksum  quad-per-frame XXH64 of the output, compared with the frame trailer (and a seek table's checksum)
+//   zl_k_range_scatter  warp-per-piece copy-out of zl_decompress_ranges
 #include "zl_dec_entropy.cuh"
 #include "zl_dec_exec.cuh"
 #include "zl_dec_large.cuh"
@@ -408,6 +409,17 @@ zl_k_xxh64_large(const u8* const* __restrict__ ptrs, const u32* __restrict__ siz
     if (threadIdx.x == 0) out[i] = h;
 }
 
+// copy-out of zl_decompress_ranges: the pieces of the frames decoded into scratch, cut into items of <= ZL_SCATTER_BYTES, a warp each
+#define ZL_SCATTER_WARPS 4
+__global__ void __launch_bounds__(ZL_SCATTER_WARPS * 32)
+zl_k_range_scatter(const ZlScatterItem* __restrict__ items, u32 n)
+{
+    const u32 i = blockIdx.x * ZL_SCATTER_WARPS + (threadIdx.x >> 5);
+    if (i >= n) return;
+    const ZlScatterItem it = items[i];
+    zl_warp_copy(it.dst, it.src, it.bytes, threadIdx.x & 31);
+}
+
 // ---- launchers ---------------------------------------------------------------------------------------
 size_t zl_literals_smem_bytes() { return ZL_QUADS_PER_WARP * sizeof(ZlLitSm) + (ZL_LIT_RING ? 32 * 16 * ZL_LIT_RING_NS : 0); }
 static size_t zl_literals_smem_dict_bytes() { return zl_literals_smem_bytes() + 2048 * sizeof(u16); }      // + the dictionary's Huffman table
@@ -602,6 +614,13 @@ cudaError_t zl_launch_build_descs(const u64* raw, u32 cnt, ZlFrameDesc* descs, u
 {
     if (!cnt) return cudaSuccess;
     zl_k_build_descs<<<1, ZL_BUILD_THREADS, 0, st>>>(raw, cnt, descs, lit0, rec0, hdr0, worst ? 1 : 0);
+    return cudaGetLastError();
+}
+
+cudaError_t zl_launch_range_scatter(const ZlScatterItem* items, u32 n, cudaStream_t st)
+{
+    if (!n) return cudaSuccess;
+    zl_k_range_scatter<<<(n + ZL_SCATTER_WARPS - 1) / ZL_SCATTER_WARPS, ZL_SCATTER_WARPS * 32, 0, st>>>(items, n);
     return cudaGetLastError();
 }
 

@@ -105,6 +105,10 @@ cudaError_t zl_launch_decode(const ZlDecodeLaunch& L, cudaStream_t st);
 // descriptors of a slice of small frames from the caller's arrays (raw = [src | dst | srcSize | dstCap], cnt u64 each), zl_dec_kernels.cu
 cudaError_t zl_launch_build_descs(const u64* raw, u32 cnt, ZlFrameDesc* descs, u64 lit0, u64 rec0, u64 hdr0, bool worst, cudaStream_t st);
 cudaError_t zl_launch_xxh64(const u8* const* ptrs, const u32* sizes, u64* out, u32 n, cudaStream_t st, bool anyLarge = false);
+// copy-out of zl_decompress_ranges: one warp per item (device memory, n of them), each at most ZL_SCATTER_BYTES
+#define ZL_SCATTER_BYTES (64u << 10)
+struct ZlScatterItem { const u8* src; u8* dst; u32 bytes; };
+cudaError_t zl_launch_range_scatter(const ZlScatterItem* items, u32 n, cudaStream_t st);
 
 // ---- compression --------------------------------------------------------------------------------------------------
 #include "zl_enc_entropy.cuh"

@@ -1,6 +1,6 @@
 // zl_seek.h -- the seek table of Zstandard's seekable format (zstd's contrib/seekable_format) and the range plan built on it: which
-// frames a byte range of the decompressed stream touches, where each is decoded and what is copied out of the edge frames.  No CUDA call:
-// tests/host/seek_check.cpp checks it on the CPU.
+// frames a byte range of the decompressed stream touches, where each is decoded and what is copied out of the edge frames -- and the plan
+// of many ranges in one batch.  No CUDA call: tests/host/seek_check.cpp and tests/host/ranges_check.cpp check it on the CPU.
 //
 // A seekable stream is N independent Zstandard frames followed by one skippable frame, the seek table:
 //   magic 0x184D2A5E | Frame_Size u32 | N entries {Compressed_Size u32, Decompressed_Size u32[, Checksum u32]} |
@@ -9,6 +9,7 @@
 // are reserved and must be 0.
 #pragma once
 #include <algorithm>
+#include <map>
 #include "zl_host.h"              // (and <vector>)
 
 #define ZL_SEEK_TABLE_MAGIC 0x184D2A5Eu
@@ -119,4 +120,105 @@ static inline size_t zl_seek_plan_range(ZlSeekPlan& p, const ZlSeekTable& t, u64
         p.edge.push_back(isEdge ? 1 : 0);
     }
     return 0;
+}
+
+// ---- many ranges (zl_decompress_ranges) ------------------------------------------------------------------------------------------
+// Item i asks for bytes [offset[i], offset[i] + length[i]) of stream streamOf[i].  Every (stream, frame) an item touches is decoded once:
+// straight into dst[item] when exactly one item touches it and covers it whole, else whole into scratch, from which each item that
+// touches it gets a piece.
+#define ZL_RANGE_SCRATCH (~(size_t)0)
+struct ZlRangeDecode { size_t stream, frame, item; u64 place; u32 size; };   // item == ZL_RANGE_SCRATCH: place is in the scratch
+struct ZlRangePiece { size_t item; u64 from, bytes, outOff; };             // scratch [from, from + bytes) -> dst[item] + outOff
+struct ZlRangesPlan {
+    std::vector<size_t> result;             // per item: its pre-decode error, or the bytes it returns if all its frames decode
+    std::vector<ZlRangeDecode> decodes;     // by stream, then frame
+    std::vector<size_t> touchStart, touch;  // item i touches decodes touch[touchStart[i] .. touchStart[i + 1]), in stream order
+    std::vector<ZlRangePiece> pieces;       // none of 0 bytes
+    u64 scratchBytes = 0;                   // every scratch frame at a 16-byte-aligned place
+};
+
+// Groups items by (src, srcSize): streamOf[i] = its stream, numbered in order of first appearance; firstItem[s] = an item of stream s.
+static inline size_t zl_ranges_streams(const void* const* src, const size_t* srcSize, size_t n, size_t* streamOf, std::vector<size_t>& firstItem)
+{
+    std::map<std::pair<const void*, size_t>, size_t> seen;
+    firstItem.clear();
+    for (size_t i = 0; i < n; i++) {
+        auto it = seen.emplace(std::make_pair(src[i], srcSize[i]), firstItem.size());
+        if (it.second) firstItem.push_back(i);
+        streamOf[i] = it.first->second;
+    }
+    return firstItem.size();
+}
+
+// tables[s] / tableErr[s]: stream s's table, or the error reading it.  Each item is checked as zl_decompress_range checks a range, in the
+// same order: table error, parameter_outOfBound, dstSize_tooSmall, (0 bytes: 0), dstBuffer_null.  A rejected item adds no frames.
+static inline void zl_ranges_plan(ZlRangesPlan& p, const std::vector<ZlSeekTable>& tables, const std::vector<size_t>& tableErr,
+                                  const size_t* streamOf, const size_t* offset, const size_t* length, void* const* dst, const size_t* dstCap,
+                                  size_t n)
+{
+    p = ZlRangesPlan();
+    p.result.assign(n, 0);
+    const size_t ns = tables.size();
+    std::vector<size_t> first(n, 0), last(n, 0);
+    std::vector<size_t> lo(ns, ~(size_t)0), hi(ns, 0);                       // per stream: the frames any accepted item touches
+    for (size_t i = 0; i < n; i++) {
+        const size_t s = streamOf[i];
+        if (zl_is_error(tableErr[s])) { p.result[i] = tableErr[s]; continue; }
+        ZlSeekPlan sp;
+        if (const size_t r = zl_seek_plan_range(sp, tables[s], offset[i], length[i])) { p.result[i] = r; continue; }
+        if (sp.bytes > dstCap[i]) { p.result[i] = ZL_ERROR(dstSize_tooSmall); continue; }
+        if (!sp.bytes) continue;
+        if (!dst[i]) { p.result[i] = ZL_ERROR(dstBuffer_null); continue; }
+        p.result[i] = sp.bytes; first[i] = sp.first; last[i] = sp.last;
+        lo[s] = std::min(lo[s], sp.first); hi[s] = std::max(hi[s], sp.last);
+    }
+    // mark[s][f - lo[s]]: 0 untouched, i + 1 touched by item i alone, SHARED by several; then the decode's index
+    const size_t SHARED = ~(size_t)0;
+    std::vector<std::vector<size_t>> mark(ns);
+    for (size_t s = 0; s < ns; s++) if (lo[s] < hi[s]) mark[s].assign(hi[s] - lo[s], 0);
+    for (size_t i = 0; i < n; i++) {
+        std::vector<size_t>& m = mark[streamOf[i]];
+        for (size_t f = first[i]; f < last[i]; f++) { size_t& k = m[f - lo[streamOf[i]]]; k = k ? SHARED : i + 1; }
+    }
+    for (size_t s = 0; s < ns; s++) {
+        const ZlSeekTable& t = tables[s];
+        for (size_t f = lo[s]; f < hi[s]; f++) {
+            size_t& k = mark[s][f - lo[s]];
+            if (!k) continue;
+            ZlRangeDecode d{s, f, ZL_RANGE_SCRATCH, 0, t.dSize[f]};
+            const size_t i = k - 1;
+            if (k != SHARED && t.dOff[f] >= offset[i] && t.dOff[f + 1] <= offset[i] + p.result[i]) { d.item = i; d.place = t.dOff[f] - offset[i]; }
+            else { d.place = p.scratchBytes; p.scratchBytes += (t.dSize[f] + 15) & ~(u64)15; }
+            k = p.decodes.size();
+            p.decodes.push_back(d);
+        }
+    }
+    p.touchStart.assign(n + 1, 0);
+    for (size_t i = 0; i < n; i++) {
+        p.touchStart[i] = p.touch.size();
+        const size_t s = streamOf[i];
+        const ZlSeekTable& t = tables[s];
+        for (size_t f = first[i]; f < last[i]; f++) {
+            const size_t id = mark[s][f - lo[s]];
+            p.touch.push_back(id);
+            if (p.decodes[id].item != ZL_RANGE_SCRATCH) continue;
+            const u64 a = std::max((u64)offset[i], t.dOff[f]), b = std::min((u64)offset[i] + p.result[i], t.dOff[f + 1]);
+            if (b > a) p.pieces.push_back({i, p.decodes[id].place + (a - t.dOff[f]), b - a, a - offset[i]});
+        }
+    }
+    p.touchStart[n] = p.touch.size();
+}
+
+// The items' results from the engine's per-decode results: an item fails with the first of its frames (in stream order) that failed, or
+// with corruption_detected when that frame produced a size other than its table's Decompressed_Size.
+static inline void zl_ranges_results(const ZlRangesPlan& p, const size_t* decodeRes, size_t* result, size_t n)
+{
+    for (size_t i = 0; i < n; i++) {
+        result[i] = p.result[i];
+        for (size_t j = p.touchStart[i]; j < p.touchStart[i + 1]; j++) {
+            const size_t id = p.touch[j], r = decodeRes[id];
+            if (zl_is_error(r)) { result[i] = r; break; }
+            if (r != p.decodes[id].size) { result[i] = ZL_ERROR(corruption_detected); break; }
+        }
+    }
 }

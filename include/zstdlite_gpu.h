@@ -173,6 +173,27 @@ size_t zl_decompress_range(ZSTD_DCtx* dctx, void* dst, size_t dstCapacity, const
 size_t zl_decompress_ranges(ZSTD_DCtx* dctx, const void* const* src, const size_t* srcSize, const size_t* offset, const size_t* length,
                             void* const* dst, const size_t* dstCapacity, size_t* result, size_t n, int ptrs_are_device);
 
+/* ---- streams in device memory (any Zstandard stream: no seek table needed) ----
+ * zl_device_frames: every frame of a Zstandard stream in DEVICE memory on the context's device (concatenated frames, skippable frames
+ * included), found on the device.  Returns the number of frames N, or an error: the same code ZSTD_decompressDCtx would return for the
+ * stream's structure -- prefix_unknown at offset 0; srcSize_wrong for a non-magic at a later frame boundary, a truncated header or
+ * block, or 1-4 trailing bytes; corruption_detected for block type 3; frameParameter_unsupported; frameParameter_windowTooLarge.
+ * When cap >= N: cOff[k] / cSize[k] receive frame k's offset and compressed size in src, dSize[k] its header's content size:
+ * ZSTD_CONTENTSIZE_UNKNOWN when the header has none, 0 for a skippable frame (ZSTD_getFrameContentSize's convention).  Each array is
+ * optional.  Call with cap = 0 first to learn N.  srcSize = 0 gives 0. */
+size_t zl_device_frames(ZSTD_DCtx* dctx, const void* src, size_t srcSize, unsigned long long* cOff,
+                        unsigned long long* cSize, unsigned long long* dSize, size_t cap);
+/* ZSTD_decompressDCtx for src and dst in device memory on the context's device: every frame, with the context's dictionary and
+ * ZSTD_d_forceIgnoreChecksum.  Returns the bytes written or an error code: the same value, and on success the same bytes, as
+ * ZSTD_decompressDCtx on host copies, with the structural errors above and dstSize_tooSmall when the content sizes overflow
+ * dstCapacity.  One difference of order: every frame is found before any is decoded, whereas ZSTD_decompressDCtx decodes a frame
+ * without a content size as soon as it reaches it -- so for a stream with a decode error at or before such a frame AND a structural
+ * error after it, this call reports the structural error.  Frames without a content size are decoded into scratch of
+ * min(blocks x blockSizeMax, dstCapacity) bytes each (at most 2 GiB per frame: memory_allocation beyond) and then moved into place,
+ * so this call decodes such a frame where ZSTD_decompressDCtx, which offers it all the capacity left, refuses more than 2 GiB.
+ * Neither call spreads over several GPUs. */
+size_t zl_decompress_device(ZSTD_DCtx* dctx, void* dst, size_t dstCapacity, const void* src, size_t srcSize);
+
 /* Several GPUs from ONE process (frames are independent: SURVEY.md 8e).  Batches of HOST buffers (zl_decompress_batch / zl_compress_batch, and
  * ZSTD_decompressDCtx on a multi-frame stream) are cut into contiguous frame ranges of about equal bytes, one per device, each handled by a helper
  * context on its own host thread; no collective, no peer traffic.  How many GPUs: zl_dctx_set_gpus(n) for a DCtx; num_threads (ZSTD_c_nbWorkers) >= 2 for

@@ -81,6 +81,9 @@ def lib():
         "zl_seekable_frames": (sz, [vp, sz, C.c_int, C.POINTER(C.c_uint), C.POINTER(C.c_uint), C.POINTER(C.c_uint), sz, C.POINTER(C.c_int)]),
         "zl_decompress_range": (sz, [vp, vp, sz, vp, sz, sz, sz, C.c_int]),
         "zl_decompress_ranges": (sz, [vp, pp, psz, psz, psz, pp, psz, psz, sz, C.c_int]),
+        # streams in device memory
+        "zl_device_frames": (sz, [vp, vp, sz, C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong), sz]),
+        "zl_decompress_device": (sz, [vp, vp, sz, vp, sz]),
         "zl_cctx_set_stream": (sz, [vp, vp]), "zl_cctx_launch_count": (C.c_ulonglong, [vp]), "zl_cctx_last_kernel_ms": (C.c_double, [vp]),
         "zl_cctx_last_stage_ms": (C.c_double, [vp, C.c_int]),
         "zl_cctx_allow_level_fallback": (sz, [vp, C.c_int]), "zl_cctx_engine_level": (C.c_int, [vp]),
@@ -117,4 +120,5 @@ EXPORTED_SYMBOLS = [
     "zl_dctx_launch_count", "zl_cctx_launch_count", "zl_dctx_last_kernel_ms", "zl_cctx_last_kernel_ms", "zl_dctx_last_stage_ms", "zl_cctx_last_stage_ms", "zl_backend_string",
     "zl_cctx_allow_level_fallback", "zl_cctx_engine_level", "zl_dctx_set_gpus",
     "zl_compress_seekable", "zl_compress_seekable_bound", "zl_seekable_frames", "zl_decompress_range", "zl_decompress_ranges",
+    "zl_device_frames", "zl_decompress_device",
 ]

@@ -9,6 +9,7 @@
 #include "../../include/zstdlite_gpu.h"
 #include "zl_batch_plan.h"            // (and zl_host.h)
 #include "zl_seek.h"
+#include "zl_stream_index.h"
 #include "zl_dec_entropy.cuh"     // ZL_HD table builders reused to digest dictionaries on the host (zstd.c:42053)
 
 #define ZL_EXPORT extern "C" __attribute__((visibility("default")))
@@ -59,76 +60,19 @@ ZL_ALIAS(const char*, ZSTD_versionString, (void))
 // ---------------------------------------------------------------------------------------------- frame introspection (host)
 size_t zl_host_frame_header(ZlHostFrameHeader* h, const void* srcv, size_t srcSize)
 {
-    const u8* ip = (const u8*)srcv;
-    memset(h, 0, sizeof(*h));
-    if (srcSize > 0 && ip == nullptr) return ZL_ERROR(GENERIC);
-    if (srcSize < 5) {                               // zstd.c:41061-41077: a too-short prefix must still look like a magic number
-        if (srcSize > 0) {
-            u8 m[4] = {0x28, 0xB5, 0x2F, 0xFD};
-            u8 sk[4] = {0x50, 0x2A, 0x4D, 0x18};
-            bool a = true, b = true;
-            for (size_t i = 0; i < srcSize && i < 4; i++) { if (ip[i] != m[i]) a = false; if (i > 0 && ip[i] != sk[i]) b = false; if (i == 0 && (ip[i] & 0xF0) != 0x50) b = false; }
-            if (!a && !b) return ZL_ERROR(prefix_unknown);
-        }
-        return 5;
-    }
-    u32 magic = zl_rd32(ip);
-    if ((magic & 0xFFFFFFF0u) == ZL_MAGIC_SKIP) {
-        if (srcSize < 8) return 8;
-        h->skippable = 1; h->contentSize = zl_rd32(ip + 4); h->headerSize = 8;
-        return 0;
-    }
-    if (magic != ZL_MAGIC) return ZL_ERROR(prefix_unknown);
-    u32 fhd = ip[4], didCode = fhd & 3, single = (fhd >> 5) & 1, fcsID = fhd >> 6;
-    u32 didSz = didCode == 3 ? 4 : didCode, fcsSz = fcsID == 0 ? (single ? 1u : 0u) : (1u << fcsID);
-    u32 hs = 5 + (single ? 0 : 1) + didSz + fcsSz;
-    if (srcSize < hs) return hs;
-    h->headerSize = hs;
-    if (fhd & 8) return ZL_ERROR(frameParameter_unsupported);
-    u32 p = 5; u64 window = 0;
-    if (!single) {
-        u32 wl = ip[p++], wlog = (wl >> 3) + 10;
-        if (wlog > 31) return ZL_ERROR(frameParameter_windowTooLarge);
-        window = 1ull << wlog; window += (window >> 3) * (wl & 7);
-    }
-    u32 did = 0;
-    if (didSz == 1) did = ip[p]; else if (didSz == 2) did = zl_rd16(ip + p); else if (didSz == 4) did = zl_rd32(ip + p);
-    p += didSz;
-    u64 fcs = ZSTD_CONTENTSIZE_UNKNOWN;
-    if (fcsID == 0) { if (single) fcs = ip[p]; } else if (fcsID == 1) fcs = zl_rd16(ip + p) + 256; else if (fcsID == 2) fcs = zl_rd32(ip + p); else fcs = zl_rd64(ip + p);
-    if (single) window = fcs;
-    h->contentSize = fcs; h->windowSize = window;
-    h->blockSizeMax = (unsigned)(window < ZL_BLOCKSIZE_MAX ? window : ZL_BLOCKSIZE_MAX);
-    h->dictID = did; h->checksumFlag = (fhd >> 2) & 1;
-    return 0;
+    if (srcSize > 0 && srcv == nullptr) { memset(h, 0, sizeof(*h)); return ZL_ERROR(GENERIC); }
+    return zl_frame_head(h, (const u8*)srcv, srcSize);
 }
 
+// the extent rule shared with the device index (zl_stream_index.h), without a step cap
 size_t zl_host_find_frame_size(const void* srcv, size_t srcSize, unsigned* nblocksOut)
 {
-    const u8* ip = (const u8*)srcv;
     if (nblocksOut) *nblocksOut = 0;
-    if (srcSize >= 8 && (zl_rd32(ip) & 0xFFFFFFF0u) == ZL_MAGIC_SKIP) {         // zstd.c:41188
-        u64 sz = (u64)zl_rd32(ip + 4) + 8;
-        if (sz > srcSize) return ZL_ERROR(srcSize_wrong);
-        return (size_t)sz;
-    }
-    ZlHostFrameHeader h;
-    size_t r = zl_host_frame_header(&h, srcv, srcSize);
-    if (zl_is_error(r)) return r;
-    if (r > 0) return ZL_ERROR(srcSize_wrong);
-    size_t pos = h.headerSize; unsigned nb = 0;
-    for (;;) {                                                                   // zstd.c:41370-41384
-        if (srcSize - pos < 3) return ZL_ERROR(srcSize_wrong);
-        u32 bh = zl_rd24(ip + pos), last = bh & 1, type = (bh >> 1) & 3, cs = bh >> 3;
-        if (type == 3) return ZL_ERROR(corruption_detected);
-        if (type == 1) cs = 1;
-        if (3 + (size_t)cs > srcSize - pos) return ZL_ERROR(srcSize_wrong);
-        pos += 3 + cs; nb++;
-        if (last) break;
-    }
-    if (h.checksumFlag) { if (srcSize - pos < 4) return ZL_ERROR(srcSize_wrong); pos += 4; }
-    if (nblocksOut) *nblocksOut = nb;
-    return pos;
+    if (srcSize > 0 && srcv == nullptr) return ZL_ERROR(GENERIC);
+    const ZlExtent x = zl_frame_extent((const u8*)srcv, srcSize, 0);
+    if (x.state) return x.err;
+    if (nblocksOut) *nblocksOut = x.nblocks;
+    return (size_t)x.end;
 }
 
 ZL_EXPORT size_t ZSTD_getFrameHeader(ZSTD_frameHeader* z, const void* src, size_t srcSize)
@@ -214,6 +158,7 @@ struct ZSTD_DCtx_s {
     ZlPinBuf hDescs, hResults, hLargeIdx, hRemain;
     ZlDevBuf dSeek; std::vector<u8> hSeek;  // zl_decompress_ranges: the scratch frames, decoded whole (device / host buffers)
     ZlDevBuf dScatter; ZlPinBuf hScatter;  // zl_decompress_ranges: the copy-out items of device buffers
+    ZlDevBuf dIdx, dIdxTile, dIdxFrames; ZlPinBuf hIdx;   // frame index of a device stream (zl_device_frames): candidates, tiles, records
     std::vector<cudaEvent_t> sliceDone;    // staged host buffers: the copy back of a slice has landed
     // devices: the context's own (bound on first use) and, for batches of host buffers, the helpers on the other GPUs of the box
     int device = -1, gpus = 0;             // gpus: 0 = ZSTDLITE_GPUS (default 1)
@@ -238,9 +183,9 @@ ZL_EXPORT size_t ZSTD_freeDCtx(ZSTD_DCtx* c)
     for (ZSTD_DCtx_s* k : c->kids) ZSTD_freeDCtx(k);
     c->kids.clear();
     ZlDeviceGuard guard(c->device);
-    ZlDevBuf* bufs[] = {&c->dDictContent, &c->dDict, &c->dRaw, &c->dDescs, &c->dInfos, &c->dResults, &c->dHdr, &c->dRec, &c->dCk, &c->dLit, &c->dNorm, &c->dUnits, &c->dCounters, &c->dLargeIdx, &c->dLb, &c->dLc, &c->dParent, &c->dRemain, &c->dSrc, &c->dDst, &c->dSeek, &c->dScatter};
+    ZlDevBuf* bufs[] = {&c->dDictContent, &c->dDict, &c->dRaw, &c->dDescs, &c->dInfos, &c->dResults, &c->dHdr, &c->dRec, &c->dCk, &c->dLit, &c->dNorm, &c->dUnits, &c->dCounters, &c->dLargeIdx, &c->dLb, &c->dLc, &c->dParent, &c->dRemain, &c->dSrc, &c->dDst, &c->dSeek, &c->dScatter, &c->dIdx, &c->dIdxTile, &c->dIdxFrames};
     for (ZlDevBuf* b : bufs) b->release();
-    c->hDescs.release(); c->hResults.release(); c->hLargeIdx.release(); c->hRemain.release(); c->hScatter.release();
+    c->hDescs.release(); c->hResults.release(); c->hLargeIdx.release(); c->hRemain.release(); c->hScatter.release(); c->hIdx.release();
     for (cudaEvent_t e : c->sliceDone) if (e) cudaEventDestroy(e);
     if (c->ev0) { cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1); }
     for (cudaEvent_t e : c->stageEv) if (e) cudaEventDestroy(e);
@@ -853,4 +798,151 @@ ZL_EXPORT size_t zl_decompress_range(ZSTD_DCtx* c, void* dst, size_t dstCap, con
     size_t result = 0;
     const size_t r = zl_decompress_ranges(c, &src, &srcSize, &offset, &length, &dst, &dstCap, &result, 1, ptrs_are_device);
     return zl_is_error(r) ? r : result;
+}
+
+// ---------------------------------------------------------------------------------------------- streams in device memory (zl_stream_index.h)
+// The frame index of a stream in device memory on the context's device: *status receives 0 or the stream's structural error (as
+// ZSTD_decompressDCtx reports it), frames every complete frame of the chain from offset 0.  Returns 0, or an error of the call itself.
+static size_t zl_device_index(ZSTD_DCtx* c, const u8* src, size_t srcSize, std::vector<ZlStreamFrame>& frames, size_t* status)
+{
+    frames.clear(); *status = 0;
+    if (!srcSize) return 0;
+    if (!src) return ZL_ERROR(GENERIC);
+    if (srcSize < 5) { *status = ZL_ERROR(srcSize_wrong); return 0; }            // zstd.c:41681, 41766
+    if (!zl_ctx_stream(&c->stream, &c->ownStream, &c->ev0, &c->ev1)) return ZL_ERROR(memory_allocation);
+    cudaStream_t st = c->stream;
+    const u64 head = (size_t)src & 15;
+    const u64 tiles1 = (head + srcSize + 16 * ZL_IDX_TILE_THREADS * ZL_IDX_TILE_CHUNKS - 1) / (16 * ZL_IDX_TILE_THREADS * ZL_IDX_TILE_CHUNKS);
+    const u64 tilesMax = std::max<u64>(tiles1, (srcSize + ZL_IDX_TILE_NODES - 1) / ZL_IDX_TILE_NODES);
+    if (tilesMax >= 0xFFFFFFFFull) return ZL_ERROR(memory_allocation);
+    // tile buffer: counts (u32) | offsets (u64, tiles + 1) | open counters of the marking passes | status
+    const size_t offAt = (tilesMax * 4 + 15) & ~(size_t)15, openAt = offAt + (tilesMax + 1) * 8, statAt = openAt + ZL_IDX_MAX_PASSES * 4;
+    if (!c->dIdxTile.reserve(statAt + sizeof(ZlIdxStatus)) || !c->hIdx.reserve(64)) return ZL_ERROR(memory_allocation);
+    u8* tb = c->dIdxTile.as<u8>();
+    u32* tileCount = (u32*)tb; u64* tileOff = (u64*)(tb + offAt); u32* open = (u32*)(tb + openAt); ZlIdxStatus* dStatus = (ZlIdxStatus*)(tb + statAt);
+    u64* h = c->hIdx.as<u64>();
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess) { (void)cudaGetLastError(); fprintf(stderr, "zstdlite_gpu: index launch failed: %s\n", cudaGetErrorString(e)); } return ZL_ERROR(GENERIC); };
+    auto fetch = [&](void* dst, const void* from, size_t n) {
+        return cudaMemcpyAsync(dst, from, n, cudaMemcpyDeviceToHost, st) == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+    };
+    // I1
+    cudaError_t e = zl_launch_idx_candidates(src, srcSize, (u32)tiles1, tileCount, tileOff, nullptr, st);
+    c->launches += 2;
+    if (e != cudaSuccess || !fetch(h, tileOff + tiles1, 8)) return fail(e);
+    const u64 n64 = h[0];
+    if (!n64) { *status = ZL_ERROR(prefix_unknown); return 0; }
+    if (n64 >= ZL_LINK_NODES) return ZL_ERROR(memory_allocation);
+    const u32 n = (u32)n64;
+    if (!c->dIdx.reserve((size_t)n * 32)) return ZL_ERROR(memory_allocation);
+    u64* cand = c->dIdx.as<u64>();
+    u32 *link = (u32*)(cand + n), *errc = link + n, *nblk = errc + n, *mark = nblk + n, *j0 = mark + n, *j1 = j0 + n;
+    e = zl_launch_idx_candidates(src, srcSize, (u32)tiles1, tileCount, tileOff, cand, st);
+    c->launches += 1;
+    // I2
+    if (e == cudaSuccess) e = zl_launch_idx_extent(src, srcSize, cand, n, ZL_IDX_W, link, errc, nblk, mark, st);
+    c->launches += 1;
+    if (e != cudaSuccess) return fail(e);
+    const u32 tiles4 = (u32)((n64 + ZL_IDX_TILE_NODES - 1) / ZL_IDX_TILE_NODES);
+    ZlIdxStatus hs{};
+    for (u32 round = 0;; round++) {
+        // I3: marking passes in groups of 4, until one pass finds every marked chain covered
+        cudaMemcpyAsync(j0, link, (size_t)n * 4, cudaMemcpyDeviceToDevice, st);
+        cudaMemsetAsync(open, 0, ZL_IDX_MAX_PASSES * 4, st);
+        for (u32 pass = 0;; pass += 4) {
+            if (pass + 4 > ZL_IDX_MAX_PASSES) return ZL_ERROR(GENERIC);          // (cannot happen: ceil(log2 n) + 1 passes cover any chain)
+            e = zl_launch_idx_jump(n, j0, j1, mark, open, pass, 4, st);
+            c->launches += 4;
+            if (e != cudaSuccess || !fetch(h, open + pass + 3, 4)) return fail(e);
+            if (((const u32*)h)[0] == 0) break;
+        }
+        // I4, first half: the chain's last candidate
+        cudaMemsetAsync(dStatus, 0xFF, sizeof(ZlIdxStatus), st);
+        e = zl_launch_idx_frames(src, srcSize, cand, n, link, errc, nblk, mark, tiles4, tileCount, tileOff, dStatus, nullptr, st);
+        c->launches += 2;
+        if (e != cudaSuccess || !fetch(h, dStatus, sizeof(ZlIdxStatus))) return fail(e);
+        memcpy(&hs, h, sizeof(hs));
+        if (hs.first != 0 || hs.link != ZL_LINK_LONG) break;
+        // frontier: the chain ends in a frame of more than ZL_IDX_W blocks (or a long look-alike): finish it on one thread
+        e = zl_launch_idx_frontier(src, srcSize, cand, n, link, errc, nblk, mark, dStatus, round >= ZL_IDX_R, st);
+        c->launches += 1;
+        if (e != cudaSuccess) return fail(e);
+    }
+    *status = zl_idx_tail_error(n64, hs.first, hs.link, hs.err);
+    if (hs.first != 0) return 0;
+    if (!fetch(h, tileOff + tiles4, 8)) return fail(cudaSuccess);
+    const u64 nf = h[0];
+    if (!c->dIdxFrames.reserve(nf * sizeof(ZlStreamFrame) + 16) || !c->hIdx.reserve(nf * sizeof(ZlStreamFrame) + 64)) return ZL_ERROR(memory_allocation);
+    e = zl_launch_idx_frames(src, srcSize, cand, n, link, errc, nblk, mark, tiles4, tileCount, tileOff, dStatus, c->dIdxFrames.as<ZlStreamFrame>(), st);
+    c->launches += 1;
+    if (e != cudaSuccess || !fetch(c->hIdx.p, c->dIdxFrames.p, nf * sizeof(ZlStreamFrame))) return fail(e);
+    const ZlStreamFrame* hf = c->hIdx.as<ZlStreamFrame>();
+    frames.assign(hf, hf + nf);
+    return 0;
+}
+
+ZL_EXPORT size_t zl_device_frames(ZSTD_DCtx* c, const void* src, size_t srcSize, unsigned long long* cOff, unsigned long long* cSize,
+                                  unsigned long long* dSize, size_t cap)
+{
+    if (!c) return ZL_ERROR(GENERIC);
+    ZlDeviceGuard guard(zl_bind_device(&c->device));
+    if (!guard.ok) return ZL_ERROR(GENERIC);
+    std::vector<ZlStreamFrame> f;
+    size_t status = 0;
+    const size_t r = zl_device_index(c, (const u8*)src, srcSize, f, &status);
+    if (zl_is_error(r)) return r;
+    if (zl_is_error(status)) return status;
+    if (cap >= f.size())
+        for (size_t k = 0; k < f.size(); k++) {
+            if (cOff) cOff[k] = f[k].cOff;
+            if (cSize) cSize[k] = f[k].cSize;
+            if (dSize) dSize[k] = f[k].dSize;
+        }
+    return f.size();
+}
+
+// ZSTD_decompressDCtx for a stream and a destination in device memory: index, then the frames with a content size in one engine call
+// straight into dst; frames without one are decoded first into scratch, and moved into place by one zl_k_range_scatter launch.
+ZL_EXPORT size_t zl_decompress_device(ZSTD_DCtx* c, void* dst, size_t dstCap, const void* src, size_t srcSize)
+{
+    if (!c) return ZL_ERROR(GENERIC);
+    ZlDeviceGuard guard(zl_bind_device(&c->device));
+    if (!guard.ok) return ZL_ERROR(GENERIC);
+    std::vector<ZlStreamFrame> f;
+    size_t status = 0;
+    size_t r = zl_device_index(c, (const u8*)src, srcSize, f, &status);
+    if (zl_is_error(r)) return r;
+    ZlDevPlan p;
+    r = zl_dev_plan_unknown(p, f, status, dstCap);
+    if (zl_is_error(r)) return r;
+    cudaStream_t st = c->stream;
+    std::vector<const void*> fsrc; std::vector<void*> fdst; std::vector<size_t> fsize, fcap;
+    auto batch = [&](const std::vector<ZlDevDecode>& d, u8* base, std::vector<size_t>& res) -> size_t {
+        const size_t m = d.size();
+        res.assign(m, 0);
+        if (!m) return 0;
+        fsrc.resize(m); fdst.resize(m); fsize.resize(m); fcap.resize(m);
+        for (size_t i = 0; i < m; i++) {
+            const ZlStreamFrame& x = f[d[i].frame];
+            fsrc[i] = (const u8*)src + x.cOff; fsize[i] = x.cSize; fdst[i] = base + d[i].place; fcap[i] = d[i].cap;
+        }
+        return zl_decompress_batch_one(c, fsrc.data(), fsize.data(), fdst.data(), fcap.data(), res.data(), m, 1);
+    };
+    std::vector<size_t> ures, kres;
+    if (!p.unknown.empty() && !c->dSeek.reserve(p.scratchBytes + 64)) return ZL_ERROR(memory_allocation);
+    r = batch(p.unknown, c->dSeek.as<u8>(), ures);
+    if (zl_is_error(r)) return r;
+    zl_dev_plan_places(p, f, ures.data(), dstCap);
+    r = batch(p.known, (u8*)dst, kres);
+    if (zl_is_error(r)) return r;
+    const size_t result = zl_dev_plan_result(p, kres.data());
+    if (zl_is_error(result) || p.pieces.empty()) return result;
+    const size_t items = p.pieces.size();
+    if (!c->hScatter.reserve(items * sizeof(ZlScatterItem)) || !c->dScatter.reserve(items * sizeof(ZlScatterItem))) return ZL_ERROR(memory_allocation);
+    ZlScatterItem* hsc = c->hScatter.as<ZlScatterItem>();
+    for (size_t i = 0; i < items; i++) hsc[i] = {c->dSeek.as<u8>() + p.pieces[i].from, (u8*)dst + p.pieces[i].to, (u32)p.pieces[i].bytes};
+    cudaMemcpyAsync(c->dScatter.p, hsc, items * sizeof(ZlScatterItem), cudaMemcpyHostToDevice, st);
+    if (zl_launch_range_scatter(c->dScatter.as<ZlScatterItem>(), (u32)items, st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
+    c->launches += 1;
+    if (cudaStreamSynchronize(st) != cudaSuccess) { (void)cudaGetLastError(); return ZL_ERROR(GENERIC); }
+    return result;
 }

@@ -3,11 +3,13 @@
 //   K2 zl_k_execute   warp-per-frame sequence execution -> frame output
 //   K3 zl_k_checksum  quad-per-frame XXH64 of the output, compared with the frame trailer (and a seek table's checksum)
 //   zl_k_range_scatter  warp-per-piece copy-out of zl_decompress_ranges
+//   zl_k_idx_*          the frame index of a stream in device memory (zl_dec_index.cuh)
 #include "zl_dec_entropy.cuh"
 #include "zl_dec_exec.cuh"
 #include "zl_dec_large.cuh"
 #include "zl_launch.h"
 #include "zl_plan.h"
+#include "zl_dec_index.cuh"
 #include <mutex>
 #include <stdlib.h>
 

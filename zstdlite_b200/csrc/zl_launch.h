@@ -109,6 +109,19 @@ cudaError_t zl_launch_xxh64(const u8* const* ptrs, const u32* sizes, u64* out, u
 #define ZL_SCATTER_BYTES (64u << 10)
 struct ZlScatterItem { const u8* src; u8* dst; u32 bytes; };
 cudaError_t zl_launch_range_scatter(const ZlScatterItem* items, u32 n, cudaStream_t st);
+// frame index of a stream in device memory (zl_dec_index.cuh, zl_stream_index.h)
+struct ZlStreamFrame { u64 cOff, cSize, dSize; u32 nblocks, bsm; };      // bsm: blockSizeMax, ZL_FRAME_SKIP for a skippable frame
+#define ZL_FRAME_SKIP 0xFFFFFFFFu
+struct ZlIdxStatus { u64 first; u32 tail, link, err, pad; };            // first candidate's offset; the chain's last candidate
+// I1: cand null: per-tile counts and their prefix sums (tileOff, tiles + 1 entries); else the candidates' offsets into cand
+cudaError_t zl_launch_idx_candidates(const u8* src, u64 srcSize, u32 tiles, u32* tileCount, u64* tileOff, u64* cand, cudaStream_t st);
+cudaError_t zl_launch_idx_extent(const u8* src, u64 srcSize, const u64* cand, u32 n, u32 cap, u32* link, u32* errc, u32* nblk, u32* mark, cudaStream_t st);
+cudaError_t zl_launch_idx_jump(u32 n, u32* j0, u32* j1, u32* mark, u32* open, u32 pass0, u32 passes, cudaStream_t st);
+cudaError_t zl_launch_idx_frontier(const u8* src, u64 srcSize, const u64* cand, u32 n, u32* link, u32* errc, u32* nblk, u32* mark,
+                                   const ZlIdxStatus* status, bool serial, cudaStream_t st);
+// I4: frames null: per-tile counts of marked candidates, their prefix sums and *status; else the frame records
+cudaError_t zl_launch_idx_frames(const u8* src, u64 srcSize, const u64* cand, u32 n, const u32* link, const u32* errc, const u32* nblk,
+                                 const u32* mark, u32 tiles, u32* tileCount, u64* tileOff, ZlIdxStatus* status, ZlStreamFrame* frames, cudaStream_t st);
 
 // ---- compression --------------------------------------------------------------------------------------------------
 #include "zl_enc_entropy.cuh"
